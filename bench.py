@@ -2,7 +2,7 @@
 """bench.py -- ELBO-gradient iterations/s on BASELINE.json configs[1]:
 Bayesian logistic regression N=1e6, d=512, S=256, MFGaussian + RMSProp (synthetic data).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--path f64|fast] [--impl reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--path f64|fast] [--impl reference] [--dump-outputs DIR]
 
 One "step" = the three hot-path calls of the reference loop (optimization.py:95-98):
 objective(var_param) (Philox draws -> sweep over all N observations -> value + gradient),
@@ -54,9 +54,18 @@ def parse():
     ap.add_argument('--no-f64', action='store_true')
     ap.add_argument('--no-graph', action='store_true', help='enqueue every step from Python instead of replaying graphs')
     ap.add_argument('--psis-draws', type=int, default=100000000)
-    ap.add_argument('--ref-seconds', type=float, default=150.0, help='time budget of the reference arm')
+    ap.add_argument('--ref-seconds', type=float, default=None,
+                    help='time budget of the reference arm: it stops timing early (after at least 2 steps) when the '
+                         'next step would exceed it; without it, all --steps steps are timed')
     ap.add_argument('--config', default='c2', choices=['c2', 'c4'], help='c2: the headline ELBO-gradient bench; c4: BASELINE configs[3]')
-    return ap.parse_args()
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='write what the last timed step computed (value, grad, var_param) as DIR/<name>.npy (float64)')
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and (args.impl != 'b200' or args.config != 'c2'):
+        ap.error('--dump-outputs applies to the headline ELBO-gradient bench (--impl b200 --config c2)')
+    return args
 
 
 def workload_name(N, d, S):
@@ -148,9 +157,9 @@ def run_reference(args):
     sec, done, workers = cpu_iterations(args.n_obs, args.dim, args.mc, args.steps, max(1, min(args.warmup, 1)),
                                         budget_s=args.ref_seconds)
     value = 1.0 / sec
+    budget = '' if args.ref_seconds is None else ' (time budget %.0f s)' % args.ref_seconds
     sample = ('oracle (numpy float64 port of the reference iteration) on all %d rows, %d of the %d requested '
-              'steps timed (time budget %.0f s), row blocks over %d threads' % (args.n_obs, done, args.steps,
-                                                                               args.ref_seconds, workers))
+              'steps timed%s, row blocks over %d threads' % (args.n_obs, done, args.steps, budget, workers))
     line = {
         'impl': 'reference', 'metric': 'elbo_grad_iters_per_sec', 'value': value, 'unit': 'iter/s',
         'n_gpus': args.gpus, 'steps': done, 'warmup': max(1, min(args.warmup, 1)), 'ms_per_step': sec * 1e3,
@@ -460,6 +469,27 @@ def time_steps(torch, eng, steps, use_graph):
     return e0.elapsed_time(e1) * 1e-3
 
 
+def device_problem(torch, vb, N, d, S, path, rank=0, world=1, dev='cuda'):
+    """(model, approx, objective) of the headline bench on this rank's rows of the seeded N x d problem."""
+    from viabel_b200.parallel import shard_rows
+    # this rank's rows [lo, hi) of the N x d problem; rank r seeds its rows with DATA_SEED + r
+    lo, hi = shard_rows(N, rank, world)
+    gen = torch.Generator(device=dev)
+    gen.manual_seed(DATA_SEED + 7919)
+    beta = torch.randn(d, generator=gen, device=dev, dtype=torch.float64) / np.sqrt(d)
+    gen.manual_seed(DATA_SEED + rank)
+    X = torch.randn(hi - lo, d, generator=gen, device=dev, dtype=torch.float64)
+    p = torch.sigmoid(X @ beta)
+    y = torch.where(torch.rand(hi - lo, generator=gen, device=dev, dtype=torch.float64) < p, 1.0, -1.0)
+    del p
+
+    model = vb.LogisticRegression(X, y, prior_scale=10.0, sharded=world > 1)
+    approx = vb.MFGaussian(d, seed=DRAW_SEED)
+    if path == 'fast':
+        model.enable_fast_path(approx)    # tcgen05 + TMA, fp16 hi/lo operand splits; fp16-exact draws (see DESIGN 4.2)
+    return model, approx, vb.ExclusiveKL(approx, model, S)
+
+
 def run_b200(args):
     import torch
     import torch.distributed as dist
@@ -477,23 +507,9 @@ def run_b200(args):
     use_graph = not args.no_graph
 
     N, d, S = args.n_obs, args.dim, args.mc
-    # this rank's rows [lo, hi) of the N x d problem; rank r seeds its rows with DATA_SEED + r
     lo, hi = shard_rows(N, rank, world)
-    gen = torch.Generator(device=dev)
-    gen.manual_seed(DATA_SEED + 7919)
-    beta = torch.randn(d, generator=gen, device=dev, dtype=torch.float64) / np.sqrt(d)
-    gen.manual_seed(DATA_SEED + rank)
-    X = torch.randn(hi - lo, d, generator=gen, device=dev, dtype=torch.float64)
-    p = torch.sigmoid(X @ beta)
-    y = torch.where(torch.rand(hi - lo, generator=gen, device=dev, dtype=torch.float64) < p, 1.0, -1.0)
-    del p
-
     path = 'fast' if args.path == 'auto' else args.path
-    model = vb.LogisticRegression(X, y, prior_scale=10.0, sharded=world > 1)
-    approx = vb.MFGaussian(d, seed=DRAW_SEED)
-    if path == 'fast':
-        model.enable_fast_path(approx)    # tcgen05 + TMA, fp16 hi/lo operand splits; fp16-exact draws (see DESIGN 4.2)
-    objective = vb.ExclusiveKL(approx, model, S)
+    model, approx, objective = device_problem(torch, vb, N, d, S, path, rank, world, dev)
     opt = vb.RMSProp(0.01)
     eng = FusedStep(objective, opt)       # the object RMSProp.optimize() drives
     eng.set_param(approx.init_param())
@@ -517,6 +533,9 @@ def run_b200(args):
     # (1) burst: the first K steps after the warm-up, GPU clocks still at their idle-boost state
     burst = max_over_ranks(time_steps(torch, eng, args.steps, use_graph))
     barrier()
+    # the settle phase's length follows the measured rate, so the timed steps restart from the state the burst left
+    # (iterate, optimiser state, draw-stream position): they compute the same thing in every run with the same arguments
+    start = eng.save_state()
     # (2) settle: the same step for >= 1.2 s, untimed for `value` but reported as `sustained`.  These boxes reach their
     # steady clocks only after a few hundred ms of load (one busy GPU is power-capped DOWN, eight lightly loaded ones
     # clock UP), so a number taken in the first 20 ms describes neither.  Same count on every rank: the step
@@ -524,9 +543,14 @@ def run_b200(args):
     n_sus = max(args.steps, min(20000, int(1.2 / max(burst / args.steps, 1e-5))))
     n_sus = (n_sus + 7) // 8 * 8
     sus = max_over_ranks(time_steps(torch, eng, n_sus, use_graph))
+    eng.rewind(start)                     # device-side copies, enqueued behind the settle phase
     # (3) the K timed steps, in the steady state, back to back with the settle phase (no idle gap)
     elapsed = max_over_ranks(time_steps(torch, eng, args.steps, use_graph))
     barrier()
+    if args.dump_outputs and rank == 0:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, t in (('value', eng.value), ('grad', eng.grad), ('var_param', eng.vp)):
+            np.save(os.path.join(args.dump_outputs, name + '.npy'), t.cpu().numpy())
     ms_per_step = elapsed / args.steps * 1e3
     clocks = sampler.stop() if sampler else None
     eng.check_comm()

@@ -241,6 +241,17 @@ class FusedStep(object):
         if snap[3] is not None:
             self.opt_m.copy_(snap[3])
 
+    def save_state(self):
+        """Device copy of everything a step reads and advances (iterate, optimiser state, step and draw-stream
+        counters), with the host's step count; no host synchronisation."""
+        return self._snapshot(), self.steps_done
+
+    def rewind(self, state):
+        """Return to a state from save_state(): the steps that follow recompute what followed it, same draws included."""
+        snap, self.steps_done = state
+        self._restore(snap)
+        self._after()
+
     def _capture(self, key, body):
         g = self._graphs.get(key)
         if g is None:
