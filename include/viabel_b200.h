@@ -399,6 +399,27 @@ int vb_mvt_log_density_f64(const double* var_param, const double* w, const doubl
                            double df, double* out, void* workspace, size_t workspace_bytes, cudaStream_t stream);
 
 /* ---------------------------------------------------------------------------------------
+ * Full-rank MultivariateT in the Cholesky reparameterisation (MultivariateT(..., reparam='cholesky')): theta_s =
+ * mu + L z_s / u_s instead of the reference's mu + (z_s / u_s) sqrtm(Sigma) (approximations.py:342-349).  Same
+ * distribution, same objectives as functions of var_param, a different per-draw map; no eigensolver, no d x d
+ * temporaries, O(S d^2) float64 tensor-core work.  Deterministic (fixed summation order, no atomics).
+ *   vb_mvt_chol_transform_f64  theta[S,d] = mu + diag(1/u) z L^T, inv_u[S] = 1/u_s, zu2[S] = |z_s/u_s|^2,
+ *                              u_s = sqrt(chi2_s / df)                             (sample :342-349)
+ *   vb_mvt_chol_objective_f64  value[1], grad[d + d(d+1)/2] of ExclusiveKL (entropy form, objectives.py:154-164) /
+ *                              AlphaDivergence (:443-460) from the model's f[S], G[S,d] at theta:
+ *                              grad_mu = c sum_s sv_s G_s,  Fbar[i,j] = c sum_s sv_s G[s,i] z[s,j]/u_s (j < i),
+ *                              Fbar[i,i] = (c sum_s sv_s G[s,i] z[s,i]/u_s) L_ii + diag_add;
+ *                              c = -1/S, sv = 1, diag_add = -1 (ExclusiveKL) or c = alpha/S, sv_s = exp(lw_s - max lw)^alpha,
+ *                              diag_add = c sum_s sv_s (AlphaDivergence)
+ * ------------------------------------------------------------------------------------- */
+int vb_mvt_chol_transform_f64(const double* var_param, const double* z, const double* chi2, double df, int S, int d,
+                              double* theta, double* inv_u, double* zu2, cudaStream_t stream);
+size_t vb_mvt_chol_objective_workspace_bytes(int S, int d);
+int vb_mvt_chol_objective_f64(const double* var_param, const double* z, const double* inv_u, const double* zu2,
+                              const double* f, const double* G, int S, int d, double df, int objective, double alpha,
+                              double* value, double* grad, void* workspace, size_t workspace_bytes, cudaStream_t stream);
+
+/* ---------------------------------------------------------------------------------------
  * Hierarchical linear regression plugin (BASELINE configs[3]) with per-sample gradients: a grouped contraction
  * (no block-expanded design matrix).  X[N,p], y[N] sorted by group; goff[G+1] device int64 row offsets;
  * theta[S,D], D = G p + p + 2 = [beta (group-major), m, log tau, log sigma]; p <= 32.

@@ -242,11 +242,23 @@ class MultivariateT(ApproximationFamily):
 
     Device path (csrc/mvt.cu + csrc/gemm_f64.cu): the Cholesky-vector unpack, Sigma = L L^T, the reparameterisation
     through the eigenbasis and every cotangent GEMM are this package's float64 tensor-core kernels; the symmetric
-    eigen-decomposition is the one library call (cuSOLVER via torch.linalg.eigh)."""
+    eigen-decomposition is the one library call (cuSOLVER via torch.linalg.eigh).
 
-    def __init__(self, dim, df, seed=1):
+    reparam='cholesky' samples theta = mu + L z / u instead (csrc/mvt_chol.cu).  L L^T = Sigma, so the draws have
+    the same distribution and ExclusiveKL / AlphaDivergence are the same functions of var_param, but the gradient is
+    a different (equally unbiased) Monte Carlo estimator: per draw it does not match the reference.  Sampling and both
+    objectives then cost O(S d^2) float64 tensor-core work with no eigensolver, no d x d temporary and no host
+    synchronisation.  Everything else (var_param layout, base draws, log_density, entropy, moments) is the same in
+    both modes."""
+
+    REPARAMS = ('sqrtm', 'cholesky')
+
+    def __init__(self, dim, df, seed=1, reparam='sqrtm'):
         if df <= 2:
             raise ValueError('df must be greater than 2')
+        if reparam not in self.REPARAMS:
+            raise ValueError("reparam must be 'sqrtm' or 'cholesky', got %r" % (reparam,))
+        self._reparam = reparam
         self._df = df
         self._seed = int(seed)
         self._offset = 0
@@ -256,6 +268,11 @@ class MultivariateT(ApproximationFamily):
     @property
     def df(self):
         return self._df
+
+    @property
+    def reparam(self):
+        """'sqrtm' (theta = mu + (z / u) sqrtm(Sigma), the reference's map) or 'cholesky' (theta = mu + L z / u)."""
+        return self._reparam
 
     def init_param(self):
         # mu = 0, Sigma = 10 I  ->  F = diag(log sqrt(10))   (approximations.py:337-340)
@@ -326,6 +343,21 @@ class MultivariateT(ApproximationFamily):
                                                  ws.numel(), _lib.stream()))
         return theta, P, zu2
 
+    def chol_transform(self, vp, chi2, z):
+        """(theta[S,d], inv_u[S], zu2[S]): theta = mu + L z / u through the triangular float64 tensor-core kernel
+        (vb_mvt_chol_transform_f64), reading L straight from var_param."""
+        if vp.numel() != self.var_param_dim:
+            raise ValueError('var_param has the wrong length')
+        S, d = int(z.shape[0]), self.dim
+        if z.dim() != 2 or int(z.shape[1]) != d or chi2.numel() != S:
+            raise ValueError('base draws must be chi2[S] and z[S, %d]' % d)
+        theta = torch.empty(S, d, dtype=F64, device=z.device)
+        inv_u = torch.empty(S, dtype=F64, device=z.device)
+        zu2 = torch.empty(S, dtype=F64, device=z.device)
+        _lib.check(_lib.lib.vb_mvt_chol_transform_f64(_lib.ptr(vp), _lib.ptr(z), _lib.ptr(chi2), float(self._df), S, d,
+                                                      _lib.ptr(theta), _lib.ptr(inv_u), _lib.ptr(zu2), _lib.stream()))
+        return theta, inv_u, zu2
+
     # -- base draws: chi-square FIRST, then normals, as the reference (:345-347) -------------------
     def base_draws(self, n_samples, seed=None):
         n, d = int(n_samples), self.dim
@@ -345,8 +377,11 @@ class MultivariateT(ApproximationFamily):
         vp = to_dev(var_param)
         chi2, z = self.base_draws(n_samples, seed) if base is None else (to_dev(base[0]).reshape(-1), to_dev(base[1]))
         self.last_base = (chi2, z)
-        _, _, w, V = self.decompose(vp)
-        theta, _, _ = self.transform(vp, chi2, z, w, V)
+        if self._reparam == 'cholesky':
+            theta, _, _ = self.chol_transform(vp, chi2, z)
+        else:
+            _, _, w, V = self.decompose(vp)
+            theta, _, _ = self.transform(vp, chi2, z, w, V)
         return like_input(theta, host)
 
     def entropy(self, var_param):

@@ -13,6 +13,7 @@
 // All GEMMs are the float64 DMMA kernel of gemm_f64.cu with the row / column / division scalings fused into its
 // pro- and epilogues.  SURVEY.md App. A.3 has the derivation.
 #include "gemm_internal.cuh"
+#include "mvt_internal.cuh"
 
 namespace vb {
 
@@ -179,9 +180,29 @@ __global__ void __launch_bounds__(256) mvt_sumlog_kernel(const double* __restric
   if (threadIdx.x == 0) out[0] = a;
 }
 
-static inline double mvt_const(double df, int d) {
-  return lgamma(0.5 * (df + d)) - lgamma(0.5 * df) - 0.5 * d * log(3.14159265358979323846 * df);
+int mvt_rows(const double* z, const double* chi2, double df, int S, int d, double* inv_u, double* zu2, cudaStream_t stream) {
+  mvt_rows_kernel<<<(S * 32 + 255) / 256, 256, 0, stream>>>(z, chi2, df, S, d, inv_u, zu2);
+  VB_CHECK_LAUNCH();
+  return VB_OK;
 }
+
+int mvt_logdiag(const double* var_param, int d, double* out, cudaStream_t stream) {
+  mvt_logdiag_kernel<<<1, 256, 0, stream>>>(var_param, d, out);
+  VB_CHECK_LAUNCH();
+  return VB_OK;
+}
+
+int mvt_weights_gmu(const double* f, const double* G, const double* zu2, const double* half_logdet, int S, int d, double df,
+                    int objective, double alpha, double* sv, double* scal, double* value, double* gmu, cudaStream_t stream) {
+  const double c = objective == VB_OBJ_EXCLUSIVE_KL ? -1.0 / S : alpha / S;
+  mvt_weights_kernel<<<1, 1024, 0, stream>>>(f, zu2, S, d, df, mvt_const(df, d), half_logdet, objective, alpha, sv, scal);
+  VB_CHECK_LAUNCH();
+  VB_CUDA(cudaMemcpyAsync(value, scal, sizeof(double), cudaMemcpyDeviceToDevice, stream));
+  mvt_gmu_kernel<<<(d + 31) / 32, 1024, 0, stream>>>(G, sv, S, d, c, gmu);
+  VB_CHECK_LAUNCH();
+  return VB_OK;
+}
+
 static inline int ew_grid(int64_t n) {
   int64_t b = (n + 255) / 256;
   const int64_t cap = 16LL * sm_count();
@@ -205,11 +226,7 @@ extern "C" int vb_mvt_unpack_f64(const double* var_param, int d, double* L, doub
   if (!var_param || d <= 0 || !L) return set_error(VB_ERR_INVALID_ARG, "mvt_unpack: bad arguments");
   mvt_unpack_kernel<<<ew_grid((int64_t)d * d), 256, 0, stream>>>(var_param, d, L);
   VB_CHECK_LAUNCH();
-  if (half_logdet) {
-    mvt_logdiag_kernel<<<1, 256, 0, stream>>>(var_param, d, half_logdet);
-    VB_CHECK_LAUNCH();
-  }
-  return VB_OK;
+  return half_logdet ? mvt_logdiag(var_param, d, half_logdet, stream) : VB_OK;
 }
 
 /* Sigma = L L^T */
@@ -236,11 +253,11 @@ extern "C" int vb_mvt_transform_f64(const double* var_param, const double* z, co
   char* ws = static_cast<char*>(workspace);
   double* inv_u = reinterpret_cast<double*>(ws);
   double* sqrtw = reinterpret_cast<double*>(ws + align_up(sizeof(double) * S, 256));
-  mvt_rows_kernel<<<(S * 32 + 255) / 256, 256, 0, stream>>>(z, chi2, df, S, d, inv_u, zu2);
-  VB_CHECK_LAUNCH();
+  int rc = mvt_rows(z, chi2, df, S, d, inv_u, zu2, stream);
+  if (rc) return rc;
   mvt_eig_kernel<<<(d + 255) / 256, 256, 0, stream>>>(w, d, sqrtw, nullptr);
   VB_CHECK_LAUNCH();
-  int rc = gemm(false, false, S, d, d, 1.0, z, d, V, d, P, d, nullptr, inv_u, nullptr, nullptr, nullptr, stream);
+  rc = gemm(false, false, S, d, d, 1.0, z, d, V, d, P, d, nullptr, inv_u, nullptr, nullptr, nullptr, stream);
   if (rc) return rc;
   return gemm(false, true, S, d, d, 1.0, P, d, V, d, theta, d, sqrtw, nullptr, var_param, nullptr, nullptr, stream);
 }
@@ -293,14 +310,11 @@ extern "C" int vb_mvt_objective_f64(const double* L, const double* half_logdet, 
   double* T = reinterpret_cast<double*>(ws + l.off_T);
   double* Lbar = reinterpret_cast<double*>(ws + l.off_Lbar);
   const double c = objective == VB_OBJ_EXCLUSIVE_KL ? -1.0 / S : alpha / S;
-  mvt_weights_kernel<<<1, 1024, 0, stream>>>(f, zu2, S, d, df, mvt_const(df, d), half_logdet, objective, alpha, sv, scal);
-  VB_CHECK_LAUNCH();
-  VB_CUDA(cudaMemcpyAsync(value, scal, sizeof(double), cudaMemcpyDeviceToDevice, stream));
-  mvt_gmu_kernel<<<(d + 31) / 32, 1024, 0, stream>>>(G, sv, S, d, c, grad);
-  VB_CHECK_LAUNCH();
+  int rc = mvt_weights_gmu(f, G, zu2, half_logdet, S, d, df, objective, alpha, sv, scal, value, grad, stream);
+  if (rc) return rc;
   mvt_eig_kernel<<<(d + 255) / 256, 256, 0, stream>>>(w, d, sqrtw, nullptr);
   VB_CHECK_LAUNCH();
-  int rc = gemm(false, false, S, d, d, 1.0, G, d, V, d, Q, d, nullptr, sv, nullptr, nullptr, nullptr, stream);     // Q = (sv . G) V
+  rc = gemm(false, false, S, d, d, 1.0, G, d, V, d, Q, d, nullptr, sv, nullptr, nullptr, nullptr, stream);     // Q = (sv . G) V
   if (rc) return rc;
   rc = gemm(true, false, d, d, S, c, P, d, Q, d, M, d, nullptr, nullptr, nullptr, sqrtw, sqrtw, stream);           // c P^T Q ./ (rw + rw')
   if (rc) return rc;

@@ -91,6 +91,8 @@ def _mvt_objective(approx, model, S, objective, alpha, var_param, base=None, see
     chi2, z = approx.base_draws(S, seed) if base is None else (to_dev(base[0]).reshape(-1), to_dev(base[1]))
     approx.last_base = (chi2, z)
     S = int(z.shape[0])
+    if approx.reparam == 'cholesky':
+        return _mvt_chol_objective(approx, model, objective, alpha, vp, chi2, z)
     L, hl, w, V = approx.decompose(vp)
     theta, P, zu2 = approx.transform(vp, chi2, z, w, V)
     f, G = model.logp_and_grad(theta)
@@ -100,6 +102,21 @@ def _mvt_objective(approx, model, S, objective, alpha, var_param, base=None, see
         _lib.ptr(L), _lib.ptr(hl), _lib.ptr(w), _lib.ptr(V), _lib.ptr(P), _lib.ptr(zu2), _lib.ptr(f.contiguous()),
         _lib.ptr(G.contiguous()), S, d, df, objective, float(alpha), _lib.ptr(out[:1]), _lib.ptr(out[1:]), _lib.ptr(ws),
         ws.numel(), _lib.stream()))
+    return out[0], out[1:]
+
+
+def _mvt_chol_objective(approx, model, objective, alpha, vp, chi2, z):
+    """The same objectives in MultivariateT's Cholesky reparameterisation, theta = mu + L z / u: triangular transform
+    -> model plugin -> vb_mvt_chol_objective_f64 (csrc/mvt_chol.cu).  No eigensolver and no host synchronisation."""
+    S, d = int(z.shape[0]), approx.dim
+    theta, inv_u, zu2 = approx.chol_transform(vp, chi2, z)
+    f, G = model.logp_and_grad(theta)
+    out = torch.empty(1 + vp.numel(), dtype=F64, device=vp.device)
+    ws = torch.empty(_lib.lib.vb_mvt_chol_objective_workspace_bytes(S, d), dtype=torch.uint8, device=vp.device)
+    _lib.check(_lib.lib.vb_mvt_chol_objective_f64(
+        _lib.ptr(vp), _lib.ptr(z), _lib.ptr(inv_u), _lib.ptr(zu2), _lib.ptr(f.contiguous()), _lib.ptr(G.contiguous()), S, d,
+        float(approx.df), objective, float(alpha), _lib.ptr(out[:1]), _lib.ptr(out[1:]), _lib.ptr(ws), ws.numel(),
+        _lib.stream()))
     return out[0], out[1:]
 
 
