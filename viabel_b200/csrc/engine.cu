@@ -628,6 +628,8 @@ extern "C" int vb_mf_step_glm(const vb_step_config* cfg, const vb_step_buffers* 
   if (cfg->optimizer == 2 && !buf->opt_m) return set_error(VB_ERR_INVALID_ARG, "mf_step: Adam needs opt_m");
   const int fast = model->fast_handle != nullptr;
   if (fast && S > fast::kPadS) return set_error(VB_ERR_UNSUPPORTED, "mf_step: the tensor-core sweep takes at most 256 samples");
+  // the pre kernel's row tiles sit on gridDim.y (at most 65535)
+  if (ceil_div(S, kPreRows) > 65535) return set_error(VB_ERR_UNSUPPORTED, "mf_step: at most 1048560 samples per step");
   StepLayout L;
   step_layout(S, d, fast, L);
   if (workspace_bytes < L.total) return set_error(VB_ERR_WORKSPACE, "mf_step: workspace too small");

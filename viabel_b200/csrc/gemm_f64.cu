@@ -7,7 +7,9 @@
 //     epilogue(v) = v * rowscale[m]  /  (divm[m] + divn[n])  +  bias[n]          (each optional)
 //
 // 64 x 64 output tiles, K slabs of 32 through shared memory, 8 warps of 16 x 32 accumulators each (the same tiling
-// as the SYRK in moments.cu).  Deterministic: no split-K.
+// as the SYRK in moments.cu).  Deterministic: no split-K.  The tiles are numbered row-major on a 1-D grid (gridDim.x
+// allows 2^31 - 1 blocks, gridDim.y only 65535), so M and N are both limited only by their int type: the GLM plugins
+// put the sample count on N in one GEMM and on M in the next.
 #include "gemm_internal.cuh"
 
 namespace vb {
@@ -23,7 +25,8 @@ __device__ __forceinline__ void dmma_g(double& c0, double& c1, double a, double 
 template <bool TA, bool TB>
 __global__ void __launch_bounds__(256) gemm_f64_kernel(GemmArgs g) {
   __shared__ double sa[kGK][kGP], sb[kGK][kGP];
-  const int m0 = blockIdx.y * kGT, n0 = blockIdx.x * kGT;
+  const unsigned tiles_n = (unsigned)ceil_div(g.N, kGT);
+  const int m0 = (int)(blockIdx.x / tiles_n) * kGT, n0 = (int)(blockIdx.x % tiles_n) * kGT;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int wm = warp >> 1, wn = warp & 1;
   const int gq = lane >> 2, t = lane & 3;
@@ -112,7 +115,9 @@ __global__ void __launch_bounds__(256) gemm_f64_kernel(GemmArgs g) {
 
 int gemm_f64(const GemmArgs& g, bool ta, bool tb, cudaStream_t stream) {
   if (g.M <= 0 || g.N <= 0 || g.K < 0 || !g.A || !g.B || !g.C) return set_error(VB_ERR_INVALID_ARG, "gemm_f64: bad arguments");
-  const dim3 grid((g.N + kGT - 1) / kGT, (g.M + kGT - 1) / kGT);
+  const int64_t tiles = ceil_div(g.M, kGT) * ceil_div(g.N, kGT);
+  if (tiles > INT32_MAX) return set_error(VB_ERR_UNSUPPORTED, "gemm_f64: more than 2^31 - 1 output tiles");
+  const dim3 grid((unsigned)tiles);
   if (ta && tb) gemm_f64_kernel<true, true><<<grid, 256, 0, stream>>>(g);
   else if (ta) gemm_f64_kernel<true, false><<<grid, 256, 0, stream>>>(g);
   else if (tb) gemm_f64_kernel<false, true><<<grid, 256, 0, stream>>>(g);

@@ -218,7 +218,8 @@ extern "C" int vb_glm_point_f64(const double* X, int64_t ldx, const double* y, i
 //   G       += A^T X_c               vb_gemm_f64 (transposed A)
 // over row chunks (the reference runs the user's numpy log density under autograd: models.py:27-39).  The link kernel
 // is elementwise over the chunk with deterministic column sums: block = 32 columns x 8 row groups, per-block partials,
-// a finishing kernel adds them in block order.
+// a finishing kernel adds them in block order.  The (column block, row block) CTAs are numbered column-fastest on a
+// 1-D grid, so Nc is not capped by gridDim.y's 65535 row blocks.
 // ---------------------------------------------------------------------------------------------------------------
 namespace vb {
 
@@ -228,8 +229,10 @@ __global__ void __launch_bounds__(256) glm_link_kernel(double* __restrict__ A, c
                                                        int link, double* __restrict__ part) {
   __shared__ double red[8][33];
   const int cx = threadIdx.x & 31, rg = threadIdx.x >> 5;
-  const int s = blockIdx.x * 32 + cx;
-  const int64_t r0 = (int64_t)blockIdx.y * kLinkRowsPerBlock;
+  const unsigned ncb = (unsigned)ceil_div(S, 32);
+  const unsigned rb = blockIdx.x / ncb;
+  const int s = (int)(blockIdx.x % ncb) * 32 + cx;
+  const int64_t r0 = (int64_t)rb * kLinkRowsPerBlock;
   const int64_t r1 = r0 + kLinkRowsPerBlock < Nc ? r0 + kLinkRowsPerBlock : Nc;
   double acc = 0.0;
   if (s < S) {
@@ -248,7 +251,7 @@ __global__ void __launch_bounds__(256) glm_link_kernel(double* __restrict__ A, c
     double t = 0.0;
 #pragma unroll
     for (int g = 0; g < 8; ++g) t += red[g][cx];
-    part[(size_t)blockIdx.y * S + s] = t;
+    part[(size_t)rb * S + s] = t;
   }
 }
 
@@ -273,11 +276,13 @@ extern "C" int vb_glm_link_f64(double* A, const double* y, int64_t Nc, int S, in
   if (!A || !y || !ll_accum || Nc <= 0 || S <= 0) return set_error(VB_ERR_INVALID_ARG, "glm_link: bad arguments");
   if (link != VB_LINK_LOGISTIC && link != VB_LINK_PROBIT) return set_error(VB_ERR_UNSUPPORTED, "glm_link: logistic or probit");
   if (!workspace || workspace_bytes < vb_glm_link_workspace_bytes(Nc, S)) return set_error(VB_ERR_WORKSPACE, "glm_link: workspace too small");
-  const int nblk = (int)((Nc + kLinkRowsPerBlock - 1) / kLinkRowsPerBlock);
+  const int64_t nblk = ceil_div(Nc, kLinkRowsPerBlock);
+  const int64_t ctas = ceil_div(S, 32) * nblk;
+  if (ctas > INT32_MAX) return set_error(VB_ERR_UNSUPPORTED, "glm_link: more than 2^31 - 1 (column, row) blocks");
   double* part = static_cast<double*>(workspace);
-  glm_link_kernel<<<dim3((S + 31) / 32, nblk), 256, 0, stream>>>(A, y, Nc, S, link, part);
+  glm_link_kernel<<<(unsigned)ctas, 256, 0, stream>>>(A, y, Nc, S, link, part);
   VB_CHECK_LAUNCH();
-  glm_link_finish_kernel<<<(S + 127) / 128, 128, 0, stream>>>(part, nblk, S, ll_accum);
+  glm_link_finish_kernel<<<(S + 127) / 128, 128, 0, stream>>>(part, (int)nblk, S, ll_accum);
   VB_CHECK_LAUNCH();
   return VB_OK;
 }

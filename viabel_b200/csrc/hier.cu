@@ -8,7 +8,8 @@
 // group (rows goff[g] .. goff[g+1]-1 belong to group g) and the likelihood is a GROUPED contraction: one CTA per
 // (group, 128 samples) stages the group's rows in shared memory, each thread owns one sample and keeps its p
 // coefficients and p gradient accumulators in registers -- 4 N p S flops instead of the 4 N (G p) S of a
-// block-expanded dense design matrix.  p <= 32.
+// block-expanded dense design matrix.  p <= 32.  The (group, sample tile) CTAs are numbered group-fastest on a 1-D
+// grid, so S is not capped by gridDim.y's 65535.
 #include "common.cuh"
 
 namespace vb {
@@ -21,8 +22,8 @@ __global__ void __launch_bounds__(kHierThreads) hier_lik_kernel(const double* __
                                                                 double* __restrict__ ssr_part, double* __restrict__ grad) {
   __shared__ double xs[kHierRows][kHierP + 1];
   __shared__ double ys[kHierRows];
-  const int g = blockIdx.x;
-  const int s = blockIdx.y * kHierThreads + threadIdx.x;
+  const int g = (int)(blockIdx.x % (unsigned)G);
+  const int s = (int)(blockIdx.x / (unsigned)G) * kHierThreads + threadIdx.x;
   const bool active = s < S;
   double beta[kHierP], acc[kHierP];
 #pragma unroll
@@ -128,7 +129,9 @@ extern "C" int vb_hier_logp_grad_f64(const double* X, const double* y, const int
   if (!workspace || workspace_bytes < vb_hier_workspace_bytes(G, S)) return set_error(VB_ERR_WORKSPACE, "hier_logp_grad: workspace too small");
   const int D = G * p + p + 2;
   double* ssr_part = static_cast<double*>(workspace);
-  hier_lik_kernel<<<dim3(G, (S + kHierThreads - 1) / kHierThreads), kHierThreads, 0, stream>>>(
+  const int64_t ctas = (int64_t)G * ceil_div(S, kHierThreads);
+  if (ctas > INT32_MAX) return set_error(VB_ERR_UNSUPPORTED, "hier_logp_grad: more than 2^31 - 1 (group, sample tile) pairs");
+  hier_lik_kernel<<<(unsigned)ctas, kHierThreads, 0, stream>>>(
       X, y, reinterpret_cast<const long long*>(goff), p, G, D, theta, S, out_grad != nullptr, ssr_part, out_grad);
   VB_CHECK_LAUNCH();
   hier_finish_kernel<<<S, 256, 0, stream>>>(theta, S, p, G, D, (long long)N, ssr_part, out_grad != nullptr, out_lp, out_grad);

@@ -39,22 +39,23 @@ __global__ void __launch_bounds__(256) mvt_logdiag_kernel(const double* __restri
   if (threadIdx.x == 0) out[0] = a;
 }
 
-// inv_u[s] = 1 / sqrt(chi2_s / df);  zu2[s] = |z_s / u_s|^2   (one warp per sample)
+// inv_u[s] = 1 / sqrt(chi2_s / df);  zu2[s] = |z_s / u_s|^2   (one warp per sample, grid-stride over samples)
 __global__ void __launch_bounds__(256) mvt_rows_kernel(const double* __restrict__ z, const double* __restrict__ chi2, double df,
                                                        int S, int d, double* __restrict__ inv_u, double* __restrict__ zu2) {
   const int lane = threadIdx.x & 31;
-  const int s = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
-  if (s >= S) return;
-  const double iu = 1.0 / sqrt(chi2[s] / df);
-  double a = 0.0;
-  for (int j = lane; j < d; j += 32) {
-    const double v = z[(size_t)s * d + j] * iu;
-    a += v * v;
-  }
-  a = warp_sum(a);
-  if (lane == 0) {
-    inv_u[s] = iu;
-    zu2[s] = a;
+  const int64_t nwarps = (int64_t)gridDim.x * (blockDim.x >> 5);
+  for (int64_t s = (blockIdx.x * (int64_t)blockDim.x + threadIdx.x) >> 5; s < S; s += nwarps) {
+    const double iu = 1.0 / sqrt(chi2[s] / df);
+    double a = 0.0;
+    for (int j = lane; j < d; j += 32) {
+      const double v = z[s * d + j] * iu;
+      a += v * v;
+    }
+    a = warp_sum(a);
+    if (lane == 0) {
+      inv_u[s] = iu;
+      zu2[s] = a;
+    }
   }
 }
 
@@ -181,7 +182,8 @@ __global__ void __launch_bounds__(256) mvt_sumlog_kernel(const double* __restric
 }
 
 int mvt_rows(const double* z, const double* chi2, double df, int S, int d, double* inv_u, double* zu2, cudaStream_t stream) {
-  mvt_rows_kernel<<<(S * 32 + 255) / 256, 256, 0, stream>>>(z, chi2, df, S, d, inv_u, zu2);
+  const int64_t blocks = ceil_div(S, 256 / 32), cap = 64LL * sm_count();
+  mvt_rows_kernel<<<(unsigned)(blocks < cap ? blocks : cap), 256, 0, stream>>>(z, chi2, df, S, d, inv_u, zu2);
   VB_CHECK_LAUNCH();
   return VB_OK;
 }

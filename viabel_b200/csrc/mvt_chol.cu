@@ -36,7 +36,8 @@ __device__ __forceinline__ int64_t tri(int64_t i) { return i * (i + 1) / 2; }
 // Column block b of theta needs the K range [0, 64 (b + 1)): its work grows with b.  CTA (p, r) computes rows
 // [32 r, 32 r + 32) of column blocks p and nb - 1 - p, so every CTA does nb + 1 slabs of 64 -- at S = 256, d = 2048 that
 // is 8 x 16 = 128 equal CTAs, one wave on 148 SMs.  8 warps, each a 16 x 16 fragment of the 32 x 64 tile; the next
-// slab is loaded into registers while the current one is multiplied.
+// slab is loaded into registers while the current one is multiplied.  The CTAs are numbered p-fastest on a 1-D grid
+// (gridDim.y would cap S at 65535 row tiles).
 struct TrmmStage {
   double a[kSlab * kTM / 256];               // Z[s, k]
   double b[kSlab * kTN / 256];               // L[n, k]
@@ -76,11 +77,13 @@ __global__ void __launch_bounds__(256) mvt_chol_trmm_kernel(const double* __rest
                                                             double* __restrict__ theta) {
   __shared__ double sa[kSlab][kPadM], sb[kSlab][kPadN];
   const int nb = (d + kTN - 1) / kTN;
-  const int m0 = blockIdx.y * kTM;
+  const unsigned npairs = (unsigned)(nb + 1) / 2;
+  const int pair = (int)(blockIdx.x % npairs);
+  const int m0 = (int)(blockIdx.x / npairs) * kTM;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int wm = warp >> 2, wn = warp & 3;
   const int gq = lane >> 2, t = lane & 3;
-  const int cb0 = blockIdx.x, cb1 = nb - 1 - (int)blockIdx.x;
+  const int cb0 = pair, cb1 = nb - 1 - pair;
   // flattened (column block, slab) sequence; column block c takes ceil(min(d, 64 (c+1)) / 32) slabs
   const int ns0 = (min(d, (cb0 + 1) * kTN) + kSlab - 1) / kSlab;
   const int total = ns0 + (cb1 == cb0 ? 0 : (min(d, (cb1 + 1) * kTN) + kSlab - 1) / kSlab);
@@ -249,9 +252,10 @@ extern "C" int vb_mvt_chol_transform_f64(const double* var_param, const double* 
   if (!(df > 2.0)) return set_error(VB_ERR_INVALID_ARG, "df must be greater than 2");
   int rc = mvt_rows(z, chi2, df, S, d, inv_u, zu2, stream);
   if (rc) return rc;
-  const int nb = (d + kTN - 1) / kTN;
-  const dim3 grid((nb + 1) / 2, (S + kTM - 1) / kTM);
-  mvt_chol_trmm_kernel<<<grid, 256, 0, stream>>>(var_param, z, inv_u, S, d, theta);
+  const int64_t nb = ceil_div(d, kTN);
+  const int64_t ctas = (nb + 1) / 2 * ceil_div(S, kTM);
+  if (ctas > INT32_MAX) return set_error(VB_ERR_UNSUPPORTED, "mvt_chol_transform: more than 2^31 - 1 tiles");
+  mvt_chol_trmm_kernel<<<(unsigned)ctas, 256, 0, stream>>>(var_param, z, inv_u, S, d, theta);
   VB_CHECK_LAUNCH();
   return VB_OK;
 }
