@@ -420,6 +420,23 @@ int vb_mvt_chol_objective_f64(const double* var_param, const double* z, const do
                               double* value, double* grad, void* workspace, size_t workspace_bytes, cudaStream_t stream);
 
 /* ---------------------------------------------------------------------------------------
+ * Streaming log-weights of the full-rank MultivariateT for vi_diagnostics (convenience.py:136-179), never storing
+ * samples[n, d].  For global draw i in [first, first + count) of an n_total-draw call: chi2_i = element offset + i of
+ * the chi-square stream, z_i[j] = element offset + n_total + (n_total & 1) + i*d + j of the normal stream (what
+ * MultivariateT.base_draws(n_total) draws), theta_i = mu + M z_i / u_i, u_i = sqrt(chi2_i / df), with M = L from the
+ * packed triangle of var_param when A == NULL (Cholesky mode) or M = A (d x d row-major, sqrtm mode: A = V diag(sqrt w)
+ * V^T formed by the caller).  log q_i is the closed form in |z_i / u_i|^2; lw[i - first] = log p(theta_i) - log q_i for
+ * target_kind 0 (sum_j N(theta_j; loc_j, scale_j)) or 1 (sum_j t_{target_df}(theta_j; loc_j, scale_j)), -log q_i for
+ * target_kind -1.  theta_out[count, d] (optional) receives theta, so that the caller can add any model's log p.
+ * Deterministic: a slice equals the same draws of a longer call bit for bit.  Workspace does not depend on n.
+ * ------------------------------------------------------------------------------------- */
+size_t vb_mvt_target_log_weights_workspace_bytes(int d);
+int vb_mvt_target_log_weights_f64(const double* var_param, const double* A, int64_t n_total, int64_t first,
+                                  int64_t count, int d, double df, uint64_t seed, uint64_t offset, int target_kind,
+                                  const double* target_loc, const double* target_scale, double target_df, double* lw,
+                                  double* theta_out, void* workspace, size_t workspace_bytes, cudaStream_t stream);
+
+/* ---------------------------------------------------------------------------------------
  * Hierarchical linear regression plugin (BASELINE configs[3]) with per-sample gradients: a grouped contraction
  * (no block-expanded design matrix).  X[N,p], y[N] sorted by group; goff[G+1] device int64 row offsets;
  * theta[S,D], D = G p + p + 2 = [beta (group-major), m, log tau, log sigma]; p <= 32.

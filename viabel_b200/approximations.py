@@ -116,6 +116,11 @@ class _MeanField(ApproximationFamily):
     def _draw(self, n, seed, offset):
         raise NotImplementedError
 
+    def stream_length(self, n_samples):
+        """Philox stream elements that n_samples draws take: n d normals (or t variates), rounded up to even."""
+        n = int(n_samples) * self.dim
+        return n + (n & 1)
+
     def base_draws(self, n_samples, seed=None):
         """Draw (n_samples, dim) base variates on the device.  With seed=None the family's own
         stream advances (like approx._rs); an explicit seed restarts a fresh stream at 0
@@ -123,7 +128,7 @@ class _MeanField(ApproximationFamily):
         n = int(n_samples) * self.dim
         if seed is None:
             out = self._draw(n, self._seed, self._offset)
-            self._offset += n + (n & 1)
+            self._offset += self.stream_length(n_samples)
         else:
             out = self._draw(n, int(seed), 0)
         return out.view(int(n_samples), self.dim)
@@ -359,6 +364,13 @@ class MultivariateT(ApproximationFamily):
         return theta, inv_u, zu2
 
     # -- base draws: chi-square FIRST, then normals, as the reference (:345-347) -------------------
+    def stream_length(self, n_samples):
+        """Philox stream elements that n_samples draws take: n chi-squares, then n d normals, each run rounded up to
+        even.  Draw i's chi-square is element i and its normals start at element n + (n & 1) + i d, so a draw can be
+        regenerated alone only with the n of the call that drew it."""
+        n, d = int(n_samples), self.dim
+        return n + (n & 1) + n * d + ((n * d) & 1)
+
     def base_draws(self, n_samples, seed=None):
         n, d = int(n_samples), self.dim
         dev = device()
@@ -369,7 +381,7 @@ class MultivariateT(ApproximationFamily):
         off2 = off + n + (n & 1)
         _lib.check(_lib.lib.vb_philox_normal_f64(_lib.ptr(z), n * d, s, off2, 0, _lib.stream()))
         if seed is None:
-            self._offset = off2 + n * d + ((n * d) & 1)
+            self._offset = off + self.stream_length(n)
         return chi2, z.view(n, d)
 
     def sample(self, var_param, n_samples, seed=None, base=None):

@@ -24,14 +24,6 @@ constexpr int kTN = 64;                      // output tile width (columns of th
 constexpr int kTM = 32;                      // transform: rows (samples) per tile
 constexpr int kPadM = kTM + 4, kPadN = kTN + 4;   // row pitches; conflict-free fragment reads
 
-__device__ __forceinline__ void dmma(double& c0, double& c1, double a, double b) {
-  asm volatile("mma.sync.aligned.m8n8k4.row.col.f64.f64.f64.f64 {%0,%1}, {%2}, {%3}, {%0,%1};\n"
-               : "+d"(c0), "+d"(c1)
-               : "d"(a), "d"(b));
-}
-
-__device__ __forceinline__ int64_t tri(int64_t i) { return i * (i + 1) / 2; }
-
 // ---- triangular transform ------------------------------------------------------------------------------------------
 // Column block b of theta needs the K range [0, 64 (b + 1)): its work grows with b.  CTA (p, r) computes rows
 // [32 r, 32 r + 32) of column blocks p and nb - 1 - p, so every CTA does nb + 1 slabs of 64 -- at S = 256, d = 2048 that

@@ -11,6 +11,16 @@ inline double mvt_const(double df, int d) {
   return lgamma(0.5 * (df + d)) - lgamma(0.5 * df) - 0.5 * d * log(3.14159265358979323846 * df);
 }
 
+// one m8n8k4 float64 MMA (DMMA) on the fragment (c0, c1) += a b
+__device__ __forceinline__ void dmma(double& c0, double& c1, double a, double b) {
+  asm volatile("mma.sync.aligned.m8n8k4.row.col.f64.f64.f64.f64 {%0,%1}, {%2}, {%3}, {%0,%1};\n"
+               : "+d"(c0), "+d"(c1)
+               : "d"(a), "d"(b));
+}
+
+// offset of row i of a packed row-major lower triangle
+__host__ __device__ __forceinline__ int64_t tri(int64_t i) { return i * (i + 1) / 2; }
+
 // inv_u[s] = 1 / sqrt(chi2_s / df),  zu2[s] = |z_s / u_s|^2
 int mvt_rows(const double* z, const double* chi2, double df, int S, int d, double* inv_u, double* zu2, cudaStream_t stream);
 
