@@ -108,7 +108,8 @@ int vb_glm_sweep_f64(const double* X, int64_t ldx, const double* y, int64_t N, i
  *   aligned device memory of vb_glm_fast_model_bytes(N,d) bytes, owned by the caller and kept
  *   alive for the lifetime of the handle): y*X split into fp16 hi and lo, zero padded.
  *   absmax_host (optional, HOST pointer) receives max|y*X|; values above 3e4 do not fit the
- *   fp16 operand range and are rejected with VB_ERR_UNSUPPORTED (use the float64 path).
+ *   fp16 operand range and are rejected with VB_ERR_UNSUPPORTED (use the float64 path), as is
+ *   a NaN or infinite entry.
  * vb_glm_fast_sweep: S <= 256 samples per call.  want_grad bit 0: gradients wanted; bit 1: only
  *   sum_s ll[s] is needed (every out_ll[s] then receives the mean, plain ExclusiveKL).  `debug`
  *   (optional, device, 49152 floats per CTA + 128 int64) receives per-phase clock64 timestamps of

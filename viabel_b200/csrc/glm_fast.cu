@@ -526,7 +526,7 @@ glm_fast_kernel(const __grid_constant__ CUtensorMap tmXh, const __grid_constant_
             const float l1p = __log2f(den) * 0.6931471805599453f;
             const float sp = (fmaxf(-a, 0.0f) + l1p) * rowvalid;           // softplus(-a)
             v[i + u] = sp;
-            spsum += sp;
+            spsum += col0 + i + u < p.S ? sp : 0.0f;                       // the total counts valid samples only
             const float sg = __fdividef(a >= 0.0f ? t : 1.0f, den);        // sigmoid(-a)
             r2[u] = sg * misc->w[col0 + i + u] * rowvalid;
             rsum += r2[u];
@@ -640,13 +640,8 @@ glm_fast_kernel(const __grid_constant__ CUtensorMap tmXh, const __grid_constant_
       epi_barrier();
       double s = 0.0;
       for (int i = 0; i < kEpiWarps; ++i) s += red[0][i];
-      // padded sample columns (theta = 0) each contributed softplus(0) = ln2 (as computed in fp32) per valid row
-      int64_t rows = 0;
-      for (int tile = blockIdx.x; tile < p.numTiles; tile += gridDim.x) {
-        const int64_t left = p.N - (int64_t)tile * kBM;
-        rows += left <= 0 ? 0 : (left < kBM ? left : kBM);
-      }
-      s -= (double)(kSP - p.S) * (double)rows * (double)(1.0f * 0.6931471805599453f);
+      // (padded sample columns are masked out of spsum: subtracting their ln 2 afterwards would leave the fp32
+      // rounding of (256 - S) ln 2 per row in the total)
       p.ll_part[(size_t)blockIdx.x * kSP + (threadIdx.x - 64)] = s / (double)p.S;
     } else {
       // lane l of (q,h) holds column 128h + 32c + l summed over rows of quarter q -> sum the 4 quarters
@@ -712,7 +707,7 @@ struct MiscP {
   uint64_t t_empty;                   // leader, count 2
   uint32_t tmem_base;
   uint32_t pad;
-  alignas(16) float rbar[kBM];        // E1 column-half 1 partial row sums
+  alignas(16) float rbar[kBM];        // E1: row sums of R over sample quarter 1 (fixed-order sum, see E1)
   alignas(16) float rb[2][2 * kBM];   // [iteration parity][row of the super-tile]: sum_s R[n,s]
 };
 static_assert(sizeof(MiscP) <= kMiscBytes, "misc smem overflow");
@@ -1187,18 +1182,25 @@ glm_fast_pair_kernel(const __grid_constant__ CUtensorMap tmX,      // 5-D: [hi|l
       ll_acc[1] += (double)lls1;
       if (tthread && it < 8) p.tim[it * 16 + 6] = clock64();
       float* rbl = &misc->rb[it & 1][128 * rank + row];
-      if (grad && k == 0) *rbl = rsum;             // row sums of R: quarter 0 stores, the others add
       fence_proxy_async();       // R tile writes -> visible to the tensor core (async proxy)
       tc_fence_before();
       epi1_barrier();
       // Z has been read and R written by this CTA: the leader may start the next GEMM1 (critical path) ...
       if (threadIdx.x == 64) mbar_arrive_cluster(r_full_leader);
       if (tthread && it < 8) p.tim[it * 16 + 7] = clock64();
-      // ... while the row sums go into BOTH CTAs' rb (E2 of either CTA sweeps all 256 rows; needed later)
+      // ... while the row sums go into BOTH CTAs' rb (E2 of either CTA sweeps all 256 rows; needed later).
+      // Row sums of R over the four sample quarters in a fixed order, so that a sweep is reproducible bit for bit.
+      // Scratch for the partials of quarters 1..3: rbar and the other parity of rb.  Nothing reads that parity before
+      // E2 of super-tile it + 1, and the peer writes it only after its E2 of super-tile it, which waits for rb_full below.
       if (grad) {
-        if (k != 0) atomicAdd(rbl, rsum);
+        float* other = misc->rb[(it + 1) & 1];
+        if (k != 0) (k == 1 ? misc->rbar : other + 128 * (k - 2))[row] = rsum;
         epi1_barrier();
-        if (k == 0) st_cluster_f32(mapa_u32(smem_u32(rbl), rank ^ 1), *rbl);
+        if (k == 0) {
+          const float s = ((rsum + misc->rbar[row]) + other[row]) + other[128 + row];
+          *rbl = s;
+          st_cluster_f32(mapa_u32(smem_u32(rbl), rank ^ 1), s);
+        }
         epi1_barrier();          // CTA-scope ordering of the stores before the (cumulative) cluster-scope release below
         if (threadIdx.x == 64) {
           mbar_arrive_cluster(rbf_own);
@@ -1289,7 +1291,7 @@ __global__ void fast_prepare_x_kernel(const double* __restrict__ X, int64_t ldx,
       float v = 0.0f;
       if (n < N && j < d) v = (float)(X[n * ldx + j] * y[n]);
       tile[r][tx] = v;
-      mx = fmaxf(mx, fabsf(v));
+      mx = fmaxf(mx, v == v ? fabsf(v) : INFINITY);      // NaN counts as out of range (fmaxf would drop it)
       sq += (double)v * (double)v;
     }
     __syncthreads();
@@ -1528,9 +1530,9 @@ extern "C" int vb_glm_fast_create(void** handle, const double* X, int64_t ldx, c
     if (e != cudaSuccess) { delete m; return set_cuda_error(e); }
     amax = stats[0];
     if (absmax_host) *absmax_host = amax;
-    if (absmax_host && !(amax < 3.0e4f)) {
+    if (!(amax < 3.0e4f)) {             // also a NaN or infinite entry of y*X
       delete m;
-      return set_error(VB_ERR_UNSUPPORTED, "glm_fast: |y*X| exceeds the fp16 operand range; use the float64 path");
+      return set_error(VB_ERR_UNSUPPORTED, "glm_fast: |y*X| exceeds the fp16 operand range or is not finite; use the float64 path");
     }
   }
   {
@@ -1629,12 +1631,17 @@ int fast_launch(void* handle, void* workspace, size_t workspace_bytes, int S, in
   fast_layout(m->N, m->d_pad, L);
   char* ws = static_cast<char*>(workspace);
 
+  // The maps are keyed on everything they encode: the workspace address, d_pad and the T8 address.  T8 follows the
+  // per-CTA partial sums, so its offset also depends on the grid, i.e. on N: two models with the same d_pad that
+  // share a workspace address place their e5m2 Theta copies at different offsets.
   static thread_local const void* cached_ws = nullptr;
+  static thread_local const void* cached_t8 = nullptr;
   static thread_local int cached_dpad = 0;
   static thread_local CUtensorMap tmTh, tmTl, tmE, tmTP, tmEP, tmTP16, tmTP8;
   // VB_FAST_FP8=0 selects the three-fp16-pass GEMM1 (A/B measurements)
   static const bool use_fp8 = [] { const char* e = getenv("VB_FAST_FP8"); return !(e && e[0] == '0'); }();
-  if (cached_ws != workspace || cached_dpad != m->d_pad) {
+  if (cached_ws != workspace || cached_dpad != m->d_pad || cached_t8 != ops.T8) {
+    cached_ws = nullptr;           // a failed encode below leaves no valid entry behind
     const uint64_t dp = (uint64_t)m->d_pad;
     const uint64_t td[4] = {64, dp, 4, 2}, ts[3] = {128, dp * 128, dp * 512};      // Tl follows Th
     const uint32_t tb[4] = {64, 32, 2, 2};
@@ -1654,6 +1661,7 @@ int fast_launch(void* handle, void* workspace, size_t workspace_bytes, int S, in
         !encode_nd(&tmTP8, ops.T8, 4, t8d, t8s, t8b, CU_TENSOR_MAP_DATA_TYPE_UINT8))
       return set_error(VB_ERR_CUDA, "glm_fast_sweep: cuTensorMapEncodeTiled failed (fp8 operands)");
     cached_ws = workspace;
+    cached_t8 = ops.T8;
     cached_dpad = m->d_pad;
   }
 
