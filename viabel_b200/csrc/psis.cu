@@ -13,8 +13,11 @@
 //   pass B (1 read, 1 write): out = x - max - lse, tail entries replaced by their smoothed values,
 //                             and sum(out), sum exp(2 out) for the CUBO / ELBO bounds.
 // Algorithmic traffic: 24 bytes per draw.  If the sample-based threshold fails (candidate buffer
-// overflow or fewer than M+1 candidates -- only possible for adversarial input) status=1 is
-// reported and the caller re-runs in exact mode, which finds the cutoff with full radix passes.
+// overflow or fewer than M+1 candidates) status=1 is reported and the caller re-runs in exact mode,
+// which finds the cutoff with full radix passes.  Ordinary inputs do reach it: on draws sorted either
+// way the 16-CTA select's group maxima (16 consecutive sample entries) are correlated, so n = 1e6
+// sorted overflows (118 733 candidates, capacity 95 321) and n = 3e4 sorted descending finds too few;
+// so do inputs periodic with the sample stride (tests/_psis_ref.py predicts each case).
 #include <float.h>
 
 #include <mutex>
@@ -1472,8 +1475,11 @@ __global__ void __launch_bounds__(256) psis_tail_scatter_kernel(double* __restri
     sv = block_sum(sv, red);
     se = block_sum(se, red);
     if (threadIdx.x == 0) {
-      result[R_SUMV] = sv + (add_tail ? sc->sumv : 0.0);           // sharded: rank 0 alone carries the tail's share
-      result[R_SUMEXP2V] = se + (add_tail ? sc->sumexp2v : 0.0);
+      sv += add_tail ? sc->sumv : 0.0;                             // sharded: rank 0 alone carries the tail's share
+      result[R_SUMV] = sv;
+      // v <= 0 or NaN, so sum v is NaN exactly when some v is; exp_nonpos flushes a NaN with the sign bit set (the
+      // v = inf - inf of a +inf draw) to 0, and the reference's sum exp(2 v) is NaN then
+      result[R_SUMEXP2V] = sv != sv ? sv : se + (add_tail ? sc->sumexp2v : 0.0);
     }
   }
 }
