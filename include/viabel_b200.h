@@ -438,6 +438,24 @@ int vb_mvt_target_log_weights_f64(const double* var_param, const double* A, int6
                                   double* theta_out, void* workspace, size_t workspace_bytes, cudaStream_t stream);
 
 /* ---------------------------------------------------------------------------------------
+ * Streaming log-weights of the low-rank LRGaussian (Sigma = B B^T + D^2, D = diag(exp(log_sigma)), var_param =
+ * [mu(d), log_sigma(d), B(d,k) row-major]) for vi_diagnostics, never storing samples[n, d].  For global draw i in
+ * [first, first + count) of an n_total-draw call: z_i[l] = element offset + i*k + l and eps_i[j] = element
+ * offset + n_total*k + ((n_total*k) & 1) + i*d + j of the normal stream (what LRGaussian.base_draws(n_total) draws),
+ * theta_i = mu + B z_i + sigma * eps_i.  With u_i = [z_i, eps_i], log q_i = -1/2 (d log 2 pi + |u_i|^2 - |P u_i|^2)
+ * - sum_j log sigma_j + sum_l log P_ll, where P (k x (k+d) row-major, formed by the caller) = [C^-1 | -C^-1 B^T D^-1]
+ * and C C^T = I + B^T D^-2 B.  P's left k x k block must be the lower-triangular C^-1 with a positive diagonal: half
+ * the log-determinant is read from that diagonal.  P may be NULL when k = 0.  lw and theta_out as in
+ * vb_mvt_target_log_weights_f64.  Deterministic: a slice equals the same draws of a longer call bit for bit.
+ * Workspace does not depend on n.
+ * ------------------------------------------------------------------------------------- */
+size_t vb_lr_target_log_weights_workspace_bytes(int d, int k);
+int vb_lr_target_log_weights_f64(const double* var_param, const double* P, int64_t n_total, int64_t first,
+                                 int64_t count, int d, int k, uint64_t seed, uint64_t offset, int target_kind,
+                                 const double* target_loc, const double* target_scale, double target_df, double* lw,
+                                 double* theta_out, void* workspace, size_t workspace_bytes, cudaStream_t stream);
+
+/* ---------------------------------------------------------------------------------------
  * Hierarchical linear regression plugin (BASELINE configs[3]) with per-sample gradients: a grouped contraction
  * (no block-expanded design matrix).  X[N,p], y[N] sorted by group; goff[G+1] device int64 row offsets;
  * theta[S,D], D = G p + p + 2 = [beta (group-major), m, log tau, log sigma]; p <= 32.

@@ -92,6 +92,9 @@ _PROTOS = {
     'vb_mvt_target_log_weights_workspace_bytes': (c_size_t, [c_int]),
     'vb_mvt_target_log_weights_f64': (c_int, [P, P, c_int64, c_int64, c_int64, c_int, c_double, c_uint64, c_uint64, c_int,
                                               P, P, c_double, P, P, P, c_size_t, P]),
+    'vb_lr_target_log_weights_workspace_bytes': (c_size_t, [c_int, c_int]),
+    'vb_lr_target_log_weights_f64': (c_int, [P, P, c_int64, c_int64, c_int64, c_int, c_int, c_uint64, c_uint64, c_int,
+                                             P, P, c_double, P, P, P, c_size_t, P]),
     'vb_hier_workspace_bytes': (c_size_t, [c_int, c_int]),
     'vb_hier_logp_grad_f64': (c_int, [P, P, P, c_int64, c_int, c_int, P, c_int, P, P, P, c_size_t, P]),
     # peer-memory communicator and the fused step (structures: viabel_b200/engine.py)

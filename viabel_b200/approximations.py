@@ -483,6 +483,13 @@ class LRGaussian(ApproximationFamily):
             raise ValueError('var_param has the wrong length')
         return vp[:d], vp[d:2 * d], vp[2 * d:].reshape(d, k)
 
+    def stream_length(self, n_samples):
+        """Philox stream elements that n_samples draws take: n k normals for z, then n d for eps, each run rounded up
+        to even.  Draw i's z starts at element i k and its eps at n k + ((n k) & 1) + i d, so a draw can be
+        regenerated alone only with the n of the call that drew it."""
+        n, d, k = int(n_samples), self.dim, self._k
+        return n * k + ((n * k) & 1) + n * d + ((n * d) & 1)
+
     def base_draws(self, n_samples, seed=None):
         n, d, k = int(n_samples), self.dim, self._k
         s, off = (self._seed, self._offset) if seed is None else (int(seed), 0)
@@ -490,7 +497,7 @@ class LRGaussian(ApproximationFamily):
         off2 = off + n * k + ((n * k) & 1)
         eps = self._normals(n * d, s, off2).view(n, d)
         if seed is None:
-            self._offset = off2 + n * d + ((n * d) & 1)
+            self._offset = off + self.stream_length(n)
         return z, eps
 
     def sample(self, var_param, n_samples, seed=None, base=None):
