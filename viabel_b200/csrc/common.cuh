@@ -123,10 +123,30 @@ __device__ __forceinline__ void link_probit(double a, double& ll, double& dl) {
     ll = log(0.5 * ex) - u * u;
     dl = 0.79788456080286535587989211986876 / ex;               // sqrt(2/pi)/erfcx(u)
   } else {
-    double P = 0.5 * erfc(u);
-    ll = log(P);
-    dl = exp(-0.5 * a * a - 0.5 * kLog2Pi) / P;
+    // a >= 0: Phi(a) = 1 - q with q = Phi(-a) <= 1/2; log1p keeps ll accurate relative to itself as Phi -> 1
+    double q = 0.5 * erfc(-u);
+    ll = log1p(-q);
+    // phi(a) with a^2 = h + l split exactly: exp(-h/2) then the first-order factor of l, so that the exponent's
+    // rounding (u a^2 / 2 absolute) does not reach dl
+    const double h = a * a, l = fma(a, a, -h);
+    dl = exp(-0.5 * h) * (1.0 - 0.5 * l) * 0.39894228040143267793994605993438 / (1.0 - q);
   }
+}
+// -(log Phi)''(a) = r (a + r), r = phi(a) / Phi(a).  For a < -6, r ~ -a and a + r cancels (relative error ~ u a^2); there
+// a + r = 1 / (x + 2 / (x + 3 / (x + ...))), x = -a, the continued fraction of the Mills ratio, whose 24 terms reach
+// full double precision for every x > 6.
+__device__ __forceinline__ double probit_curvature(double a, double r) {
+  if (a >= -6.0) return r * (a + r);
+  const double x = -a;
+  double t = 0.0;
+#pragma unroll
+  for (int k = 24; k >= 2; --k) t = k / (x + t);
+  return r / (x + t);
+}
+// sigmoid(a) sigmoid(-a) = e / (1 + e)^2, e = exp(-|a|): no 1 - sigmoid cancellation for either sign
+__device__ __forceinline__ double logistic_curvature(double a) {
+  const double e = exp(-fabs(a)), inv = 1.0 / (1.0 + e);
+  return e * inv * inv;
 }
 
 }  // namespace vb

@@ -89,6 +89,7 @@ struct SweepArgs {
   double* ll_part;   // [grid][WC*32]
   double* gmu_part;  // [grid][KG*8]
   double* ge_part;   // [grid][KG*8]
+  double* ge_rows;   // [grid][warps][KG*8], per-warp ge rows in global memory when they do not fit on chip (!PRIV)
 };
 
 template <int LINK>
@@ -115,7 +116,11 @@ __device__ __forceinline__ void link_eval(double z, double yv, double auxv, doub
 // the time (profiles/f64_ncu_full_r02.csv: `wait` was the top stall reason).
 // PRIV: every warp accumulates ge into its own shared-memory row (plain read-modify-write) instead of atomicAdd on
 // one shared row -- a double-precision shared atomic is a compare-and-swap loop, and 16 warps spinning on the same
-// 8 addresses per step were ~10 % of the sweep's samples.  Used whenever the rows fit beside the X tile.
+// 8 addresses per step were ~10 % of the sweep's samples.  Used whenever the rows fit beside the X tile.  Otherwise each
+// warp adds into its own row of a global-memory slice (a fire-and-forget RED that stays in L2; one thread per address, so
+// the adds land in program order).  Either way the rows are summed in warp order at the end, and the row sums of R
+// (rbar) also go through per-warp rows summed in warp order: no sum depends on the order in which warps arrive, so the
+// outputs are bitwise reproducible.
 template <int BM, int LINK, int JN, bool PRIV>
 __global__ void __launch_bounds__(32 * (32 / JN), 1) glm_sweep_f64_kernel(SweepArgs a) {
   constexpr int MT = BM / 8;
@@ -127,12 +132,18 @@ __global__ void __launch_bounds__(32 * (32 / JN), 1) glm_sweep_f64_kernel(SweepA
   double* ys = Xs + (size_t)BM * a.P;       // [BM]
   double* rbar = ys + BM;                   // [BM]
   double* gmu_s = rbar + BM;                // [Dp]
-  double* ge_s = gmu_s + Dp;                // [Dp], or [warps][Dp] with PRIV
+  double* ge_s = gmu_s + Dp;                // [warps][Dp] with PRIV; without, the slot holds rbar_w
+  double* rbar_w = PRIV ? ge_s + (size_t)kSweepWarps * Dp : ge_s;   // [warps][BM] per-warp row sums of R
+  double* ge_g = PRIV ? nullptr : a.ge_rows + (size_t)blockIdx.x * kSweepWarps * Dp;
 
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const int g = lane >> 2, t = lane & 3;
 
-  for (int j = tid; j < (PRIV ? 1 + kSweepWarps : 2) * Dp; j += kSweepThreads) gmu_s[j] = 0.0;   // gmu_s and ge_s are adjacent
+  for (int j = tid; j < (PRIV ? 1 + kSweepWarps : 1) * Dp; j += kSweepThreads) gmu_s[j] = 0.0;   // gmu_s and ge_s are adjacent
+  if (!PRIV && a.want_grad) {
+    // ordered before the first RED by the __syncthreads at the top of the first tile
+    for (int j = tid; j < kSweepWarps * Dp; j += kSweepThreads) ge_g[j] = 0.0;
+  }
 
   const int numSuper = (a.WC + kSweepWarps - 1) / kSweepWarps;
   const bool vec_ok = ((a.ldx & 1) == 0) && ((reinterpret_cast<uintptr_t>(a.X) & 15) == 0);
@@ -175,10 +186,7 @@ __global__ void __launch_bounds__(32 * (32 / JN), 1) glm_sweep_f64_kernel(SweepA
           Xs[(size_t)r * a.P + c] = (n < a.N && c < a.d) ? a.X[n * a.ldx + c] : 0.0;
         }
       }
-      if (tid < BM) {
-        ys[tid] = (n0 + tid < a.N) ? a.y[n0 + tid] : 0.0;
-        rbar[tid] = 0.0;
-      }
+      if (tid < BM) ys[tid] = (n0 + tid < a.N) ? a.y[n0 + tid] : 0.0;
       __syncthreads();
 
       double acc[MT][JN][2];
@@ -255,11 +263,18 @@ __global__ void __launch_bounds__(32 * (32 / JN), 1) glm_sweep_f64_kernel(SweepA
             double rs = rsum[i];
             rs += __shfl_xor_sync(0xffffffffu, rs, 1);
             rs += __shfl_xor_sync(0xffffffffu, rs, 2);
-            if (t == 0) atomicAdd(&rbar[8 * i + g], rs);
+            if (t == 0) rbar_w[warp * BM + 8 * i + g] = rs;
           }
         }
       }
       if (a.want_grad) {
+        __syncthreads();   // rbar_w complete
+        if (tid < BM) {
+          const int nact = min(kSweepWarps, a.WC - sc * kSweepWarps);
+          double v = 0.0;
+          for (int w2 = 0; w2 < nact; ++w2) v += rbar_w[w2 * BM + tid];   // fixed order: deterministic
+          rbar[tid] = v;
+        }
         __syncthreads();   // rbar complete
         // ---- gmu[j] += sum_n X[n,j] rbar[n] -------------------------------------------------
         for (int j = tid; j < Dp; j += kSweepThreads) {
@@ -325,8 +340,8 @@ __global__ void __launch_bounds__(32 * (32 / JN), 1) glm_sweep_f64_kernel(SweepA
                 v.y += p1;
                 *q = v;
               } else {
-                atomicAdd(&ge_s[8 * jb + 2 * t], p0);
-                atomicAdd(&ge_s[8 * jb + 2 * t + 1], p1);
+                atomicAdd(&ge_g[(size_t)warp * Dp + 8 * jb + 2 * t], p0);
+                atomicAdd(&ge_g[(size_t)warp * Dp + 8 * jb + 2 * t + 1], p1);
               }
             }
 #pragma unroll
@@ -356,9 +371,13 @@ __global__ void __launch_bounds__(32 * (32 / JN), 1) glm_sweep_f64_kernel(SweepA
   if (a.want_grad) {
     for (int j = tid; j < Dp; j += kSweepThreads) {
       a.gmu_part[(size_t)blockIdx.x * Dp + j] = gmu_s[j];
-      double v = ge_s[j];
+      double v;
       if (PRIV) {
+        v = ge_s[j];
         for (int w2 = 1; w2 < kSweepWarps; ++w2) v += ge_s[(size_t)w2 * Dp + j];      // fixed order: deterministic
+      } else {
+        v = __ldcg(ge_g + j);                                                          // L2: where the REDs landed
+        for (int w2 = 1; w2 < kSweepWarps; ++w2) v += __ldcg(ge_g + (size_t)w2 * Dp + j);
       }
       a.ge_part[(size_t)blockIdx.x * Dp + j] = v;
     }
@@ -380,7 +399,7 @@ struct SweepPlan {
   int BM, KG, P, WC, SB, JN, priv, grid;
   int64_t numTiles;
   size_t smem;
-  size_t off_thetaP, off_baseP, off_wP, off_auxP, off_ll, off_gmu, off_ge, total;
+  size_t off_thetaP, off_baseP, off_wP, off_auxP, off_ll, off_gmu, off_ge, off_ge_rows, total;
 };
 
 static bool make_plan(int64_t N, int d, int64_t S, SweepPlan& p) {
@@ -402,10 +421,16 @@ static bool make_plan(int64_t N, int d, int64_t S, SweepPlan& p) {
     }
   }
   if (p.BM == 0) return false;
-  {   // per-warp ge rows when they fit beside the tile
-    const size_t extra = sizeof(double) * (size_t)(32 / p.JN - 1) * Dp;
+  {   // per-warp ge rows when they fit beside the tile; the per-warp rbar rows after them, or in the unused ge slot
+    const int warps = 32 / p.JN;
+    const size_t extra = sizeof(double) * ((size_t)(warps - 1) * Dp + (size_t)warps * p.BM);
     p.priv = (p.smem + extra <= 227 * 1024) ? 1 : 0;
-    if (p.priv) p.smem += extra;
+    if (p.priv) {
+      p.smem += extra;
+    } else if (warps * p.BM > Dp) {
+      p.smem += sizeof(double) * (size_t)(warps * p.BM - Dp);
+      if (p.smem > 227 * 1024) return false;
+    }
   }
   p.numTiles = ceil_div(N, p.BM);
   int sms = sm_count();
@@ -424,6 +449,7 @@ static bool make_plan(int64_t N, int d, int64_t S, SweepPlan& p) {
   p.off_ll = take((size_t)p.grid * p.SB * 8 * sizeof(double));
   p.off_gmu = take((size_t)p.grid * Dp * sizeof(double));
   p.off_ge = take((size_t)p.grid * Dp * sizeof(double));
+  p.off_ge_rows = take(p.priv ? 0 : (size_t)p.grid * (32 / p.JN) * Dp * sizeof(double));
   p.total = off;
   return true;
 }
@@ -494,6 +520,7 @@ extern "C" int vb_glm_sweep_f64(const double* X, int64_t ldx, const double* y, i
   a.ll_part = reinterpret_cast<double*>(ws + p.off_ll);
   a.gmu_part = reinterpret_cast<double*>(ws + p.off_gmu);
   a.ge_part = reinterpret_cast<double*>(ws + p.off_ge);
+  a.ge_rows = reinterpret_cast<double*>(ws + p.off_ge_rows);
 
   {
     const int64_t total = (int64_t)p.SB * p.KG * 32;

@@ -64,10 +64,10 @@ __global__ void __launch_bounds__(256) glm_point_kernel(const double* __restrict
           double ll, dl;
           if (link == VB_LINK_LOGISTIC) {
             link_logistic(a, ll, dl);
-            c = dl * (1.0 - dl);                       // sigmoid(a) sigmoid(-a)
+            c = logistic_curvature(a);                 // sigmoid(a) sigmoid(-a)
           } else {
             link_probit(a, ll, dl);
-            c = dl * (a + dl);                         // -(log Phi)'' = r (a + r)
+            c = probit_curvature(a, dl);               // -(log Phi)'' = r (a + r)
           }
           ll_acc += ll;
           r = yv * dl;
