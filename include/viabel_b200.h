@@ -113,9 +113,9 @@ int vb_glm_sweep_f64(const double* X, int64_t ldx, const double* y, int64_t N, i
  * vb_glm_fast_sweep: S <= 256 samples per call.  want_grad bit 0: gradients wanted; bit 1: only
  *   sum_s ll[s] is needed (every out_ll[s] then receives the mean, plain ExclusiveKL).  `debug`
  *   (optional, device, 49152 floats per CTA + 128 int64) receives per-phase clock64 timestamps of
- *   CTA 0 (and, with the one-CTA kernel, the raw accumulators of each CTA's first tile).
- *   The default kernel runs CTA pairs (tcgen05 cta_group::2, clusters of 2); the environment
- *   variable VB_FAST_KERNEL=single selects the one-CTA kernel for A/B measurements.
+ *   CTA 0 in its 128 int64 after the floats.
+ *   The kernel runs CTA pairs (tcgen05 cta_group::2, clusters of 2); a device that cannot
+ *   schedule them gets VB_ERR_UNSUPPORTED (use the float64 path).
  * Workspace and model_mem must be 1024-byte aligned.
  * ------------------------------------------------------------------------------------- */
 size_t vb_glm_fast_model_bytes(int64_t N, int d);

@@ -32,12 +32,12 @@ SMEM = 227 * 1024
 
 
 # ---- the sweep's plan (make_plan in glm_f64.cu) ---------------------------------------------------------------------
-def plan(d, jn=2):
+def plan(d):
     """(BM, priv) of the sweep at dimension d, or None where it returns VB_ERR_UNSUPPORTED."""
     KG = -(-d // 8)
     Dp = KG * 8
     P = Dp + 8 if Dp % 16 == 0 else Dp + 16
-    warps = 32 // jn
+    warps = 16
     for bm in (32, 16, 8):
         smem = 8 * (bm * P + 2 * bm + 2 * Dp)
         if smem <= SMEM:

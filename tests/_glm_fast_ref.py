@@ -8,25 +8,23 @@ and, with ll_total_only, the mean over s of ll in every slot.  The reference wal
 (error ~1e-13, far below every budget here).
 
 Error model, per element, from the kernel's numerics (glm_fast.cu):
-  GEMM1  fp16 hi/lo split of fp32-cast operands, two correction products (e5m2 copies in the default CTA-pair kernel,
-         fp16 in the three-pass variants), fp32 accumulation:
+  GEMM1  fp16 hi/lo split of fp32-cast operands, two correction products on e5m2 copies, fp32 accumulation:
              |dz_ns| <= c_z u_d A_ns,  u_d = 2^-20 + (d/16 + 2) 2^-24,  A_ns = sum_j |y_n x_nj theta_sj|
   E1     MUFU ex2 / lg2 / rcp, ~2^-21 relative; fp32 column sums of 32 rows
   R      stored in fp16: 2^-11 relative plus 2^-25 absolute (subnormal range); rsum (gmu) is fp32, not rounded
   E      stored in fp16: exact for fp16-exact draws, 2^-11 relative otherwise
-  E2     x read as X_h + 2^-ax e5m2(X_l 2^ax) (about 2^-14 relative; exactly X_h + X_l in the fp16 variants), fp32 sums
+  E2     x read as X_h + 2^-ax e5m2(X_l 2^ax) (about 2^-14 relative), fp32 sums
 Two bounds per element:
   worst-case  W = W0 + c_z Wz            (must never be exceeded)
   statistical T = bias + k sqrt(var)     (roundings are unbiased: k 2^-12 sqrt(sum (x r e)^2) for R and alike; the
                                           roundings of theta and E are shared by all rows and add up coherently over n;
                                           `bias` allows 2^-20 of the absolute sum for the MUFU approximations)
-c_z and k are calibrated on a B200 (DESIGN.md 2 lists the largest err / bound ratios measured per output and variant).
+c_z and k are calibrated on a B200 (DESIGN.md 2 lists the largest err / bound ratios measured per output).
 """
 import numpy as np
 
-# calibrated constants per kernel variant ('pair' = CTA-pair kernel with e5m2 corrections, the default;
-# 'fp16' = VB_FAST_FP8=0, three fp16 passes; 'single' = VB_FAST_KERNEL=single, the one-CTA kernel, three fp16 passes)
-C_Z = {'pair': 8.0, 'fp16': 4.0, 'single': 4.0}
+# calibrated constants
+C_Z = 8.0
 K_STAT = 8.0
 
 LN2 = float(np.log(2.0))
@@ -89,22 +87,19 @@ def alpha_weights(S, seed):
 class Reference(object):
     """ll / gmu / ge in float64 and the ingredients of both bounds (c_z and k are applied in `bounds`)."""
 
-    def __init__(self, X, y, theta, base, w=None, exact=True, variant='pair', ax=None, chunk=8192):
+    def __init__(self, X, y, theta, base, w=None, exact=True, ax=None, chunk=8192):
         X = np.asarray(X, dtype=np.float64)
         N, d = X.shape
         S = theta.shape[0]
-        self.N, self.d, self.S, self.variant = N, d, S, variant
+        self.N, self.d, self.S = N, d, S
         w = np.ones(S) if w is None else np.asarray(w, dtype=np.float64)
         self.w = w
         e = np.zeros((S, d)) if base is None else np.asarray(base, dtype=np.float64)
         ae, e2 = np.abs(e), e * e
         at, t2 = np.abs(theta), theta * theta
         u_d = 2.0 ** -20 + (d / 16.0 + 2.0) * 2.0 ** -24
-        if variant == 'pair':
-            ax = fp8_scales(X, y)[0] if ax is None else ax
-            u_x, floor_x, u_t = 2.0 ** -14, 2.0 ** (-17 - ax), 2.0 ** -13
-        else:
-            u_x, floor_x, u_t = 2.0 ** -22, 2.0 ** -25, 2.0 ** -21
+        ax = fp8_scales(X, y)[0] if ax is None else ax
+        u_x, floor_x, u_t = 2.0 ** -14, 2.0 ** (-17 - ax), 2.0 ** -13
         u_e = 0.0 if exact else 2.0 ** -11
         self.ll = np.zeros(S)
         self.gmu = np.zeros(d)
@@ -117,7 +112,7 @@ class Reference(object):
         self.Bll, self.Vllz = np.zeros(S), np.zeros(S)
         self.Bgmu, self.Vgmu, self.Vgmuz = np.zeros(d), np.zeros(d), np.zeros(d)
         self.Bge, self.Vge, self.Vgez = np.zeros(d), np.zeros(d), np.zeros(d)
-        # the roundings of theta (u_t: its e5m2 / fp16 low parts) and of E are shared by every row: their effects add up
+        # the roundings of theta (u_t: its e5m2 low part) and of E are shared by every row: their effects add up
         # coherently over n, through these column sums
         Gs, Gd, Gr = np.zeros((S, d)), np.zeros((S, d)), np.zeros((S, d))
         self._data = (X, y, theta, e, w)
@@ -174,22 +169,20 @@ class Reference(object):
         r = w * sigmoid(-z)
         return -softplus(-z), x * r.sum(), x * (r @ e)
 
-    def bounds(self, c_z=None, k=K_STAT):
+    def bounds(self, c_z=C_Z, k=K_STAT):
         """{'ll'|'gmu'|'ge': (worst-case bound, statistical bound)} per element."""
-        c_z = C_Z[self.variant] if c_z is None else c_z
         return {'ll': (self.Wll0 + c_z * self.Wllz, self.Bll + k * np.sqrt(c_z ** 2 * self.Vllz + self.Vllc)),
                 'gmu': (self.Wgmu0 + c_z * self.Wgmuz,
                         self.Bgmu + k * np.sqrt(self.Vgmu + c_z ** 2 * self.Vgmuz + self.Vgmuc)),
                 'ge': (self.Wge0 + c_z * self.Wgez, self.Bge + k * np.sqrt(self.Vge + c_z ** 2 * self.Vgez + self.Vgec))}
 
-    def total_bound(self, c_z=None):
+    def total_bound(self, c_z=C_Z):
         """Budget of S * (the ll_total_only mean) against sum_s ll[s]: the per-sample worst cases plus 2^-19 per
         valid row for the fp32 chunk sums that carry the padded columns' ln 2 (subtracted afterwards)."""
-        c_z = C_Z[self.variant] if c_z is None else c_z
         return float(np.sum(self.Wll0 + c_z * self.Wllz)) + 2.0 ** -19 * self.N * max(1, 256 // 64)
 
 
-def ratios(ref, ll, gmu, ge, c_z=None, k=K_STAT):
+def ratios(ref, ll, gmu, ge, c_z=C_Z, k=K_STAT):
     """Largest err / bound per output: {'ll': (worst, stat), ...}."""
     b = ref.bounds(c_z, k)
     out = {}
@@ -212,8 +205,6 @@ CASES = [
     (1, 2048, 65, False), (256, 31, 1, False), (38017, 1, 64, False), (127, 1000, 192, True), (255, 2048, 2, False),
     (128, 1, 129, False), (18688, 1000, 63, False),
 ]
-# the core subset that also runs with the kernel variants
-VARIANT_CASES = [CASES[i] for i in (0, 3, 4, 8, 9, 10, 12, 15)]
 
 
 def case_seed(N, d, S):
@@ -258,7 +249,7 @@ def mutations(ref):
     return out
 
 
-def detected(ref, dll, dgmu, dge, c_z=None, k=K_STAT):
+def detected(ref, dll, dgmu, dge, c_z=C_Z, k=K_STAT):
     """Largest |change| / statistical bound over every element: > 1 means the element-wise check catches it."""
     b = ref.bounds(c_z, k)
     return max(float(np.max(np.abs(dll) / b['ll'][1])), float(np.max(np.abs(dgmu) / b['gmu'][1])),

@@ -7,14 +7,13 @@ from _glm_f64_ref import (CASES, Reference, alpha_weights, case_links, case_seed
 
 
 def test_plan_regimes():
-    """The mirror of make_plan: X-tile height and per-warp ge rows by d, for 16 warps (default) and 8 (VB_F64_JN=4)."""
+    """The mirror of make_plan: X-tile height and per-warp ge rows by d, for the sweep's 16 warps."""
     want = [(1, 576, 32, True), (577, 832, 32, False), (833, 864, 16, True), (865, 1600, 16, False),
             (1601, 2896, 8, False)]
     for lo, hi, bm, priv in want:
         for d in (lo, hi):
             assert plan(d) == (bm, priv), d
     assert plan(2897) is None
-    assert plan(577, 4) == (32, True) and plan(1601, 4) == (8, True)
 
 
 def test_reference_matches_the_oracle():

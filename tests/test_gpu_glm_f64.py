@@ -2,11 +2,6 @@
 per-element worst-case bounds (tests/_glm_f64_ref.py) at d, S and N around its plan regimes, tiles, super-chunks and
 CTA wave, in every mode; vb_glm_link_f64 and vb_glm_point_f64 against mpmath per element; the Hessian SYRK against
 long double.  Bitwise reproducibility is required wherever the kernels promise fixed-order sums."""
-import json
-import os
-import subprocess
-import sys
-
 import numpy as np
 import pytest
 import torch
@@ -78,10 +73,10 @@ def sweep(X, y, theta, base, link, w=None, aux=None, want_grad=1, ldx=None, xoff
     return rc, o[0][:S], None, None
 
 
-def run_case(N, d, S, links=None, full=True):
+def run_case(N, d, S):
     """Every mode of one shape; returns {link/mode: {output: err / bound}}."""
     res = {}
-    for li, link in enumerate(case_links(N, S) if links is None else links):
+    for li, link in enumerate(case_links(N, S)):
         X, y, theta, base, aux = make_case(N, d, S, link, case_seed(N, d, S))
         ax = aux if link == 'gaussian' else None
         ref = Reference(X, y, theta, base, link, aux=aux)
@@ -97,7 +92,7 @@ def run_case(N, d, S, links=None, full=True):
         rw = sweep(X, y, theta, base, link, w=w, aux=ax)
         assert _eq(rw[1], ll), 'weights change ll'
         res[link + '/weighted'] = ratios(refw, rw[1], rw[2], rw[3])
-        if full and li == 0:
+        if li == 0:
             # NaN-filled workspace (the default fill), repeated; wide and unaligned X: the scalar staging path
             for kw in ({}, {}, {'ldx': d + 1}, {'ldx': d + 8}, {'xoff': 1}, {'ldx': d + 8, 'xoff': 1}):
                 r2 = sweep(X, y, theta, base, link, aux=ax, **kw)
@@ -137,29 +132,6 @@ def test_sweep_edges():
     rows = lambda d: sms * 16 * (-(-d // 8) * 8) * 8
     assert ws(577) - ws(576) >= rows(577) and ws(865) - ws(864) >= rows(865)
     assert ws(864) < ws(832)
-
-
-def _jn4_child():
-    out = {'ws_differs': _L().lib.vb_glm_sweep_workspace_bytes(1000, 64, 15) != int(os.environ['VB_WS_JN2']),
-           'cases': []}
-    for N, d, S in [CASES[i] for i in (3, 13, 16, 21, 25, 29)]:
-        out['cases'].append({'shape': [N, d, S], 'res': run_case(N, d, S, links=('logistic', 'probit'), full=False)})
-    print('JN4-RESULT ' + json.dumps(out))
-
-
-def test_sweep_jn4_variant():
-    """VB_F64_JN=4 (8 warps of 32 samples, read once per process) in a child process, against the same bounds."""
-    here = os.path.dirname(os.path.abspath(__file__))
-    code = ('import sys; sys.path[:0] = [%r, %r]; import test_gpu_glm_f64 as t; t._jn4_child()'
-            % (here, os.path.dirname(here)))
-    cmd = [sys.executable] + (['-s'] if sys.flags.no_user_site else []) + ['-c', code]
-    env = dict(os.environ, VB_F64_JN='4', VB_WS_JN2=str(_L().lib.vb_glm_sweep_workspace_bytes(1000, 64, 15)))
-    p = subprocess.run(cmd, env=env, capture_output=True, text=True, timeout=600)
-    assert p.returncode == 0, p.stdout[-3000:] + p.stderr[-3000:]
-    out = json.loads([ln for ln in p.stdout.splitlines() if ln.startswith('JN4-RESULT ')][-1][len('JN4-RESULT '):])
-    assert out['ws_differs']
-    for c in out['cases']:
-        _check(c['res'], ('JN=4',) + tuple(c['shape']))
 
 
 @pytest.mark.parametrize('d', [512, 1024])

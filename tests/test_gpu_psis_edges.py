@@ -2,11 +2,7 @@
 the sampled run must take the path the host mirror predicts (status, and the exact candidate count on status 0), and
 after the exact-mode fallback every output must match oracle.viabel_oracle.psislw_1d -- maximum and shifted cutoff
 bit-equal, tail set and rank order bit-exact, k-hat, outputs and moments to 1e-10 -- in the two-pass, exact,
-moments-only and unaligned forms, draw-sharded, past 2^31 draws, and with the first version of pass A."""
-import os
-import subprocess
-import sys
-
+moments-only and unaligned forms, draw-sharded (with and without an output array) and past 2^31 draws."""
 import numpy as np
 import pytest
 import torch
@@ -17,7 +13,6 @@ from _problems import psis_case
 pytestmark = pytest.mark.gpu
 TOL = 1e-10
 R_KHAT, R_SIGMA, R_N2, R_CUTOFF, R_LSE, R_MAX, R_STATUS, R_SUMV, R_SUMEXP2V, R_M, R_NCAND, R_SMOOTHED = range(12)
-V1_ENV = {'VB_PSIS_PASS_A': 'v1', 'VB_PSIS_ONEPASS': '0'}
 
 
 @pytest.fixture(scope='module')
@@ -106,7 +101,7 @@ def _run_matrix(psis, key, lw, reff, variants=True):
     _, res3, ti, tr = psis.psislw_device(t, out, reff, True, True)
     res3 = res3.cpu().numpy()
     _check(res3, out.cpu().numpy(), ref, _value_order(ti, tr, int(res3[R_N2])), (key, 'exact'))
-    # k-hat and moments only (one pass over the draws unless VB_PSIS_ONEPASS=0)
+    # k-hat and moments only (one pass over the draws)
     res4, _, _ = _fallback(psis, t, None, reff, False)
     for slot in (R_KHAT, R_SIGMA, R_N2, R_CUTOFF, R_LSE, R_MAX, R_M, R_SMOOTHED):
         a, b = res4[slot], res2[slot]
@@ -128,7 +123,7 @@ def _run_matrix(psis, key, lw, reff, variants=True):
 @pytest.mark.parametrize('name', list(P.NAMED))
 def test_named_cases(psis, name):
     lw = P.named_case(name)
-    _run_matrix(psis, name, lw, 1.0, variants=os.environ.get('VB_PSIS_PASS_A') != 'v1')
+    _run_matrix(psis, name, lw, 1.0)
 
 
 @pytest.mark.parametrize('name,reff', P.reff_cases())
@@ -147,6 +142,8 @@ def test_small_n(psis, kind):
 # ---- draw-sharded: shards driven in one process, the exchange by hand ------------------------------------------------
 def _sharded(psis, x, cuts, reff=1.0):
     """The loop of psislw_sharded: local(sampled), global, apply; every shard reruns exact when any status is 1.
+    Each shard also applies without an output array (pass B moments only), which must give the same moments to
+    1e-12 (its exp(2 v) is a different polynomial form).
     Returns the outputs, the replicated result, the summed moments and the sampled local status of each shard."""
     n, world = x.numel(), len(cuts) - 1
     shards = [psis.PsisShard(x[cuts[r]:cuts[r + 1]], cuts[r], n, reff, world, r) for r in range(world)]
@@ -161,6 +158,10 @@ def _sharded(psis, x, cuts, reff=1.0):
             s.global_(recs)
             o = torch.empty_like(s.lw)
             rr = s.apply(o).cpu().numpy()
+            rm = s.apply(None).cpu().numpy()
+            for slot in range(R_SUMV, R_SUMEXP2V + 1):
+                a, b = rm[slot], rr[slot]
+                assert _same(a, b) or abs(a - b) <= 1e-12 * abs(b), ('apply(None)', slot, a, b)
             mom += rr[R_SUMV:R_SUMEXP2V + 1]
             outs.append(o)
             if res is None:
@@ -255,19 +256,3 @@ def test_more_than_2pow31_draws(psis):
     out[cut:] = outs[1]
     del outs
     check_out(res, out, ('2^31', 'sharded'))
-
-
-# ---- the first version of pass A and the two-pass moments, selected per process --------------------------------------
-def test_pass_a_v1_child():
-    """psis_pass_a_kernel + psis_cand_hist_kernel (VB_PSIS_PASS_A=v1) and the two-pass k-hat-only form
-    (VB_PSIS_ONEPASS=0) are chosen once per process: a child runs the named-case matrix with both set."""
-    if os.environ.get('VB_PSIS_PASS_A') == 'v1':
-        pytest.skip('already the child')
-    here = os.path.dirname(os.path.abspath(__file__))
-    cmd = [sys.executable] + (['-s'] if sys.flags.no_user_site else []) + [
-        '-m', 'pytest', '-q', '-p', 'no:cacheprovider', '-m', 'gpu', os.path.join(here, 'test_gpu_psis_edges.py'),
-        '-k', 'test_named_cases']
-    p = subprocess.run(cmd, env=dict(os.environ, **V1_ENV), capture_output=True, text=True, timeout=900,
-                       cwd=os.path.dirname(here))
-    assert p.returncode == 0, p.stdout[-4000:] + p.stderr[-2000:]
-    assert ('%d passed' % len(P.NAMED)) in p.stdout, p.stdout[-2000:]

@@ -41,7 +41,7 @@ if len(sys.argv) > 1 and sys.argv[1] == 'time':
             m.sweep(th, bs, None, True, ll_total_only=tot)
         e1.record(); torch.cuda.synchronize()
         ms = e0.elapsed_time(e1) / 20
-        print('C2 sweep ll_total_only=%d %.4f ms  %.1f TFLOP/s algorithmic  (VB_FAST_KERNEL=%s)' % (tot, ms, 4.0 * N * d * S / ms / 1e9, os.environ.get('VB_FAST_KERNEL', 'pair')))
+        print('C2 sweep ll_total_only=%d %.4f ms  %.1f TFLOP/s algorithmic' % (tot, ms, 4.0 * N * d * S / ms / 1e9))
 else:
     for c in [(128, 128, 64), (128, 128, 64), (1003, 13, 7), (300, 256, 256), (257, 1024, 256), (5, 2048, 3), (40000, 64, 256), (100000, 512, 256)]:
         case(*c)

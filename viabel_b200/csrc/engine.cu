@@ -246,34 +246,30 @@ __global__ void __launch_bounds__(256) mf_pre_kernel(StepCfg c, StepPtrs p, fast
   }
   if (!c.fast) return;
   __syncthreads();
-  {   // Theta^T hi / lo: column jj of the tile, 4 consecutive samples per thread -> 8-byte stores, 32-byte runs
+  {   // Theta^T hi: column jj of the tile, 4 consecutive samples per thread -> 8-byte stores, 32-byte runs
     const int jj = threadIdx.x >> 2, q4 = (threadIdx.x & 3) * 4;
     __align__(8) __half hi[4];
-    __align__(8) __half lo[4];
-    float lof[4];                      // residual in fp32: the e5m2 copy must not inherit an fp16 underflow of lo
+    float lof[4];                      // residual in fp32: the e5m2 copy must not inherit an fp16 underflow
 #pragma unroll
     for (int u = 0; u < 4; ++u) {
       const float t = tt[jj][q4 + u];
       hi[u] = __float2half_rn(t);
       lof[u] = t - __half2float(hi[u]);
-      lo[u] = __float2half_rn(lof[u]);
     }
     const int sg = s0 + q4;                                     // 16 | 64: the 4 samples stay inside one 64-group
     const size_t o = ((size_t)(sg >> 6) * c.d_pad + (j0 + jj)) * 64 + (sg & 63);
     *reinterpret_cast<uint2*>(ops.Th + o) = *reinterpret_cast<const uint2*>(hi);
-    *reinterpret_cast<uint2*>(ops.Tl + o) = *reinterpret_cast<const uint2*>(lo);
-    if (ops.T8) {      // e5m2 copies for the fp8 correction passes: Theta_h * 2^-ax and Theta_l * 2^bx, 128-sample groups
-      const float sh = exp2f((float)-ops.ax), sl = exp2f((float)ops.bx);
-      uint32_t h8 = 0, l8 = 0;
+    // e5m2 copies for the fp8 correction passes: Theta_h * 2^-ax and Theta_l * 2^bx, 128-sample groups
+    const float sh = exp2f((float)-ops.ax), sl = exp2f((float)ops.bx);
+    uint32_t h8 = 0, l8 = 0;
 #pragma unroll
-      for (int u = 0; u < 4; ++u) {
-        h8 |= (uint32_t)fast::to_e5m2(__half2float(hi[u]) * sh) << (8 * u);
-        l8 |= (uint32_t)fast::to_e5m2(lof[u] * sl) << (8 * u);
-      }
-      const size_t o8 = ((size_t)(sg >> 7) * c.d_pad + (j0 + jj)) * 128 + (sg & 127);
-      *reinterpret_cast<uint32_t*>(ops.T8 + o8) = h8;
-      *reinterpret_cast<uint32_t*>(ops.T8 + (size_t)2 * c.d_pad * 128 + o8) = l8;
+    for (int u = 0; u < 4; ++u) {
+      h8 |= (uint32_t)fast::to_e5m2(__half2float(hi[u]) * sh) << (8 * u);
+      l8 |= (uint32_t)fast::to_e5m2(lof[u] * sl) << (8 * u);
     }
+    const size_t o8 = ((size_t)(sg >> 7) * c.d_pad + (j0 + jj)) * 128 + (sg & 127);
+    *reinterpret_cast<uint32_t*>(ops.T8 + o8) = h8;
+    *reinterpret_cast<uint32_t*>(ops.T8 + (size_t)2 * c.d_pad * 128 + o8) = l8;
   }
   if (blockIdx.x == 0 && blockIdx.y == 0) ops.wf[threadIdx.x] = (int)threadIdx.x < c.S ? 1.0f : 0.0f;
 }

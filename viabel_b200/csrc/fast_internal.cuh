@@ -14,10 +14,9 @@ constexpr int kPadS = 256;      // padded sample count of a sweep (= kSP in glm_
 
 struct FastOperands {
   __half* Th;    // Theta^T hi  [4][d_pad][64]
-  __half* Tl;    // Theta^T lo
   __half* E;     // base draws  [d_pad/64][256][64]
   float* wf;     // sample weights [256]
-  // fp8 correction operands (VB_FAST_FP8 scheme): e5m2 copies [2: Theta_h * 2^-ax | Theta_l * 2^bx][2 groups][d_pad][128 s]
+  // fp8 correction operands: e5m2 copies [2: Theta_h * 2^-ax | Theta_l * 2^bx][2 groups][d_pad][128 s]
   uint8_t* T8;
   int ax, bx;    // static power-of-two scales of the model (X_l8 = X_l * 2^ax, X_h8 = X_h * 2^-bx): each pass's operand scales multiply to 1
 };

@@ -81,7 +81,7 @@ struct SweepArgs {
   const double2* baseP;
   const double* wP;
   const double* auxP;
-  int WC;   // number of warp-chunks of 8 * JN samples (S padded to that)
+  int WC;   // number of warp-chunks of 8 * kJN samples (S padded to that)
   int KG;   // ceil(d/8)
   int P;    // shared-memory row pitch of the X tile, in doubles
   int want_grad;
@@ -109,11 +109,11 @@ __device__ __forceinline__ void link_eval(double z, double yv, double auxv, doub
   }
 }
 
-// JN = 8-sample blocks per warp.  JN = 4: 8 warps of 32 samples (the first version); JN = 2: 16 warps of 16 samples --
-// the same operand traffic from L2 (every warp still loads only its own slice of theta / E), twice the shared-memory
-// reads of the X tile (far from a bound), and FOUR warps per scheduler instead of two: with two, a warp's link
-// epilogue, its shuffles and the fixed issue distance between dependent DMMAs left the FP64 tensor pipe idle 39 % of
-// the time (profiles/f64_ncu_full_r02.csv: `wait` was the top stall reason).
+// kJN = 8-sample blocks per warp: 16 warps of 16 samples.  Against 8 warps of 32 samples this is the same operand
+// traffic from L2 (every warp still loads only its own slice of theta / E), twice the shared-memory reads of the X tile
+// (far from a bound), and FOUR warps per scheduler instead of two: with two, a warp's link epilogue, its shuffles and
+// the fixed issue distance between dependent DMMAs left the FP64 tensor pipe idle 39 % of the time
+// (profiles/f64_ncu_full_r02.csv: `wait` was the top stall reason).
 // PRIV: every warp accumulates ge into its own shared-memory row (plain read-modify-write) instead of atomicAdd on
 // one shared row -- a double-precision shared atomic is a compare-and-swap loop, and 16 warps spinning on the same
 // 8 addresses per step were ~10 % of the sweep's samples.  Used whenever the rows fit beside the X tile.  Otherwise each
@@ -121,10 +121,11 @@ __device__ __forceinline__ void link_eval(double z, double yv, double auxv, doub
 // the adds land in program order).  Either way the rows are summed in warp order at the end, and the row sums of R
 // (rbar) also go through per-warp rows summed in warp order: no sum depends on the order in which warps arrive, so the
 // outputs are bitwise reproducible.
-template <int BM, int LINK, int JN, bool PRIV>
-__global__ void __launch_bounds__(32 * (32 / JN), 1) glm_sweep_f64_kernel(SweepArgs a) {
+constexpr int kJN = 2;
+template <int BM, int LINK, bool PRIV>
+__global__ void __launch_bounds__(32 * (32 / kJN), 1) glm_sweep_f64_kernel(SweepArgs a) {
   constexpr int MT = BM / 8;
-  constexpr int kSweepWarps = 32 / JN;
+  constexpr int kSweepWarps = 32 / kJN;
   constexpr int kSweepThreads = 32 * kSweepWarps;
   extern __shared__ __align__(16) double smem[];
   const int Dp = a.KG * 8;
@@ -151,9 +152,9 @@ __global__ void __launch_bounds__(32 * (32 / JN), 1) glm_sweep_f64_kernel(SweepA
   for (int sc = 0; sc < numSuper; ++sc) {
     const int wc = sc * kSweepWarps + warp;
     const bool active = wc < a.WC;
-    double llacc[JN][2];
+    double llacc[kJN][2];
 #pragma unroll
-    for (int jn = 0; jn < JN; ++jn)
+    for (int jn = 0; jn < kJN; ++jn)
 #pragma unroll
       for (int c = 0; c < 2; ++c) {
         llacc[jn][c] = 0.0;
@@ -189,23 +190,23 @@ __global__ void __launch_bounds__(32 * (32 / JN), 1) glm_sweep_f64_kernel(SweepA
       if (tid < BM) ys[tid] = (n0 + tid < a.N) ? a.y[n0 + tid] : 0.0;
       __syncthreads();
 
-      double acc[MT][JN][2];
+      double acc[MT][kJN][2];
       if (active) {
-        // ---- phase A: z = X_tile . theta^T for this warp's 32 samples ------------------
+        // ---- phase A: z = X_tile . theta^T for this warp's 8 * kJN samples -------------
 #pragma unroll
         for (int i = 0; i < MT; ++i)
 #pragma unroll
-          for (int jn = 0; jn < JN; ++jn) acc[i][jn][0] = acc[i][jn][1] = 0.0;
+          for (int jn = 0; jn < kJN; ++jn) acc[i][jn][0] = acc[i][jn][1] = 0.0;
 
-        const double2* tp = a.thetaP + ((size_t)wc * JN * a.KG) * 32 + lane;
+        const double2* tp = a.thetaP + ((size_t)wc * kJN * a.KG) * 32 + lane;
         const size_t sbStride = (size_t)a.KG * 32;
-        double2 bcur[JN], bnxt[JN];
+        double2 bcur[kJN], bnxt[kJN];
 #pragma unroll
-        for (int jn = 0; jn < JN; ++jn) bcur[jn] = tp[jn * sbStride];
+        for (int jn = 0; jn < kJN; ++jn) bcur[jn] = tp[jn * sbStride];
         for (int kg = 0; kg < a.KG; ++kg) {
           if (kg + 1 < a.KG) {
 #pragma unroll
-            for (int jn = 0; jn < JN; ++jn) bnxt[jn] = tp[jn * sbStride + (size_t)(kg + 1) * 32];
+            for (int jn = 0; jn < kJN; ++jn) bnxt[jn] = tp[jn * sbStride + (size_t)(kg + 1) * 32];
           }
           double2 af[MT];
 #pragma unroll
@@ -216,24 +217,24 @@ __global__ void __launch_bounds__(32 * (32 / JN), 1) glm_sweep_f64_kernel(SweepA
 #pragma unroll
           for (int i = 0; i < MT; ++i)
 #pragma unroll
-            for (int jn = 0; jn < JN; ++jn) dmma884(acc[i][jn][0], acc[i][jn][1], af[i].x, bcur[jn].x);
+            for (int jn = 0; jn < kJN; ++jn) dmma884(acc[i][jn][0], acc[i][jn][1], af[i].x, bcur[jn].x);
 #pragma unroll
           for (int i = 0; i < MT; ++i)
 #pragma unroll
-            for (int jn = 0; jn < JN; ++jn) dmma884(acc[i][jn][0], acc[i][jn][1], af[i].y, bcur[jn].y);
+            for (int jn = 0; jn < kJN; ++jn) dmma884(acc[i][jn][0], acc[i][jn][1], af[i].y, bcur[jn].y);
 #pragma unroll
-          for (int jn = 0; jn < JN; ++jn) bcur[jn] = bnxt[jn];
+          for (int jn = 0; jn < kJN; ++jn) bcur[jn] = bnxt[jn];
         }
 
         // ---- phase B: link epilogue in registers -----------------------------------------
         // (the per-sample weights are re-read here, L1 hits, rather than held in registers across the tile: phase C
         // needs those registers to keep its DMMA chains interleaved)
-        double wv[JN][2], av[JN][2];
+        double wv[kJN][2], av[kJN][2];
 #pragma unroll
-        for (int jn = 0; jn < JN; ++jn)
+        for (int jn = 0; jn < kJN; ++jn)
 #pragma unroll
           for (int c = 0; c < 2; ++c) {
-            const int s = wc * (8 * JN) + jn * 8 + 2 * t + c;
+            const int s = wc * (8 * kJN) + jn * 8 + 2 * t + c;
             wv[jn][c] = __ldg(a.wP + s);
             av[jn][c] = (LINK == VB_LINK_GAUSSIAN) ? __ldg(a.auxP + s) : 1.0;
           }
@@ -245,7 +246,7 @@ __global__ void __launch_bounds__(32 * (32 / JN), 1) glm_sweep_f64_kernel(SweepA
           const double rv = (n0 + r < a.N) ? 1.0 : 0.0;
           double rs = 0.0;
 #pragma unroll
-          for (int jn = 0; jn < JN; ++jn)
+          for (int jn = 0; jn < kJN; ++jn)
 #pragma unroll
             for (int c = 0; c < 2; ++c) {
               double ll, rr;
@@ -288,17 +289,17 @@ __global__ void __launch_bounds__(32 * (32 / JN), 1) glm_sweep_f64_kernel(SweepA
           // Software pipelined: the DMMAs of column block jb + 1 are issued BEFORE the reduction of block jb (its
           // dependent X products, three shuffle levels and the shared-memory update), so that chain of latencies
           // runs under tensor work of the same warp instead of in front of it.
-          const double2* bp = a.baseP + ((size_t)wc * JN * a.KG) * 32 + lane;
+          const double2* bp = a.baseP + ((size_t)wc * kJN * a.KG) * 32 + lane;
           const size_t sbStride = (size_t)a.KG * 32;
           double* ge_w = PRIV ? ge_s + (size_t)warp * Dp : ge_s;
-          double2 e1[JN];
+          double2 e1[kJN];
           double tc0[MT], tc1[MT], tn0[MT], tn1[MT];
-          auto issue = [&](double (&u0)[MT], double (&u1)[MT], const double2 (&e)[JN]) {
+          auto issue = [&](double (&u0)[MT], double (&u1)[MT], const double2 (&e)[kJN]) {
 #pragma unroll
             for (int i = 0; i < MT; ++i) u0[i] = u1[i] = 0.0;
             // MT independent accumulation chains, interleaved (a chain's next DMMA is MT instructions away)
 #pragma unroll
-            for (int jn = 0; jn < JN; ++jn) {
+            for (int jn = 0; jn < kJN; ++jn) {
 #pragma unroll
               for (int i = 0; i < MT; ++i) dmma884(u0[i], u1[i], acc[i][jn][0], e[jn].x);
 #pragma unroll
@@ -306,18 +307,18 @@ __global__ void __launch_bounds__(32 * (32 / JN), 1) glm_sweep_f64_kernel(SweepA
             }
           };
 #pragma unroll
-          for (int jn = 0; jn < JN; ++jn) e1[jn] = bp[jn * sbStride];
+          for (int jn = 0; jn < kJN; ++jn) e1[jn] = bp[jn * sbStride];
           issue(tc0, tc1, e1);
           if (a.KG > 1) {
 #pragma unroll
-            for (int jn = 0; jn < JN; ++jn) e1[jn] = bp[jn * sbStride + 32];
+            for (int jn = 0; jn < kJN; ++jn) e1[jn] = bp[jn * sbStride + 32];
           }
 #pragma unroll 2
           for (int jb = 0; jb < a.KG; ++jb) {
             if (jb + 1 < a.KG) issue(tn0, tn1, e1);
             if (jb + 2 < a.KG) {      // the E fragments of block jb + 2 arrive under this block's reduction
 #pragma unroll
-              for (int jn = 0; jn < JN; ++jn) e1[jn] = bp[jn * sbStride + (size_t)(jb + 2) * 32];
+              for (int jn = 0; jn < kJN; ++jn) e1[jn] = bp[jn * sbStride + (size_t)(jb + 2) * 32];
             }
             double p0 = 0.0, p1 = 0.0;
 #pragma unroll
@@ -357,13 +358,13 @@ __global__ void __launch_bounds__(32 * (32 / JN), 1) glm_sweep_f64_kernel(SweepA
     // ---- per-CTA log-likelihood partials for this super-chunk ------------------------------
     if (active) {
 #pragma unroll
-      for (int jn = 0; jn < JN; ++jn)
+      for (int jn = 0; jn < kJN; ++jn)
 #pragma unroll
         for (int c = 0; c < 2; ++c) {
           double v = llacc[jn][c];
 #pragma unroll
           for (int o = 4; o < 32; o <<= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-          if (g == 0) a.ll_part[(size_t)blockIdx.x * a.WC * (8 * JN) + wc * (8 * JN) + jn * 8 + 2 * t + c] = v;
+          if (g == 0) a.ll_part[(size_t)blockIdx.x * a.WC * (8 * kJN) + wc * (8 * kJN) + jn * 8 + 2 * t + c] = v;
         }
     }
   }  // super-chunks
@@ -396,7 +397,7 @@ __global__ void reduce_partials_f64_kernel(const double* __restrict__ part, int 
 }
 
 struct SweepPlan {
-  int BM, KG, P, WC, SB, JN, priv, grid;
+  int BM, KG, P, WC, SB, priv, grid;
   int64_t numTiles;
   size_t smem;
   size_t off_thetaP, off_baseP, off_wP, off_auxP, off_ll, off_gmu, off_ge, off_ge_rows, total;
@@ -406,11 +407,8 @@ static bool make_plan(int64_t N, int d, int64_t S, SweepPlan& p) {
   p.KG = (int)ceil_div(d, 8);
   const int Dp = p.KG * 8;
   p.P = (Dp % 16 == 0) ? Dp + 8 : Dp + 16;
-  // VB_F64_JN=4 selects the first version's 8 warps x 32 samples (A/B timing)
-  static const int jn = [] { const char* e = getenv("VB_F64_JN"); return (e && e[0] == '4') ? 4 : 2; }();
-  p.JN = jn;
-  p.WC = (int)ceil_div(S, 8 * p.JN);
-  p.SB = p.WC * p.JN;
+  p.WC = (int)ceil_div(S, 8 * kJN);
+  p.SB = p.WC * kJN;
   p.BM = 0;
   for (int bm : {32, 16, 8}) {
     size_t bytes = sizeof(double) * ((size_t)bm * p.P + 2 * bm + 2 * (size_t)Dp);
@@ -422,7 +420,7 @@ static bool make_plan(int64_t N, int d, int64_t S, SweepPlan& p) {
   }
   if (p.BM == 0) return false;
   {   // per-warp ge rows when they fit beside the tile; the per-warp rbar rows after them, or in the unused ge slot
-    const int warps = 32 / p.JN;
+    const int warps = 32 / kJN;
     const size_t extra = sizeof(double) * ((size_t)(warps - 1) * Dp + (size_t)warps * p.BM);
     p.priv = (p.smem + extra <= 227 * 1024) ? 1 : 0;
     if (p.priv) {
@@ -449,28 +447,23 @@ static bool make_plan(int64_t N, int d, int64_t S, SweepPlan& p) {
   p.off_ll = take((size_t)p.grid * p.SB * 8 * sizeof(double));
   p.off_gmu = take((size_t)p.grid * Dp * sizeof(double));
   p.off_ge = take((size_t)p.grid * Dp * sizeof(double));
-  p.off_ge_rows = take(p.priv ? 0 : (size_t)p.grid * (32 / p.JN) * Dp * sizeof(double));
+  p.off_ge_rows = take(p.priv ? 0 : (size_t)p.grid * (32 / kJN) * Dp * sizeof(double));
   p.total = off;
   return true;
 }
 
-template <int BM, int LINK, int JN, bool PRIV>
+template <int BM, int LINK, bool PRIV>
 static int launch_sweep_priv(const SweepArgs& a, const SweepPlan& p, cudaStream_t stream) {
-  auto kern = glm_sweep_f64_kernel<BM, LINK, JN, PRIV>;
+  auto kern = glm_sweep_f64_kernel<BM, LINK, PRIV>;
   VB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)p.smem));
-  kern<<<p.grid, 32 * (32 / JN), p.smem, stream>>>(a);
+  kern<<<p.grid, 32 * (32 / kJN), p.smem, stream>>>(a);
   VB_CHECK_LAUNCH();
   return VB_OK;
 }
 
-template <int BM, int LINK, int JN>
-static int launch_sweep_jn(const SweepArgs& a, const SweepPlan& p, cudaStream_t stream) {
-  return p.priv ? launch_sweep_priv<BM, LINK, JN, true>(a, p, stream) : launch_sweep_priv<BM, LINK, JN, false>(a, p, stream);
-}
-
 template <int BM, int LINK>
 static int launch_sweep(const SweepArgs& a, const SweepPlan& p, cudaStream_t stream) {
-  return p.JN == 4 ? launch_sweep_jn<BM, LINK, 4>(a, p, stream) : launch_sweep_jn<BM, LINK, 2>(a, p, stream);
+  return p.priv ? launch_sweep_priv<BM, LINK, true>(a, p, stream) : launch_sweep_priv<BM, LINK, false>(a, p, stream);
 }
 
 template <int LINK>

@@ -1,36 +1,37 @@
 // Tensor-core "fast path" of the GLM model plugin (logistic link), sm_100a only:
-// TMA -> shared memory -> tcgen05.mma (fp16 operands, fp32 accumulators in TMEM).
+// TMA -> shared memory -> tcgen05.mma (fp16 / e5m2 operands, fp32 accumulators in TMEM).
 //
-// Per 128-observation tile, one persistent CTA per SM:
-//   GEMM1  Z[n,s]  = sum_j Xy[n,j] Theta[s,j]        M=128 (n), N=256 (s), K=d
-//          three fp16 passes  Xh.Th + Xl.Th + Xh.Tl  (Xy = y*X and Theta split hi+lo: 22-bit operands)
-//          (the CTA-pair kernel, the default, runs the two correction products Xl.Th and Xh.Tl on e5m2 copies with
-//          reciprocal power-of-two scales as kind::f8f6f4 MMAs: see glm_fast_pair_kernel)
+// One kernel, glm_fast_pair_kernel: persistent clusters of two CTAs (cta_group::2), each pair working on a 256-row
+// super-tile (two 128-observation tiles) at a time:
+//   GEMM1  Z[n,s]  = sum_j Xy[n,j] Theta[s,j]        M=256 (n), N=256 (s), K=d
+//          Xy = y*X and Theta are split hi + lo (22-bit operands): one fp16 pass Xh.Th plus the two correction
+//          products Xl.Th and Xh.Tl on e5m2 copies with reciprocal power-of-two scales, as kind::f8f6f4 MMAs
 //   E1     link epilogue out of TMEM: ll[s] += -softplus(-z), R[n,s] = w_s*sigmoid(-z) -> fp16 tile in
 //          shared memory (the N x S logits / residuals never touch HBM), rbar[n] = sum_s R[n,s]
-//   GEMM2  Tt[j,n] = sum_s E[s,j] R[n,s]             M=128 (j), N=128 (n), K=256 (s); A = E (MN-major)
+//   GEMM2  Tt[j,n] = sum_s E[s,j] R[n,s]             M=256 (j), N=128 (n), K=256 (s); A = E (MN-major)
 //   E2     thread owns j: ge[j] += sum_n Xy[n,j] Tt[j,n],  gmu[j] += sum_n Xy[n,j] rbar[n]
-//          (Xy chunk re-read through TMA, an L2 hit)
+//          (Xy = X_h + X_l8 2^-ax read straight from global memory, an L2 hit)
 // Replaces the same reference code as glm_f64.cu (user log_density under autograd:
 // models.py:27-39, objectives.py:161-167).  Tolerance of this path: 1e-4 relative (BASELINE.json).
 //
-// Warp roles: warp 0 = TMA producer, warp 1 = MMA issuer + TMEM owner, warps 2..9 = epilogue.
-// Shared memory: 10 x 16 KB operand ring, 64 KB R tile, barriers.  TMEM: Z 256 cols, Tt 2 x 128 cols.
+// Shared memory per CTA: 10 x 16 KB operand ring, 64 KB R tile, barriers.  TMEM: Z 256 cols, Tt 2 x 128 cols.
 //
-// HBM layout (chosen for the kernel, produced once by vb_glm_fast_create):
-//   Xt_h, Xt_l : fp16 [numTiles][2][d_pad][64]   "tile-transposed": for each 128-row tile and each 64-row half the
-//                d_pad x 64 block (column j = one 128-byte row) is contiguous, so GEMM1 reads it as an MN-major
-//                A operand (64-element groups, 128-byte swizzle) and E2's column-owning threads read 128-byte rows.
-//   Tt_h, Tt_l : fp16 [4][d_pad][64]  Theta^T in 64-sample groups (MN-major B operand), rebuilt every sweep
-//   E          : fp16 [d_pad/64][256][64]  base draws in 64-column groups (MN-major A operand of GEMM2)
+// HBM layout (chosen for the kernel; X produced once by vb_glm_fast_create, Theta and E rebuilt every sweep):
+//   X_h, X_l : fp16 [numTiles][2][d_pad][64]   "tile-transposed": for each 128-row tile and each 64-row half the
+//              d_pad x 64 block (column j = one 128-byte row) is contiguous, so GEMM1 reads it as an MN-major
+//              A operand (64-element groups, 128-byte swizzle) and E2's column-owning threads read 128-byte runs.
+//              X_l only feeds fast_prepare_x8_kernel.
+//   X8       : e5m2 [X_l 2^ax | X_h 2^-bx][numTiles][d_pad][128]   one 128-byte row = a tile's 128 rows of column j
+//   Th       : fp16 [4][d_pad][64]  Theta_h^T in 64-sample groups (MN-major B operand)
+//   T8       : e5m2 [Theta_h 2^-ax | Theta_l 2^bx][2][d_pad][128]  Theta^T in 128-sample groups
+//   E        : fp16 [d_pad/64][256][64]  base draws in 64-column groups (MN-major A operand of GEMM2)
 // Every operand group is a dense array of 128-byte rows, so ONE multi-dimensional TMA box per pipeline stage and
 // operand writes all its groups (the TMA unit is op-rate bound at 4 KB boxes).
 // All operands are MN-major with the 128-byte swizzle, so the K extent of a pipeline stage is free:
-// GEMM1 streams K = 32 per stage (16 KB for X hi+lo, 16 KB each for Theta lo / hi).
+// GEMM1 streams K = 32 per stage (16 KB for X, 16 KB for Theta).
 #include <cuda.h>
 #include <cuda_fp16.h>
 
-#include <cstdlib>
 #include <cstring>
 #include <mutex>
 
@@ -48,8 +49,6 @@ constexpr int kRingBytes = kSlotBytes * kNumSlots;      // 163840
 constexpr int kRBytes = kBM * kSP * 2;                  // 65536
 constexpr int kMiscBytes = 3072;
 constexpr int kSmemBytes = kRingBytes + kRBytes + kMiscBytes;   // 232448 = 227 KB
-constexpr int kEpiWarps = 8;
-constexpr int kThreads = 64 + 32 * kEpiWarps;           // 320
 constexpr uint32_t kTmemCols = 512;
 
 // ---- PTX wrappers ------------------------------------------------------------------------------
@@ -61,23 +60,6 @@ __device__ __forceinline__ void mbar_init(uint32_t bar, uint32_t count) {
 __device__ __forceinline__ void mbar_expect_tx(uint32_t bar, uint32_t bytes) {
   asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
 }
-__device__ __forceinline__ void mbar_arrive(uint32_t bar) {
-  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory");
-}
-__device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
-  uint32_t done;
-  do {
-    asm volatile(
-        "{\n"
-        ".reg .pred p;\n"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n"
-        "selp.u32 %0, 1, 0, p;\n"
-        "}\n"
-        : "=r"(done)
-        : "r"(bar), "r"(parity)
-        : "memory");
-  } while (!done);
-}
 __device__ __forceinline__ float fast_exp2(float x) {
   float y;
   asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x));
@@ -88,12 +70,6 @@ __device__ __forceinline__ void fence_proxy_async() { asm volatile("fence.proxy.
 __device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
 __device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
 
-__device__ __forceinline__ void tma_load_2d(uint32_t dst, const CUtensorMap* map, int c0, int c1, uint32_t bar) {
-  asm volatile(
-      "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3}], [%4];" ::"r"(dst),
-      "l"(map), "r"(c0), "r"(c1), "r"(bar)
-      : "memory");
-}
 __device__ __forceinline__ void tma_load_3d_pair(uint32_t dst, const CUtensorMap* map, int c0, int c1, int c2, uint32_t bar_cluster) {
   asm volatile(
       "cp.async.bulk.tensor.3d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3, %4}], [%5];" ::"r"(dst),
@@ -107,31 +83,9 @@ __device__ __forceinline__ void tma_load_4d_pair(uint32_t dst, const CUtensorMap
       "l"(map), "r"(c0), "r"(c1), "r"(c2), "r"(c3), "r"(bar_cluster)
       : "memory");
 }
-__device__ __forceinline__ void tma_load_5d_pair(uint32_t dst, const CUtensorMap* map, int c0, int c1, int c2, int c3, int c4,
-                                                 uint32_t bar_cluster) {
-  asm volatile(
-      "cp.async.bulk.tensor.5d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3, %4, %5, %6}], [%7];" ::"r"(dst),
-      "l"(map), "r"(c0), "r"(c1), "r"(c2), "r"(c3), "r"(c4), "r"(bar_cluster)
-      : "memory");
-}
 __device__ __forceinline__ void prefetch_tmap(const CUtensorMap* map) {
   asm volatile("prefetch.tensormap [%0];" ::"l"(map) : "memory");
 }
-
-__device__ __forceinline__ void umma_f16(uint32_t d_tmem, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
-  asm volatile(
-      "{\n"
-      ".reg .pred p;\n"
-      "setp.ne.b32 p, %4, 0;\n"
-      "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n"
-      "}\n" ::"r"(d_tmem),
-      "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
-__device__ __forceinline__ void umma_commit(uint32_t bar) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");
-}
-
 
 // ---- cluster / CTA-pair helpers (cta_group::2) ---------------------------------------------------
 __device__ __forceinline__ uint32_t cluster_ctarank() {
@@ -185,13 +139,6 @@ __device__ __forceinline__ void mbar_wait_cl_sleep(uint32_t bar, uint32_t parity
 }
 __device__ __forceinline__ void st_cluster_f32(uint32_t cluster_addr, float v) {
   asm volatile("st.shared::cluster.f32 [%0], %1;" ::"r"(cluster_addr), "f"(v) : "memory");
-}
-// TMA load into this CTA's shared memory, completion bytes signalled on a barrier of the pair's leader CTA
-__device__ __forceinline__ void tma_load_2d_pair(uint32_t dst, const CUtensorMap* map, int c0, int c1, uint32_t bar_cluster) {
-  asm volatile(
-      "cp.async.bulk.tensor.2d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3}], [%4];" ::"r"(dst),
-      "l"(map), "r"(c0), "r"(c1), "r"(bar_cluster)
-      : "memory");
 }
 __device__ __forceinline__ void umma_f16_pair(uint32_t d_tmem, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
   asm volatile(
@@ -274,28 +221,12 @@ struct Params {
   double* ll_part;   // [grid][256]
   double* gmu_part;  // [grid][d_pad]
   double* ge_part;   // [grid][d_pad]
-  float* dbg;        // optional: Z of this CTA's first tile [128][256], then Tt of j-block 0 [128][128]
   long long* tim;    // optional: clock64 timestamps of CTA 0
   int uniform_w;     // 1: every valid sample has weight 1 (w == NULL on the host side)
-  const __half* Xh;  // pair kernel: E2 reads its X rows from global memory
-  const __half* Xl;
-  const uint8_t* Xl8;  // fp8 scheme: e5m2 of X_l * 2^ax, [tile][d_pad][128 n]
+  const __half* Xh;  // E2 reads its X rows from global memory
   float xl_scale;      // 2^-ax
+  const uint8_t* Xl8;  // e5m2 of X_l * 2^ax, [tile][d_pad][128 n]
 };
-
-struct Misc {
-  uint64_t empty[kNumSlots];          // per 16 KB slot: consumer -> producer
-  uint64_t g1_full[4];                // per GEMM1 stage (3 slots, 48 KB), ring of 4 phases
-  uint64_t e_full[2];                 // per GEMM2 block: the 4 E slots (64 KB)
-  uint64_t x_full[2][2];              // per GEMM2 block and tile-row half: X hi + lo slots (32 KB)
-  uint64_t z_full, r_full, t_full[2], t_empty[2];
-  uint32_t tmem_base;
-  uint32_t pad;
-  alignas(16) float w[kSP];
-  alignas(16) float rbar[2][kBM];
-  alignas(16) float rb[kBM];
-};
-static_assert(sizeof(Misc) <= kMiscBytes, "misc smem overflow");
 
 __device__ __forceinline__ bool elect_one() {
   uint32_t pred;
@@ -308,379 +239,9 @@ __device__ __forceinline__ bool elect_one() {
       : "=r"(pred));
   return pred != 0;
 }
-__device__ __forceinline__ void epi_barrier() { asm volatile("bar.sync 1, 256;" ::: "memory"); }
-
-// fill sequence of one tile (identical in every role):
-//   GEMM1 stage kc (K = 32):  3*kc + 0 : X  (hi n0 | hi n1 | lo n0 | lo n1, 4 KB each)
-//                             3*kc + 1 : Theta_lo^T (4 sample groups of 64, 4 KB each)
-//                             3*kc + 2 : Theta_hi^T
-//   GEMM2 block jb (128 j):   G + 8*jb + g   (g = 0..3): E rows 64g..64g+63 (2 boxes of 64 j, 8 KB each)
-//                             G + 8*jb + 4 + a (a = 0,1): X hi, n-half a (2 boxes of 64 j-rows, 8 KB each)
-//                             G + 8*jb + 6 + a          : X lo, n-half a            with G = 3*KC
-__global__ void __launch_bounds__(kThreads, 1)
-glm_fast_kernel(const __grid_constant__ CUtensorMap tmXh, const __grid_constant__ CUtensorMap tmXl,
-                const __grid_constant__ CUtensorMap tmXh2, const __grid_constant__ CUtensorMap tmXl2,
-                const __grid_constant__ CUtensorMap tmTh, const __grid_constant__ CUtensorMap tmTl,
-                const __grid_constant__ CUtensorMap tmE, Params p) {
-  extern __shared__ __align__(1024) uint8_t smem[];
-  uint8_t* ring = smem;
-  uint8_t* rtile = smem + kRingBytes;
-  Misc* misc = reinterpret_cast<Misc*>(smem + kRingBytes + kRBytes);
-  const uint32_t ring_u = smem_u32(ring), rtile_u = smem_u32(rtile);
-
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int KC = p.d_pad / 32, JB = p.d_pad / 128;
-  const int G = 3 * KC;
-  const int fillsPerTile = G + (p.want_grad ? 8 * JB : 0);
-
-  if (threadIdx.x == 0) {
-    for (int i = 0; i < kNumSlots; ++i) mbar_init(smem_u32(&misc->empty[i]), 1);
-    for (int i = 0; i < 4; ++i) mbar_init(smem_u32(&misc->g1_full[i]), 1);
-    for (int i = 0; i < 2; ++i) {
-      mbar_init(smem_u32(&misc->e_full[i]), 1);
-      mbar_init(smem_u32(&misc->x_full[i][0]), 1);
-      mbar_init(smem_u32(&misc->x_full[i][1]), 1);
-    }
-    mbar_init(smem_u32(&misc->z_full), 1);
-    mbar_init(smem_u32(&misc->r_full), 1);
-    for (int i = 0; i < 2; ++i) {
-      mbar_init(smem_u32(&misc->t_full[i]), 1);
-      mbar_init(smem_u32(&misc->t_empty[i]), 1);
-    }
-    fence_barrier_init();
-  }
-  for (int i = threadIdx.x; i < kSP; i += kThreads) misc->w[i] = p.w[i];
-  if (warp == 1) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(&misc->tmem_base)),
-                 "r"(kTmemCols)
-                 : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-  }
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem = misc->tmem_base;
-
-  if (warp == 0) {
-    // ================================ TMA producer ================================
-    if (lane == 0) {
-      prefetch_tmap(&tmXh); prefetch_tmap(&tmXl); prefetch_tmap(&tmXh2); prefetch_tmap(&tmXl2);
-      prefetch_tmap(&tmTh); prefetch_tmap(&tmTl); prefetch_tmap(&tmE);
-      uint32_t fill = 0, sc = 0, bc = 0;
-      auto acquire = [&]() -> uint32_t {       // next ring slot, once its previous contents are consumed
-        const uint32_t slot = fill % kNumSlots, par = (fill / kNumSlots) & 1;
-        mbar_wait(smem_u32(&misc->empty[slot]), par ^ 1);
-        ++fill;
-        return ring_u + slot * kSlotBytes;
-      };
-      for (int tile = blockIdx.x; tile < p.numTiles; tile += gridDim.x) {
-        const int r0 = tile * 2 * p.d_pad;      // first row of this tile in the [tile][half][j] x 64 view of X
-        for (int kc = 0; kc < KC; ++kc, ++sc) {
-          const int j0 = kc * 32;
-          const uint32_t bar = smem_u32(&misc->g1_full[sc & 3]);
-          mbar_expect_tx(bar, 3 * kSlotBytes);
-          uint32_t dst = acquire();
-          tma_load_2d(dst, &tmXh, 0, r0 + j0, bar);
-          tma_load_2d(dst + 4096, &tmXh, 0, r0 + p.d_pad + j0, bar);
-          tma_load_2d(dst + 8192, &tmXl, 0, r0 + j0, bar);
-          tma_load_2d(dst + 12288, &tmXl, 0, r0 + p.d_pad + j0, bar);
-          dst = acquire();
-#pragma unroll
-          for (int g = 0; g < 4; ++g) tma_load_2d(dst + g * 4096, &tmTl, 0, g * p.d_pad + j0, bar);
-          dst = acquire();
-#pragma unroll
-          for (int g = 0; g < 4; ++g) tma_load_2d(dst + g * 4096, &tmTh, 0, g * p.d_pad + j0, bar);
-        }
-        if (p.want_grad) {
-          for (int jb = 0; jb < JB; ++jb, ++bc) {
-            const int j0 = jb * 128;
-            const uint32_t ebar = smem_u32(&misc->e_full[bc & 1]);
-            mbar_expect_tx(ebar, 4 * kSlotBytes);
-            for (int g = 0; g < 4; ++g) {
-              const uint32_t dst = acquire();
-              tma_load_2d(dst, &tmE, 0, (j0 >> 6) * kSP + 64 * g, ebar);
-              tma_load_2d(dst + 8192, &tmE, 0, ((j0 >> 6) + 1) * kSP + 64 * g, ebar);
-            }
-            mbar_expect_tx(smem_u32(&misc->x_full[bc & 1][0]), 2 * kSlotBytes);
-            mbar_expect_tx(smem_u32(&misc->x_full[bc & 1][1]), 2 * kSlotBytes);
-            for (int a = 0; a < 2; ++a) {
-              const uint32_t dst = acquire(), xbar = smem_u32(&misc->x_full[bc & 1][a]);
-              tma_load_2d(dst, &tmXh2, 0, r0 + a * p.d_pad + j0, xbar);
-              tma_load_2d(dst + 8192, &tmXh2, 0, r0 + a * p.d_pad + j0 + 64, xbar);
-            }
-            for (int a = 0; a < 2; ++a) {
-              const uint32_t dst = acquire(), xbar = smem_u32(&misc->x_full[bc & 1][a]);
-              tma_load_2d(dst, &tmXl2, 0, r0 + a * p.d_pad + j0, xbar);
-              tma_load_2d(dst + 8192, &tmXl2, 0, r0 + a * p.d_pad + j0 + 64, xbar);
-            }
-          }
-        }
-      }
-    }
-  } else if (warp == 1) {
-    // ================================ MMA issuer (whole warp converged, one elected lane issues) ==========
-    constexpr uint32_t idesc1 = make_idesc(128, 256, 1, 1);   // Z : A = Xt (MN-major), B = Theta^T (MN-major)
-    constexpr uint32_t idesc2 = make_idesc(128, 128, 1, 0);   // Tt: A = E (MN-major),  B = R (K-major)
-    uint32_t ltile = 0, sc = 0, bc = 0;
-    for (int tile = blockIdx.x; tile < p.numTiles; tile += gridDim.x, ++ltile) {
-      const uint32_t fbase = ltile * fillsPerTile;
-      if (p.tim && blockIdx.x == 0 && ltile < 8 && lane == 0) p.tim[ltile * 16 + 0] = clock64();
-      // ---- GEMM1: per stage, pass 1 = Xh.Tl (Theta_lo released right after), then Xh.Th, Xl.Th ----
-      for (int kc = 0; kc < KC; ++kc, ++sc) {
-        const uint32_t f0 = fbase + 3 * kc;
-        const uint32_t s0 = f0 % kNumSlots, s1 = (f0 + 1) % kNumSlots, s2 = (f0 + 2) % kNumSlots;
-        const uint32_t ax = ring_u + s0 * kSlotBytes, bl = ring_u + s1 * kSlotBytes, bh = ring_u + s2 * kSlotBytes;
-        mbar_wait(smem_u32(&misc->g1_full[sc & 3]), (sc >> 2) & 1);
-        tc_fence_after();
-        if (elect_one()) {
-          // MN-major operands: 16 K-rows of 128 bytes per K step (2048 B), 64-element groups along M/N at +4096
-#pragma unroll
-          for (int k = 0; k < 2; ++k)
-            umma_f16(tmem, make_desc(ax + k * 2048, 4096, 1024), make_desc(bl + k * 2048, 4096, 1024), idesc1,
-                     (kc | k) ? 1u : 0u);
-          umma_commit(smem_u32(&misc->empty[s1]));
-#pragma unroll
-          for (int k = 0; k < 2; ++k)
-            umma_f16(tmem, make_desc(ax + k * 2048, 4096, 1024), make_desc(bh + k * 2048, 4096, 1024), idesc1, 1u);
-#pragma unroll
-          for (int k = 0; k < 2; ++k)
-            umma_f16(tmem, make_desc(ax + 8192 + k * 2048, 4096, 1024), make_desc(bh + k * 2048, 4096, 1024), idesc1, 1u);
-          umma_commit(smem_u32(&misc->empty[s0]));
-          umma_commit(smem_u32(&misc->empty[s2]));
-          if (kc == KC - 1) umma_commit(smem_u32(&misc->z_full));
-        }
-        __syncwarp();
-      }
-      if (p.tim && blockIdx.x == 0 && ltile < 8 && lane == 0) p.tim[ltile * 16 + 1] = clock64();
-      // ---- GEMM2 ----  (r_full also means "Z has been read": the next tile may overwrite it)
-      mbar_wait(smem_u32(&misc->r_full), ltile & 1);
-      tc_fence_after();
-      if (p.tim && blockIdx.x == 0 && ltile < 8 && lane == 0) p.tim[ltile * 16 + 2] = clock64();
-      if (p.want_grad) {
-        for (int jb = 0; jb < JB; ++jb, ++bc) {
-          const uint32_t buf = bc & 1;
-          mbar_wait(smem_u32(&misc->t_empty[buf]), ((bc >> 1) & 1) ^ 1);
-          mbar_wait(smem_u32(&misc->e_full[buf]), (bc >> 1) & 1);
-          tc_fence_after();
-          if (elect_one()) {
-            const uint32_t dT = tmem + 256 + 128 * buf;
-#pragma unroll
-            for (int g = 0; g < 4; ++g) {
-              const uint32_t slot = (fbase + G + 8 * jb + g) % kNumSlots;
-              const uint32_t es = ring_u + slot * kSlotBytes;
-#pragma unroll
-              for (int k = 0; k < 4; ++k) {
-                // A = E^T tile: 64 j per 128-byte row, 16 s rows per K step, second 64-j group at +8 KB
-                umma_f16(dT, make_desc(es + k * 2048, 8192, 1024), make_desc(rtile_u + g * 16384 + k * 32, 16, 1024),
-                         idesc2, (g | k) ? 1u : 0u);
-              }
-              umma_commit(smem_u32(&misc->empty[slot]));
-            }
-            umma_commit(smem_u32(&misc->t_full[buf]));
-          }
-          __syncwarp();
-          if (p.tim && blockIdx.x == 0 && ltile < 8 && jb < 4 && lane == 0) p.tim[ltile * 16 + 3 + jb] = clock64();
-        }
-      }
-    }
-  } else {
-    // ================================ epilogue warps ================================
-    const int ew = warp - 2;
-    const int q = warp & 3;            // TMEM lane quarter this warp may access
-    const int h = ew >> 2;             // column half (E1: samples, E2: tile rows)
-    const int row = 32 * q + lane;     // TMEM lane = tile row (E1) or j within block (E2)
-    const uint32_t lane_addr = tmem + ((uint32_t)(32 * q) << 16);
-    double ll_acc[4] = {0.0, 0.0, 0.0, 0.0};
-    double ge_acc[16], gmu_acc[16];
-#pragma unroll
-    for (int i = 0; i < 16; ++i) ge_acc[i] = gmu_acc[i] = 0.0;
-    uint32_t ltile = 0, tcount = 0;
-    for (int tile = blockIdx.x; tile < p.numTiles; tile += gridDim.x, ++ltile) {
-      const uint32_t fbase = ltile * fillsPerTile;
-      const int64_t n = (int64_t)tile * kBM + row;
-      const float rowvalid = n < p.N ? 1.0f : 0.0f;
-      // -------- E1: link epilogue on Z --------
-      mbar_wait(smem_u32(&misc->z_full), ltile & 1);
-      tc_fence_after();
-      if (p.tim && blockIdx.x == 0 && ltile < 8 && threadIdx.x == 64) p.tim[ltile * 16 + 8] = clock64();
-      float rsum = 0.0f;
-#pragma unroll 1
-      for (int c = 0; c < 4; ++c) {
-        const int col0 = 128 * h + 32 * c;
-        float v[32];
-        tmem_ld32(lane_addr + col0, v);
-        if (p.dbg && ltile == 0) {
-#pragma unroll
-          for (int i = 0; i < 32; ++i) p.dbg[(size_t)blockIdx.x * 49152 + row * 256 + col0 + i] = v[i];
-        }
-        uint32_t packed[16];
-        float spsum = 0.0f;
-#pragma unroll
-        for (int i = 0; i < 32; i += 2) {
-          float r2[2];
-#pragma unroll
-          for (int u = 0; u < 2; ++u) {
-            const float a = v[i + u];
-            const float t = fast_exp2(-fabsf(a) * 1.4426950408889634f);
-            const float den = 1.0f + t;
-            const float l1p = __log2f(den) * 0.6931471805599453f;
-            const float sp = (fmaxf(-a, 0.0f) + l1p) * rowvalid;           // softplus(-a)
-            v[i + u] = sp;
-            spsum += col0 + i + u < p.S ? sp : 0.0f;                       // the total counts valid samples only
-            const float sg = __fdividef(a >= 0.0f ? t : 1.0f, den);        // sigmoid(-a)
-            r2[u] = sg * misc->w[col0 + i + u] * rowvalid;
-            rsum += r2[u];
-          }
-          const __half2 hh = __floats2half2_rn(r2[0], r2[1]);
-          packed[i >> 1] = *reinterpret_cast<const uint32_t*>(&hh);
-        }
-        // R tile: K-group g (64 samples, 16 KB), row-major 128-byte rows, 128B swizzle
-        {
-          const int g = col0 >> 6;
-          const int cbase = (col0 & 63) >> 3;          // first 16-byte chunk of this 32-sample run
-          uint8_t* rowp = rtile + g * 16384 + row * 128;
-#pragma unroll
-          for (int u = 0; u < 4; ++u) {
-            const int chunk = (cbase + u) ^ (row & 7);
-            *reinterpret_cast<uint4*>(rowp + chunk * 16) =
-                make_uint4(packed[4 * u], packed[4 * u + 1], packed[4 * u + 2], packed[4 * u + 3]);
-          }
-        }
-        if (p.ll_total_only) {
-          ll_acc[0] += (double)spsum;       // only the grand total is needed
-        } else {
-          // column sums of softplus over this warp's 32 rows (transpose-reduce): lane l ends with column l
-#pragma unroll
-          for (int o = 16, cnt = 16; o >= 1; o >>= 1, cnt >>= 1) {
-            const bool up = (lane & o) != 0;
-#pragma unroll
-            for (int i = 0; i < cnt; ++i) {
-              const float send = up ? v[i] : v[i + cnt];
-              const float keep = up ? v[i + cnt] : v[i];
-              v[i] = keep + __shfl_xor_sync(0xffffffffu, send, o);
-            }
-          }
-          ll_acc[c] += (double)v[0];
-        }
-      }
-      misc->rbar[h][row] = rsum;
-      fence_proxy_async();       // R tile writes -> visible to the tensor core (async proxy)
-      tc_fence_before();
-      epi_barrier();
-      if (threadIdx.x == 64) mbar_arrive(smem_u32(&misc->r_full));
-      if (p.tim && blockIdx.x == 0 && ltile < 8 && threadIdx.x == 64) p.tim[ltile * 16 + 9] = clock64();
-      if (!p.want_grad) continue;
-      if (h == 0) misc->rb[row] = misc->rbar[0][row] + misc->rbar[1][row];
-      epi_barrier();
-      // -------- E2: thread owns column j = 128*jb + row and the tile rows [64h, 64h+64) --------
-#pragma unroll 1
-      for (int jb = 0; jb < JB; ++jb, ++tcount) {
-        const uint32_t buf = tcount & 1;
-        const uint32_t fh = fbase + G + 8 * jb + 4 + h, fl = fh + 2;
-        const uint32_t sh = fh % kNumSlots, sl = fl % kNumSlots;
-        mbar_wait(smem_u32(&misc->x_full[buf][h]), (tcount >> 1) & 1);
-        mbar_wait(smem_u32(&misc->t_full[buf]), (tcount >> 1) & 1);
-        tc_fence_after();
-        if (p.tim && blockIdx.x == 0 && ltile < 8 && threadIdx.x == 64 && jb < 4) p.tim[ltile * 16 + 10 + jb] = clock64();
-        const int rr = row & 63;
-        const uint8_t* xh = ring + sh * kSlotBytes + (row >> 6) * 8192 + rr * 128;
-        const uint8_t* xl = ring + sl * kSlotBytes + (row >> 6) * 8192 + rr * 128;
-        float ge = 0.0f, gm = 0.0f;
-#pragma unroll 1
-        for (int part = 0; part < 2; ++part) {
-          const int nb = 64 * h + 32 * part;
-          float tv[32];
-          tmem_ld32(lane_addr + 256 + 128 * buf + nb, tv);
-          if (p.dbg && ltile == 0 && jb == 0) {
-#pragma unroll
-            for (int i = 0; i < 32; ++i) p.dbg[(size_t)blockIdx.x * 49152 + 32768 + row * 128 + nb + i] = tv[i];
-          }
-#pragma unroll
-          for (int c = 0; c < 4; ++c) {
-            const int cc = 4 * part + c;                       // 16-byte chunk = 8 consecutive tile rows
-            const uint4 vh = *reinterpret_cast<const uint4*>(xh + ((cc ^ (rr & 7)) << 4));
-            const uint4 vl = *reinterpret_cast<const uint4*>(xl + ((cc ^ (rr & 7)) << 4));
-            const float4 rb0 = *reinterpret_cast<const float4*>(&misc->rb[nb + 8 * c]);
-            const float4 rb1 = *reinterpret_cast<const float4*>(&misc->rb[nb + 8 * c + 4]);
-            const float rbv[8] = {rb0.x, rb0.y, rb0.z, rb0.w, rb1.x, rb1.y, rb1.z, rb1.w};
-            const uint32_t hw[4] = {vh.x, vh.y, vh.z, vh.w}, lw[4] = {vl.x, vl.y, vl.z, vl.w};
-#pragma unroll
-            for (int e = 0; e < 4; ++e) {
-              const float2 fh2 = __half22float2(*reinterpret_cast<const __half2*>(&hw[e]));
-              const float2 fl2 = __half22float2(*reinterpret_cast<const __half2*>(&lw[e]));
-              const float x0 = fh2.x + fl2.x, x1 = fh2.y + fl2.y;
-              ge = fmaf(x0, tv[8 * c + 2 * e], ge);
-              ge = fmaf(x1, tv[8 * c + 2 * e + 1], ge);
-              gm = fmaf(x0, rbv[2 * e], gm);
-              gm = fmaf(x1, rbv[2 * e + 1], gm);
-            }
-          }
-        }
-        ge_acc[jb & 15] += (double)ge;
-        gmu_acc[jb & 15] += (double)gm;
-        tc_fence_before();
-        epi_barrier();
-        if (p.tim && blockIdx.x == 0 && ltile < 8 && threadIdx.x == 64 && jb == JB - 1) p.tim[ltile * 16 + 14] = clock64();
-        if (threadIdx.x == 64) {
-          mbar_arrive(smem_u32(&misc->t_empty[buf]));
-#pragma unroll
-          for (int i = 4; i < 8; ++i) mbar_arrive(smem_u32(&misc->empty[(fbase + G + 8 * jb + i) % kNumSlots]));
-        }
-      }
-    }
-    // -------- per-CTA partial sums (the operand ring is idle by now: use it as scratch) --------
-    double (*red)[kBM] = reinterpret_cast<double (*)[kBM]>(ring);
-    if (p.ll_total_only) {
-      // every thread holds a partial of the grand total: spread total / 256 over the columns
-      double tot = ll_acc[0];
-#pragma unroll
-      for (int o = 16; o > 0; o >>= 1) tot += __shfl_xor_sync(0xffffffffu, tot, o);
-      epi_barrier();
-      if (lane == 0) red[0][ew] = tot;
-      epi_barrier();
-      double s = 0.0;
-      for (int i = 0; i < kEpiWarps; ++i) s += red[0][i];
-      // (padded sample columns are masked out of spsum: subtracting their ln 2 afterwards would leave the fp32
-      // rounding of (256 - S) ln 2 per row in the total)
-      p.ll_part[(size_t)blockIdx.x * kSP + (threadIdx.x - 64)] = s / (double)p.S;
-    } else {
-      // lane l of (q,h) holds column 128h + 32c + l summed over rows of quarter q -> sum the 4 quarters
-      for (int c = 0; c < 4; ++c) {
-        epi_barrier();
-        if (q != 0) red[h][(q - 1) * 32 + lane] = ll_acc[c];       // 3 x 32 slots per column half
-        epi_barrier();
-        if (q == 0) {
-          const double s = ll_acc[c] + red[h][lane] + red[h][32 + lane] + red[h][64 + lane];
-          p.ll_part[(size_t)blockIdx.x * kSP + 128 * h + 32 * c + lane] = s;
-        }
-      }
-    }
-    if (p.want_grad) {
-      for (int jb = 0; jb < JB; ++jb) {
-        epi_barrier();
-        if (h == 1) {
-          red[0][row] = ge_acc[jb & 15];
-          red[1][row] = gmu_acc[jb & 15];
-        }
-        epi_barrier();
-        if (h == 0) {
-          p.ge_part[(size_t)blockIdx.x * p.d_pad + jb * 128 + row] = ge_acc[jb & 15] + red[0][row];
-          p.gmu_part[(size_t)blockIdx.x * p.d_pad + jb * 128 + row] = gmu_acc[jb & 15] + red[1][row];
-        }
-      }
-    }
-  }
-
-  tc_fence_before();
-  __syncthreads();
-  if (warp == 1) {
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"(kTmemCols) : "memory");
-  }
-}
-
 
 // =================================================================================================
-// CTA-pair kernel (cta_group::2): two CTAs of a cluster work on a 256-row super-tile.
+// The sweep kernel (cta_group::2): two CTAs of a cluster work on a 256-row super-tile.
 //   GEMM1  M = 256 (rank r owns rows 128r..128r+127), N = 256: each CTA stages only HALF of Theta^T per K stage
 //   GEMM2  M = 256 j (rank r owns j-block r of the 256-j pair block), N = 128 tile rows (64 from each CTA's R tile),
 //          two such units (tile-row halves) per group; each CTA stages only its half of E, one 16 KB slot per
@@ -688,8 +249,8 @@ glm_fast_kernel(const __grid_constant__ CUtensorMap tmXh, const __grid_constant_
 //   E2     reads its X values straight from global memory / L2 (256-bit evict-first loads; a thread owns column j,
 //          whose 64 rows of a tile half are one contiguous 128-byte run in the tile-transposed layout), so the
 //          operand ring only carries tensor-core operands
-// Operand fills per 128 rows drop from 1280 KB to 896 KB (d = 512), 640 KB of them through TMA -- the single-CTA
-// kernel is bound by the per-SM fill rate.  GEMM2 of super-tile i-1 is interleaved with GEMM1 of super-tile i (the
+// Pairing the CTAs takes the operand fills per 128 rows from 1280 KB (one CTA per tile, bound by the per-SM fill rate)
+// to 896 KB at d = 512, 640 KB of them through TMA.  GEMM2 of super-tile i-1 is interleaved with GEMM1 of super-tile i (the
 // R tile of i-1 stays valid until E1 of i starts, which is after every MMA issued before Z(i) was committed), so
 // the tensor pipe only idles during E1; one pool of 16 epilogue warps runs E2 of i-1 and then E1 of i.
 // Warps: 0 producer, 1 MMA (rank 0 issues for the pair), 2..17 epilogue (E2 of super-tile i-1, then E1 of i).
@@ -816,23 +377,22 @@ __device__ __forceinline__ void link_chunk_total(float (&v)[32], uint32_t (&pack
 }
 
 // Fill sequence of iteration i (identical in every role and in both CTAs; `fill` counts 16 KB slots):
-//   for kc in 0..KC-1:  slot A = X (hi n0 | hi n1 | lo n0 | lo n1), slot B = Theta_hi (2 groups) | Theta_lo (2 groups)
+//   for kc in 0..KC-1:  slot A = X_h (2 halves, 8 KB) | X_l8 | X_h8 (4 KB each: 32 j-rows x 128 n bytes),
+//                       slot B = Theta_h (2 groups, 8 KB) | Theta_h8 | Theta_l8 (this CTA's 128 samples)
 //       after the stages with (kc & 7) == 1 (and i > 0): the 4 E slots of GEMM2 group jbp = kc >> 3 of super-tile i-1,
 //       consumed after stage (kc & 7) == 3
 //   a last iteration i = nIter only carries the GEMM2 groups of the final super-tile.
-// FP8 (VB_FAST_FP8, tools/emulate_fp8_scheme.py): the two CORRECTION passes of GEMM1 run on e5m2 copies with reciprocal
-// power-of-two scales, (X_l 2^ax)(Theta_h 2^-ax) and (X_h 2^-bx)(Theta_l 2^bx), as kind::f8f6f4 (K = 32 per instruction,
-// twice the fp16 rate): their terms are 2^-11 of the product, so 3 significant bits per operand leave 2^-13 overall --
-// GEMM1 costs 1 + 1/2 + 1/2 pass units instead of 3.  A stage keeps its 2 x 16 KB: slot A = X_h (2 halves, 8 KB) | X_l8 |
-// X_h8 (4 KB each: 32 j-rows x 128 n bytes), slot B = Theta_h (2 groups, 8 KB) | Theta_h8 | Theta_l8 (this CTA's 128
-// samples).  E2 takes its X as X_h + X_l8 2^-ax (3 bytes per element from L2 instead of 4).
-template <bool FP8>
+// The two CORRECTION passes of GEMM1 run on e5m2 copies with reciprocal power-of-two scales
+// (tools/emulate_fp8_scheme.py), (X_l 2^ax)(Theta_h 2^-ax) and (X_h 2^-bx)(Theta_l 2^bx), as kind::f8f6f4 (K = 32 per
+// instruction, twice the fp16 rate): their terms are 2^-11 of the product, so 3 significant bits per operand leave
+// 2^-13 overall -- GEMM1 costs 1 + 1/2 + 1/2 fp16 pass units instead of 3.  E2 takes its X as X_h + X_l8 2^-ax
+// (3 bytes per element from L2 instead of 4).
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreadsP, 1)
-glm_fast_pair_kernel(const __grid_constant__ CUtensorMap tmX,      // 5-D: [hi|lo][tile][half][j][64 n]; FP8: 4-D [tile][half][j][64 n] (X_h)
-                     const __grid_constant__ CUtensorMap tmT,      // 4-D: [hi|lo][group][j][64 s];      FP8: 3-D [group][j][64 s] (Theta_h)
+glm_fast_pair_kernel(const __grid_constant__ CUtensorMap tmX,      // 4-D [tile][half][j][64 n] (X_h)
+                     const __grid_constant__ CUtensorMap tmT,      // 3-D [group][j][64 s] (Theta_h)
                      const __grid_constant__ CUtensorMap tmE,      // 3-D: [j group][s][64 j]
-                     const __grid_constant__ CUtensorMap tmX8,     // FP8: 4-D [X_l8|X_h8][tile][j][128 n] bytes
-                     const __grid_constant__ CUtensorMap tmT8,     // FP8: 4-D [Theta_h8|Theta_l8][group][j][128 s] bytes
+                     const __grid_constant__ CUtensorMap tmX8,     // 4-D [X_l8|X_h8][tile][j][128 n] bytes
+                     const __grid_constant__ CUtensorMap tmT8,     // 4-D [Theta_h8|Theta_l8][group][j][128 s] bytes
                      Params p) {
   extern __shared__ __align__(1024) uint8_t smem[];
   uint8_t* ring = smem;
@@ -881,7 +441,7 @@ glm_fast_pair_kernel(const __grid_constant__ CUtensorMap tmX,      // 5-D: [hi|l
     // ================================ TMA producer (both CTAs) ================================
     if (lane == 0) {
       prefetch_tmap(&tmX); prefetch_tmap(&tmT); prefetch_tmap(&tmE);
-      if (FP8) { prefetch_tmap(&tmX8); prefetch_tmap(&tmT8); }
+      prefetch_tmap(&tmX8); prefetch_tmap(&tmT8);
       uint32_t fill = 0, sc = 0, ec = 0;
       auto acquire = [&]() -> uint32_t {
         const uint32_t slot = fill % kNumSlots, par = (fill / kNumSlots) & 1;
@@ -909,17 +469,11 @@ glm_fast_pair_kernel(const __grid_constant__ CUtensorMap tmX,      // 5-D: [hi|l
             if (leader) mbar_expect_tx(bar_l, 4 * kSlotBytes);
             const uint32_t bar = mapa_u32(bar_l, 0);
             uint32_t dst = acquire();
-            if (FP8) {
-              tma_load_4d_pair(dst, &tmX, 0, j0, 0, tile, bar);            // X_h n0 | n1: 8 KB
-              tma_load_4d_pair(dst + 8192, &tmX8, 0, j0, tile, 0, bar);    // X_l8 | X_h8: 2 x 4 KB
-              dst = acquire();
-              tma_load_3d_pair(dst, &tmT, 0, j0, 2 * (int)rank, bar);      // Theta_h g0 | g1 (this CTA's half): 8 KB
-              tma_load_4d_pair(dst + 8192, &tmT8, 0, j0, (int)rank, 0, bar);   // Theta_h8 | Theta_l8 of its 128 samples
-            } else {
-              tma_load_5d_pair(dst, &tmX, 0, j0, 0, tile, 0, bar);         // hi n0 | hi n1 | lo n0 | lo n1: 16 KB
-              dst = acquire();
-              tma_load_4d_pair(dst, &tmT, 0, j0, 2 * (int)rank, 0, bar);   // Theta_hi g0 | g1 | Theta_lo g0 | g1 (this CTA's half)
-            }
+            tma_load_4d_pair(dst, &tmX, 0, j0, 0, tile, bar);            // X_h n0 | n1: 8 KB
+            tma_load_4d_pair(dst + 8192, &tmX8, 0, j0, tile, 0, bar);    // X_l8 | X_h8: 2 x 4 KB
+            dst = acquire();
+            tma_load_3d_pair(dst, &tmT, 0, j0, 2 * (int)rank, bar);      // Theta_h g0 | g1 (this CTA's half): 8 KB
+            tma_load_4d_pair(dst + 8192, &tmT8, 0, j0, (int)rank, 0, bar);   // Theta_h8 | Theta_l8 of its 128 samples
             if (grad && it > 0 && (kc & 7) == 1) g2_fills(kc >> 3);     // two stages ahead of the group that consumes them
           }
         } else if (grad && it > 0) {
@@ -973,36 +527,20 @@ glm_fast_pair_kernel(const __grid_constant__ CUtensorMap tmX,      // 5-D: [hi|l
           for (int kc = 0; kc < KC; ++kc, ++sc) {
             const uint32_t sa = fill % kNumSlots, sb = (fill + 1) % kNumSlots;
             fill += 2;
-            const uint32_t ax = ring_u + sa * kSlotBytes, bh = ring_u + sb * kSlotBytes, bl = bh + 8192;
+            const uint32_t ax = ring_u + sa * kSlotBytes, bh = ring_u + sb * kSlotBytes;
             const long long c0 = timing ? clock64() : 0;
             mbar_wait_cl(smem_u32(&misc->g1_full[sc % kFullRing]), (sc / kFullRing) & 1);
             if (timing) w_g1 += clock64() - c0;
             tc_fence_after();
-            if (FP8) {
-              if (elect_one()) {
-                constexpr uint32_t idesc8 = make_idesc8(256, 256, 1, 1);
+            if (elect_one()) {
+              constexpr uint32_t idesc8 = make_idesc8(256, 256, 1, 1);
 #pragma unroll
-                for (int k = 0; k < 2; ++k)                 // X_h . Theta_h, fp16, K = 16 each
-                  umma_f16_pair(tmem, make_desc(ax + k * 2048, 4096, 1024), make_desc(bh + k * 2048, 4096, 1024), idesc1,
-                                (kc | k) ? 1u : 0u);
-                // corrections, e5m2, K = 32: one 128-byte row holds all 128 rows / samples of this CTA (a single MN group)
-                umma_f8_pair(tmem, make_desc(ax + 8192, 4096, 1024), make_desc(bh + 8192, 4096, 1024), idesc8, 1u);     // X_l8 . Theta_h8
-                umma_f8_pair(tmem, make_desc(ax + 12288, 4096, 1024), make_desc(bh + 12288, 4096, 1024), idesc8, 1u);   // X_h8 . Theta_l8
-                umma_commit_pair(smem_u32(&misc->empty[sa]));
-                umma_commit_pair(smem_u32(&misc->empty[sb]));
-                if (kc == KC - 1) umma_commit_pair(smem_u32(&misc->z_full));
-              }
-            } else if (elect_one()) {
-#pragma unroll
-              for (int k = 0; k < 2; ++k)
-                umma_f16_pair(tmem, make_desc(ax + k * 2048, 4096, 1024), make_desc(bl + k * 2048, 4096, 1024), idesc1,
+              for (int k = 0; k < 2; ++k)                 // X_h . Theta_h, fp16, K = 16 each
+                umma_f16_pair(tmem, make_desc(ax + k * 2048, 4096, 1024), make_desc(bh + k * 2048, 4096, 1024), idesc1,
                               (kc | k) ? 1u : 0u);
-#pragma unroll
-              for (int k = 0; k < 2; ++k)
-                umma_f16_pair(tmem, make_desc(ax + k * 2048, 4096, 1024), make_desc(bh + k * 2048, 4096, 1024), idesc1, 1u);
-#pragma unroll
-              for (int k = 0; k < 2; ++k)
-                umma_f16_pair(tmem, make_desc(ax + 8192 + k * 2048, 4096, 1024), make_desc(bh + k * 2048, 4096, 1024), idesc1, 1u);
+              // corrections, e5m2, K = 32: one 128-byte row holds all 128 rows / samples of this CTA (a single MN group)
+              umma_f8_pair(tmem, make_desc(ax + 8192, 4096, 1024), make_desc(bh + 8192, 4096, 1024), idesc8, 1u);     // X_l8 . Theta_h8
+              umma_f8_pair(tmem, make_desc(ax + 12288, 4096, 1024), make_desc(bh + 12288, 4096, 1024), idesc8, 1u);   // X_h8 . Theta_l8
               umma_commit_pair(smem_u32(&misc->empty[sa]));
               umma_commit_pair(smem_u32(&misc->empty[sb]));
               if (kc == KC - 1) umma_commit_pair(smem_u32(&misc->z_full));
@@ -1051,24 +589,16 @@ glm_fast_pair_kernel(const __grid_constant__ CUtensorMap tmX,      // 5-D: [hi|l
     auto e2_group = [&](int itp, int jbp) {      // GEMM2 group jbp of iteration itp: this warp's 64 tile rows
       const int sup = cluster_id + itp * num_clusters;
       const int j = jbp * 256 + 128 * (int)rank + row;
-      // this thread's X values: column j, the 64 rows of half nh2 of tile t2 (128 contiguous bytes), hi and lo
+      // this thread's X values: column j, the 64 rows of half nh2 of tile t2 (128 contiguous bytes of X_h, 64 of X_l8)
       const __half* xhp = p.Xh + ((size_t)((2 * sup + t2) * 2 + nh2) * p.d_pad + j) * 64;
-      const __half* xlp = p.Xl + ((size_t)((2 * sup + t2) * 2 + nh2) * p.d_pad + j) * 64;
-      uint32_t xa[32], xb[32];                   // [0,16): hi, [16,32): lo of a 32-row step (FP8: [16,24) = 32 e5m2 bytes)
+      uint32_t xa[32], xb[32];                   // [0,16): hi, [16,24): 32 e5m2 bytes of lo, of a 32-row step
       ldg256(xhp, xa);                           // X does not depend on the MMA: in flight while waiting
       ldg256(xhp + 16, xa + 8);
       ldg256(xhp + 32, xb);
       ldg256(xhp + 48, xb + 8);
-      if (FP8) {
-        const uint8_t* xl8 = p.Xl8 + ((size_t)(2 * sup + t2) * p.d_pad + j) * 128 + 64 * nh2;
-        ldg256(xl8, xa + 16);
-        ldg256(xl8 + 32, xb + 16);
-      } else {
-        ldg256(xlp, xa + 16);
-        ldg256(xlp + 16, xa + 24);
-        ldg256(xlp + 32, xb + 16);
-        ldg256(xlp + 48, xb + 24);
-      }
+      const uint8_t* xl8 = p.Xl8 + ((size_t)(2 * sup + t2) * p.d_pad + j) * 128 + 64 * nh2;
+      ldg256(xl8, xa + 16);
+      ldg256(xl8 + 32, xb + 16);
       float ge = 0.0f, gm = 0.0f;
       auto compute = [&](const uint32_t* x, int part) {
         const float* rbp = &misc->rb[itp & 1][128 * t2 + 64 * nh2 + 32 * part];
@@ -1077,18 +607,11 @@ glm_fast_pair_kernel(const __grid_constant__ CUtensorMap tmX,      // 5-D: [hi|l
 #pragma unroll
         for (int e = 0; e < 16; ++e) {
           const float2 fh2 = __half22float2(*reinterpret_cast<const __half2*>(&x[e]));
-          float x0, x1;
-          if (FP8) {
-            // an e5m2 byte is the high byte of the fp16 with the same value: spread two bytes into an fp16 pair
-            const uint32_t h2 = __byte_perm(x[16 + (e >> 1)], 0u, (e & 1) ? 0x3424u : 0x1404u);
-            const float2 fl2 = __half22float2(*reinterpret_cast<const __half2*>(&h2));
-            x0 = fmaf(fl2.x, p.xl_scale, fh2.x);
-            x1 = fmaf(fl2.y, p.xl_scale, fh2.y);
-          } else {
-            const float2 fl2 = __half22float2(*reinterpret_cast<const __half2*>(&x[16 + e]));
-            x0 = fh2.x + fl2.x;
-            x1 = fh2.y + fl2.y;
-          }
+          // an e5m2 byte is the high byte of the fp16 with the same value: spread two bytes into an fp16 pair
+          const uint32_t h2 = __byte_perm(x[16 + (e >> 1)], 0u, (e & 1) ? 0x3424u : 0x1404u);
+          const float2 fl2 = __half22float2(*reinterpret_cast<const __half2*>(&h2));
+          const float x0 = fmaf(fl2.x, p.xl_scale, fh2.x);
+          const float x1 = fmaf(fl2.y, p.xl_scale, fh2.y);
           const float2 rb2 = *reinterpret_cast<const float2*>(rbp + 2 * e);
           ge = fmaf(x0, tv[2 * e], ge);
           ge = fmaf(x1, tv[2 * e + 1], ge);
@@ -1328,10 +851,10 @@ __global__ void fast_prepare_x8_kernel(const __half* __restrict__ Xh, const __ha
   }
 }
 
-// Theta^T hi/lo [4][d_pad][64], E [d_pad/64][256][64] (fp16) and weights, zero padded
+// Theta^T hi [4][d_pad][64], E [d_pad/64][256][64] (fp16), the e5m2 Theta copies and weights, zero padded
 __global__ void fast_prepare_theta_kernel(const double* __restrict__ theta, const double* __restrict__ base,
                                           const double* __restrict__ w, int64_t S, int d, int d_pad,
-                                          __half* __restrict__ Th, __half* __restrict__ Tl, __half* __restrict__ E,
+                                          __half* __restrict__ Th, __half* __restrict__ E,
                                           float* __restrict__ wf, uint8_t* __restrict__ T8, int ax, int bx) {
   PDL_SYNC();
   const int64_t total = (int64_t)kSP * d_pad;
@@ -1352,13 +875,9 @@ __global__ void fast_prepare_theta_kernel(const double* __restrict__ theta, cons
       const size_t o = ((size_t)(s >> 6) * d_pad + j) * 64 + (s & 63);
       Th[o] = hi;
       const float lof = t - __half2float(hi);       // fp32 residual: the e5m2 copy must not inherit an fp16 underflow
-      const __half lo = __float2half_rn(lof);
-      Tl[o] = lo;
-      if (T8) {
-        const size_t o8 = ((size_t)(s >> 7) * d_pad + j) * 128 + (s & 127);
-        T8[o8] = to_e5m2(__half2float(hi) * exp2f((float)-ax));
-        T8[(size_t)2 * d_pad * 128 + o8] = to_e5m2(lof * exp2f((float)bx));
-      }
+      const size_t o8 = ((size_t)(s >> 7) * d_pad + j) * 128 + (s & 127);
+      T8[o8] = to_e5m2(__half2float(hi) * exp2f((float)-ax));
+      T8[(size_t)2 * d_pad * 128 + o8] = to_e5m2(lof * exp2f((float)bx));
     }
   }
   for (int64_t s = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; s < kSP; s += (int64_t)gridDim.x * blockDim.x)
@@ -1434,27 +953,18 @@ static bool encode_nd(CUtensorMap* map, const void* base, int rank, const uint64
                    CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   return r == CUDA_SUCCESS;
 }
-// 2-D view [rows][64] with a [box_rows][64] box (the one-CTA kernel)
-static bool encode_2d(CUtensorMap* map, const void* base, uint64_t rows, uint32_t box_rows) {
-  const uint64_t dims[2] = {64, rows}, strides[1] = {128};
-  const uint32_t box[2] = {64, box_rows};
-  return encode_nd(map, base, 2, dims, strides, box);
-}
 
 struct FastModel {
   int64_t N, numTiles;
   int d, d_pad;
   const __half* Xh;
-  const __half* Xl;
-  CUtensorMap tmXh, tmXl, tmXh2, tmXl2;      // one-CTA kernel: 2-D views
-  CUtensorMap tmXP;                          // pair kernel: 5-D [hi|lo][tile][half][j][64]
-  const uint8_t* X8;                         // fp8 scheme: e5m2 [X_l 2^ax | X_h 2^-bx][tile][d_pad][128]
+  const uint8_t* X8;                         // e5m2 [X_l 2^ax | X_h 2^-bx][tile][d_pad][128]
   int ax, bx;
-  CUtensorMap tmXP16, tmXP8;                 // fp8 scheme: 4-D [tile][half][j][64] over X_h; 4-D [which][tile][j][128] bytes
+  CUtensorMap tmXP16, tmXP8;                 // 4-D [tile][half][j][64] over X_h; 4-D [which][tile][j][128] bytes
 };
 
 struct FastLayout {
-  size_t off_Th, off_Tl, off_E, off_w, off_ll, off_gmu, off_ge, off_T8, total;
+  size_t off_Th, off_E, off_w, off_ll, off_gmu, off_ge, off_T8, total;
   int grid;
 };
 
@@ -1466,7 +976,6 @@ static void fast_layout(int64_t N, int d_pad, FastLayout& L) {
   size_t off = 0;
   auto take = [&](size_t bytes) { size_t o = off; off = align_up(off + bytes, 1024); return o; };
   L.off_Th = take((size_t)kSP * d_pad * 2);
-  L.off_Tl = take((size_t)kSP * d_pad * 2);
   L.off_E = take((size_t)kSP * d_pad * 2);
   L.off_w = take(kSP * sizeof(float));
   L.off_ll = take((size_t)L.grid * kSP * sizeof(double));
@@ -1516,7 +1025,6 @@ extern "C" int vb_glm_fast_create(void** handle, const double* X, int64_t ldx, c
   __half* Xl = Xh + elems;
   float* absmax = reinterpret_cast<float*>(Xl + elems);
   m->Xh = Xh;
-  m->Xl = Xl;
   cudaError_t e = cudaMemsetAsync(absmax, 0, 16, stream);          // [0]: max |y X| (float), [2..3]: sum of squares (double)
   if (e != cudaSuccess) { delete m; return set_cuda_error(e); }
   fast_prepare_x_kernel<<<sm_count() * 8, 256, 0, stream>>>(X, ldx, y, N, d, m->numTiles, m->d_pad, Xh, Xl, absmax);
@@ -1556,15 +1064,6 @@ extern "C" int vb_glm_fast_create(void** handle, const double* X, int64_t ldx, c
                                                                exp2f((float)-m->bx), X8);
     e = cudaGetLastError();
     if (e != cudaSuccess) { delete m; return set_cuda_error(e); }
-  }
-  const uint64_t rows = (uint64_t)m->numTiles * 2 * m->d_pad;
-  const uint64_t xd[5] = {64, (uint64_t)m->d_pad, 2, (uint64_t)m->numTiles, 2};
-  const uint64_t xs[4] = {128, (uint64_t)m->d_pad * 128, (uint64_t)m->d_pad * 256, (uint64_t)elems * 2};
-  const uint32_t xb[5] = {64, 32, 2, 1, 2};
-  if (!encode_2d(&m->tmXh, Xh, rows, 32) || !encode_2d(&m->tmXl, Xl, rows, 32) || !encode_2d(&m->tmXh2, Xh, rows, 64) ||
-      !encode_2d(&m->tmXl2, Xl, rows, 64) || !encode_nd(&m->tmXP, Xh, 5, xd, xs, xb)) {
-    delete m;
-    return set_error(VB_ERR_CUDA, "glm_fast_create: cuTensorMapEncodeTiled failed");
   }
   const uint64_t x16d[4] = {64, (uint64_t)m->d_pad, 2, (uint64_t)m->numTiles};
   const uint64_t x16s[3] = {128, (uint64_t)m->d_pad * 128, (uint64_t)m->d_pad * 256};
@@ -1609,7 +1108,6 @@ int fast_operands(void* handle, void* workspace, size_t workspace_bytes, FastOpe
     return set_error(VB_ERR_INVALID_ARG, "glm_fast_sweep: workspace must be 1024-byte aligned");
   char* ws = static_cast<char*>(workspace);
   ops->Th = reinterpret_cast<__half*>(ws + L.off_Th);
-  ops->Tl = reinterpret_cast<__half*>(ws + L.off_Tl);
   ops->E = reinterpret_cast<__half*>(ws + L.off_E);
   ops->wf = reinterpret_cast<float*>(ws + L.off_w);
   ops->T8 = reinterpret_cast<uint8_t*>(ws + L.off_T8);
@@ -1618,7 +1116,7 @@ int fast_operands(void* handle, void* workspace, size_t workspace_bytes, FastOpe
   return VB_OK;
 }
 
-// Launches the sweep kernel on operands already packed into the workspace (Th, Tl, E, wf); the per-CTA / per-pair
+// Launches the sweep kernel on operands already packed into the workspace (Th, E, wf, T8); the per-CTA / per-pair
 // partial sums stay in the workspace and are described by `parts` (ll partials are sums of softplus: sign -1).
 int fast_launch(void* handle, void* workspace, size_t workspace_bytes, int S, int want_grad, int ll_total_only,
                 int uniform_w, float* debug, cudaStream_t stream, FastPartials* parts) {
@@ -1637,29 +1135,19 @@ int fast_launch(void* handle, void* workspace, size_t workspace_bytes, int S, in
   static thread_local const void* cached_ws = nullptr;
   static thread_local const void* cached_t8 = nullptr;
   static thread_local int cached_dpad = 0;
-  static thread_local CUtensorMap tmTh, tmTl, tmE, tmTP, tmEP, tmTP16, tmTP8;
-  // VB_FAST_FP8=0 selects the three-fp16-pass GEMM1 (A/B measurements)
-  static const bool use_fp8 = [] { const char* e = getenv("VB_FAST_FP8"); return !(e && e[0] == '0'); }();
+  static thread_local CUtensorMap tmTP16, tmEP, tmTP8;
   if (cached_ws != workspace || cached_dpad != m->d_pad || cached_t8 != ops.T8) {
     cached_ws = nullptr;           // a failed encode below leaves no valid entry behind
     const uint64_t dp = (uint64_t)m->d_pad;
-    const uint64_t td[4] = {64, dp, 4, 2}, ts[3] = {128, dp * 128, dp * 512};      // Tl follows Th
-    const uint32_t tb[4] = {64, 32, 2, 2};
-    const uint64_t ed[3] = {64, (uint64_t)kSP, dp / 64}, es[2] = {128, (uint64_t)kSP * 128};
-    const uint32_t eb[3] = {64, 64, 2};
-    if (reinterpret_cast<char*>(ops.Tl) - reinterpret_cast<char*>(ops.Th) != (ptrdiff_t)(dp * 512))
-      return set_error(VB_ERR_CUDA, "glm_fast_sweep: Theta hi/lo are not adjacent");
-    if (!encode_2d(&tmTh, ops.Th, 4 * dp, 32) || !encode_2d(&tmTl, ops.Tl, 4 * dp, 32) ||
-        !encode_2d(&tmE, ops.E, (dp / 64) * kSP, 64) || !encode_nd(&tmTP, ops.Th, 4, td, ts, tb) ||
-        !encode_nd(&tmEP, ops.E, 3, ed, es, eb))
-      return set_error(VB_ERR_CUDA, "glm_fast_sweep: cuTensorMapEncodeTiled failed");
     const uint64_t t16d[3] = {64, dp, 4}, t16s[2] = {128, dp * 128};
     const uint32_t t16b[3] = {64, 32, 2};
+    const uint64_t ed[3] = {64, (uint64_t)kSP, dp / 64}, es[2] = {128, (uint64_t)kSP * 128};
+    const uint32_t eb[3] = {64, 64, 2};
     const uint64_t t8d[4] = {128, dp, 2, 2}, t8s[3] = {128, dp * 128, dp * 256};
     const uint32_t t8b[4] = {128, 32, 1, 2};
-    if (!encode_nd(&tmTP16, ops.Th, 3, t16d, t16s, t16b) ||
+    if (!encode_nd(&tmTP16, ops.Th, 3, t16d, t16s, t16b) || !encode_nd(&tmEP, ops.E, 3, ed, es, eb) ||
         !encode_nd(&tmTP8, ops.T8, 4, t8d, t8s, t8b, CU_TENSOR_MAP_DATA_TYPE_UINT8))
-      return set_error(VB_ERR_CUDA, "glm_fast_sweep: cuTensorMapEncodeTiled failed (fp8 operands)");
+      return set_error(VB_ERR_CUDA, "glm_fast_sweep: cuTensorMapEncodeTiled failed");
     cached_ws = workspace;
     cached_t8 = ops.T8;
     cached_dpad = m->d_pad;
@@ -1676,15 +1164,11 @@ int fast_launch(void* handle, void* workspace, size_t workspace_bytes, int S, in
   p.ll_part = reinterpret_cast<double*>(ws + L.off_ll);
   p.gmu_part = reinterpret_cast<double*>(ws + L.off_gmu);
   p.ge_part = reinterpret_cast<double*>(ws + L.off_ge);
-  p.dbg = debug;
   p.tim = debug ? reinterpret_cast<long long*>(debug + (size_t)49152 * L.grid) : nullptr;
   p.Xh = m->Xh;
-  p.Xl = m->Xl;
   p.Xl8 = m->X8;
   p.xl_scale = exp2f((float)-m->ax);
   p.uniform_w = uniform_w;
-  // kernel choice: the CTA-pair kernel unless the device cannot co-schedule clusters of two such CTAs
-  // (VB_FAST_KERNEL=single forces the one-CTA kernel, for A/B measurements)
   int pair_clusters = 0;
   {
     // function attributes and the cluster occupancy are per device: cache them per device ordinal, under a lock
@@ -1696,69 +1180,55 @@ int fast_launch(void* handle, void* workspace, size_t workspace_bytes, int S, in
     if (dev < 0 || dev >= 64) return set_error(VB_ERR_UNSUPPORTED, "glm_fast_sweep: device ordinal out of range");
     std::lock_guard<std::mutex> lock(mu);
     if (!ready[dev]) {
-      VB_CUDA(cudaFuncSetAttribute(glm_fast_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes));
-      VB_CUDA(cudaFuncSetAttribute(glm_fast_pair_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes));
-      VB_CUDA(cudaFuncSetAttribute(glm_fast_pair_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes));
-      const char* env = getenv("VB_FAST_KERNEL");
+      VB_CUDA(cudaFuncSetAttribute(glm_fast_pair_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes));
       int nc = 0;
-      if (!(env && strcmp(env, "single") == 0)) {
-        cudaLaunchConfig_t qc = {};
-        qc.gridDim = dim3(sm_count() & ~1);
-        qc.blockDim = dim3(kThreadsP);
-        qc.dynamicSmemBytes = kSmemBytes;
-        cudaLaunchAttribute qa[1];
-        qa[0].id = cudaLaunchAttributeClusterDimension;
-        qa[0].val.clusterDim.x = 2;
-        qa[0].val.clusterDim.y = 1;
-        qa[0].val.clusterDim.z = 1;
-        qc.attrs = qa;
-        qc.numAttrs = 1;
-        if (cudaOccupancyMaxActiveClusters(&nc, glm_fast_pair_kernel<true>, &qc) != cudaSuccess) {
-          cudaGetLastError();
-          nc = 0;
-        }
+      cudaLaunchConfig_t qc = {};
+      qc.gridDim = dim3(sm_count() & ~1);
+      qc.blockDim = dim3(kThreadsP);
+      qc.dynamicSmemBytes = kSmemBytes;
+      cudaLaunchAttribute qa[1];
+      qa[0].id = cudaLaunchAttributeClusterDimension;
+      qa[0].val.clusterDim.x = 2;
+      qa[0].val.clusterDim.y = 1;
+      qa[0].val.clusterDim.z = 1;
+      qc.attrs = qa;
+      qc.numAttrs = 1;
+      if (cudaOccupancyMaxActiveClusters(&nc, glm_fast_pair_kernel, &qc) != cudaSuccess) {
+        cudaGetLastError();
+        nc = 0;
       }
       cached[dev] = nc;
       ready[dev] = true;
     }
     pair_clusters = cached[dev];
   }
-  int nblk_ll = L.grid, nblk_g = L.grid;
-  if (pair_clusters > 0) {
-    const int64_t numSuper = m->numTiles / 2;
-    int clusters = pair_clusters < L.grid / 2 ? pair_clusters : L.grid / 2;
-    if (clusters < 1) clusters = 1;
-    if (numSuper < clusters) clusters = (int)numSuper;
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3(2 * clusters);
-    cfg.blockDim = dim3(kThreadsP);
-    cfg.dynamicSmemBytes = kSmemBytes;
-    cfg.stream = stream;
-    cudaLaunchAttribute at[2];
-    at[0].id = cudaLaunchAttributeClusterDimension;
-    at[0].val.clusterDim.x = 2;
-    at[0].val.clusterDim.y = 1;
-    at[0].val.clusterDim.z = 1;
-    at[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    at[1].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = at;
-    cfg.numAttrs = 2;
-    if (use_fp8)
-      VB_CUDA(cudaLaunchKernelEx(&cfg, glm_fast_pair_kernel<true>, m->tmXP16, tmTP16, tmEP, m->tmXP8, tmTP8, p));
-    else
-      VB_CUDA(cudaLaunchKernelEx(&cfg, glm_fast_pair_kernel<false>, m->tmXP, tmTP, tmEP, m->tmXP8, tmTP8, p));
-    nblk_ll = 2 * clusters;
-    nblk_g = clusters;              // one row of gradient partials per pair (a CTA owns half of the columns)
-  } else {
-    glm_fast_kernel<<<L.grid, kThreads, kSmemBytes, stream>>>(m->tmXh, m->tmXl, m->tmXh2, m->tmXl2, tmTh, tmTl, tmE, p);
-    VB_CHECK_LAUNCH();
-  }
+  if (pair_clusters <= 0)
+    return set_error(VB_ERR_UNSUPPORTED, "glm_fast_sweep: the CTA-pair kernel cannot be scheduled on this device; use the float64 path");
+  const int64_t numSuper = m->numTiles / 2;
+  int clusters = pair_clusters < L.grid / 2 ? pair_clusters : L.grid / 2;
+  if (clusters < 1) clusters = 1;
+  if (numSuper < clusters) clusters = (int)numSuper;
+  cudaLaunchConfig_t cfg = {};
+  cfg.gridDim = dim3(2 * clusters);
+  cfg.blockDim = dim3(kThreadsP);
+  cfg.dynamicSmemBytes = kSmemBytes;
+  cfg.stream = stream;
+  cudaLaunchAttribute at[2];
+  at[0].id = cudaLaunchAttributeClusterDimension;
+  at[0].val.clusterDim.x = 2;
+  at[0].val.clusterDim.y = 1;
+  at[0].val.clusterDim.z = 1;
+  at[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+  at[1].val.programmaticStreamSerializationAllowed = 1;
+  cfg.attrs = at;
+  cfg.numAttrs = 2;
+  VB_CUDA(cudaLaunchKernelEx(&cfg, glm_fast_pair_kernel, m->tmXP16, tmTP16, tmEP, m->tmXP8, tmTP8, p));
   if (parts) {
     parts->ll_part = p.ll_part;
     parts->gmu_part = p.gmu_part;
     parts->ge_part = p.ge_part;
-    parts->nblk_ll = nblk_ll;
-    parts->nblk_g = nblk_g;
+    parts->nblk_ll = 2 * clusters;
+    parts->nblk_g = clusters;       // one row of gradient partials per pair (a CTA owns half of the columns)
     parts->stride_ll = kSP;
     parts->stride_g = m->d_pad;
   }
@@ -1772,7 +1242,7 @@ extern "C" int vb_glm_fast_sweep(void* handle, const double* theta, const double
                                  int want_grad, double* out_ll, double* out_gmu, double* out_ge, void* workspace,
                                  size_t workspace_bytes, float* debug, cudaStream_t stream) {
   // want_grad bit 0: gradients wanted; bit 1: only sum_s ll[s] is needed (each out_ll[s] receives the mean)
-  // (debug + 49152*grid floats, when debug is given, is followed by 128 int64 timestamp slots)
+  // (when debug is given, debug + 49152*grid floats holds 128 int64 clock64 timestamp slots of CTA 0)
   FastModel* m = static_cast<FastModel*>(handle);
   const int ll_total_only = (want_grad >> 1) & 1;
   want_grad &= 1;
@@ -1783,7 +1253,7 @@ extern "C" int vb_glm_fast_sweep(void* handle, const double* theta, const double
   int rc = fast_operands(handle, workspace, workspace_bytes, &ops);
   if (rc) return rc;
   VB_CUDA(launch_pdl(fast_prepare_theta_kernel, dim3(128), dim3(256), stream, theta, want_grad ? base : nullptr, w, S, m->d, m->d_pad,
-                     ops.Th, ops.Tl, ops.E, ops.wf, ops.T8, ops.ax, ops.bx));
+                     ops.Th, ops.E, ops.wf, ops.T8, ops.ax, ops.bx));
   FastPartials parts;
   rc = fast_launch(handle, workspace, workspace_bytes, (int)S, want_grad, ll_total_only, w ? 0 : 1, debug, stream, &parts);
   if (rc) return rc;

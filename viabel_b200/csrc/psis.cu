@@ -347,141 +347,6 @@ __global__ void __launch_bounds__(kSelThreads) psis_sample_select_kernel(const d
 // memory and flushed with ONE global atomic per CTA (same-address atomics with a return value
 // serialise at ~2 ns each in L2: one per candidate-bearing warp iteration cost more than the HBM pass).
 constexpr int kStage = 64;      // per-warp staging entries (>= 2 * 32: every push of up to 32 candidates checks for room)
-__global__ void __launch_bounds__(256) psis_pass_a_kernel(const double* __restrict__ lw, int64_t n, int64_t idx_off,
-                                                          PsisScalars* sc, double* __restrict__ cand_x,
-                                                          int64_t* __restrict__ cand_i, unsigned int cap,
-                                                          double* __restrict__ blk_sum) {
-  __shared__ double red[32];
-  __shared__ unsigned long long redk[32];
-  __shared__ double etab_s[kExpTab];
-  __shared__ double sx[8][kStage];
-  __shared__ long long si[8][kStage];
-  __shared__ unsigned int wcnt[8], cta_base;
-  const uint32_t etab = load_exp_table(etab_s);
-  const double t0 = sc->t0;
-  const bool all = !(t0 > -INFINITY);       // threshold -inf: everything is a candidate
-  // single comparison x >= thr: in exact mode candidates are STRICTLY above t0
-  const double thr = all ? -INFINITY : (sc->strict ? nextafter(t0, INFINITY) : t0);
-  if (blockIdx.x == 0 && threadIdx.x == 0) sc->tbase = t0;         // this version's sums are relative to t0 itself
-  double mx = -INFINITY, acc0 = 0.0, acc1 = 0.0;
-  const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
-  const int64_t nthreads = (int64_t)gridDim.x * blockDim.x;
-  const int64_t tid = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
-  unsigned int staged = 0;                  // warp-uniform number of staged candidates
-  auto flush_warp = [&]() {
-    unsigned int base = 0;
-    if (lane == 0) base = atomicAdd(&sc->ncand, staged);
-    base = __shfl_sync(0xffffffffu, base, 0);
-    for (unsigned int i = lane; i < staged; i += 32)
-      if (base + i < cap) {
-        cand_x[base + i] = sx[w][i];
-        cand_i[base + i] = si[w][i];
-      }
-    __syncwarp();
-    staged = 0;
-  };
-  auto push = [&](double x, int64_t i, bool is_cand) {
-    const unsigned int ball = __ballot_sync(0xffffffffu, is_cand);
-    if (ball) {
-      if (is_cand) {
-        mx = fmax(mx, x);
-        const unsigned int slot = staged + __popc(ball & ((1u << lane) - 1));
-        sx[w][slot] = x;
-        si[w][slot] = i + idx_off;      // global draw index (idx_off = this rank's first draw)
-      }
-      staged += __popc(ball);
-    }
-  };
-  const bool aligned = (reinterpret_cast<uintptr_t>(lw) & 31) == 0;
-  int64_t done = 0;
-  if (aligned && !all) {
-    // 2 x LDG.128 per thread per iteration (4 doubles), warp-uniform trip count
-    const int64_t n4 = n / 4;
-    const int64_t iters = (n4 + nthreads - 1) / nthreads;
-    const double2 ninf = make_double2(-INFINITY, -INFINITY);
-    double2 na = ninf, nb = ninf;                     // software pipeline: next iteration's loads in flight
-    if (tid < n4) {
-      na = __ldcs(reinterpret_cast<const double2*>(lw) + 2 * tid);
-      nb = __ldcs(reinterpret_cast<const double2*>(lw) + 2 * tid + 1);
-    }
-    for (int64_t it = 0; it < iters; ++it) {
-      const int64_t q = it * nthreads + tid;
-      const double2 a = na, b = nb;
-      const int64_t qn = q + nthreads;
-      na = ninf;
-      nb = ninf;
-      if (qn < n4) {
-        na = __ldcs(reinterpret_cast<const double2*>(lw) + 2 * qn);
-        nb = __ldcs(reinterpret_cast<const double2*>(lw) + 2 * qn + 1);
-      }
-      const bool c0 = a.x >= thr, c1 = a.y >= thr, c2 = b.x >= thr, c3 = b.y >= thr;
-      // exponentials of the (overwhelmingly common) non-candidates: two independent chains
-      const double e0 = exp_nonpos(a.x - t0, etab), e1 = exp_nonpos(a.y - t0, etab);
-      const double e2 = exp_nonpos(b.x - t0, etab), e3 = exp_nonpos(b.y - t0, etab);
-      acc0 += (c0 ? 0.0 : e0) + (c2 ? 0.0 : e2);
-      acc1 += (c1 ? 0.0 : e1) + (c3 ? 0.0 : e3);
-      if (__any_sync(0xffffffffu, c0 | c1 | c2 | c3)) {
-        if (staged + 32 > kStage) flush_warp();
-        push(a.x, 4 * q, c0);
-        if (staged + 32 > kStage) flush_warp();
-        push(a.y, 4 * q + 1, c1);
-        if (staged + 32 > kStage) flush_warp();
-        push(b.x, 4 * q + 2, c2);
-        if (staged + 32 > kStage) flush_warp();
-        push(b.y, 4 * q + 3, c3);
-      }
-    }
-    done = n4 * 4;
-  }
-  {   // remainder (and the whole array when unaligned or when everything is a candidate)
-    const int64_t rest = n - done;
-    const int64_t iters = (rest + nthreads - 1) / nthreads;
-    for (int64_t it = 0; it < iters; ++it) {
-      const int64_t i = done + it * nthreads + tid;
-      const bool v = i < n;
-      const double x = v ? lw[i] : -INFINITY;
-      const bool c = v && (all || x >= thr);
-      if (v && !c) acc0 += exp_nonpos(x - t0, etab);
-      if (staged + 32 > kStage) flush_warp();
-      push(x, i, c);
-    }
-  }
-  // block reductions and the single per-CTA flush of the staged candidates
-  double acc = warp_sum(acc0 + acc1);
-  unsigned long long mk = dkey(mx);
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) {
-    unsigned long long t = __shfl_xor_sync(0xffffffffu, mk, o);
-    mk = t > mk ? t : mk;
-  }
-  if (lane == 0) { red[w] = acc; redk[w] = mk; wcnt[w] = staged; }
-  __syncthreads();
-  if (w == 0) {
-    double a = lane < 8 ? red[lane] : 0.0;
-    unsigned long long k = lane < 8 ? redk[lane] : 0ull;
-    unsigned int c = lane < 8 ? wcnt[lane] : 0u;
-    a = warp_sum(a);
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) {
-      unsigned long long t = __shfl_xor_sync(0xffffffffu, k, o);
-      k = t > k ? t : k;
-      c += __shfl_xor_sync(0xffffffffu, c, o);
-    }
-    if (lane == 0) {
-      blk_sum[blockIdx.x] = a;
-      if (k > dkey(-INFINITY)) atomicMax(&sc->maxkey, k);
-      cta_base = c ? atomicAdd(&sc->ncand, c) : 0u;
-    }
-  }
-  __syncthreads();
-  unsigned int base = cta_base;
-  for (int u = 0; u < w; ++u) base += wcnt[u];
-  for (unsigned int i = lane; i < staged; i += 32)
-    if (base + i < cap) {
-      cand_x[base + i] = sx[w][i];
-      cand_i[base + i] = si[w][i];
-    }
-}
 
 // linear value bins of the candidate histogram over [t0, hist_hi] (monotone in x)
 __device__ __forceinline__ unsigned int cbin(double x, double lo, double scale) {
@@ -513,7 +378,7 @@ __device__ __forceinline__ double exp_core(double d, uint32_t tab) {
   return __hiloint2double(__double2hiint(v) + ((n & ~(kExpTab - 1)) << 12), __double2loint(v));
 }
 
-// pass A, lean form.  What the profile of the first version showed: 150 instructions per 4 draws of which only 52
+// pass A, lean form.  A plain loop over predicated quads profiled at 150 instructions per 4 draws of which only 52
 // are double-precision arithmetic -- the rest were the two selects per draw (candidate, underflow), the -inf
 // initialisation of predicated loads, register copies of the software pipeline and 64-bit index arithmetic.  Here
 // the main loop covers only iterations in which every thread has a full quad (no predication), is unrolled by two so
@@ -1708,12 +1573,6 @@ static void psis_ptrs(char* ws, const PsisPlan& p, PsisPtrs& q) {
 }
 
 // stage 1 (per rank): threshold, pass A over this rank's draws
-// VB_PSIS_PASS_A=v1 selects the first version of the kernel (A/B timing)
-static bool pass_a_v1() {
-  static const bool v1 = [] { const char* e = getenv("VB_PSIS_PASS_A"); return e && e[0] == 'v' && e[1] == '1'; }();
-  return v1;
-}
-
 static int psis_stage_local(const double* lw, int64_t n, int64_t idx_off, int exact, const PsisPlan& p, PsisPtrs& q,
                             cudaStream_t stream, int onepass = 0) {
   psis_init_kernel<<<8, 1024, 0, stream>>>(q.sc, p.M, q.ghist, q.vhist, onepass, (long long)n);
@@ -1739,8 +1598,6 @@ static int psis_stage_local(const double* lw, int64_t n, int64_t idx_off, int ex
   }
   if (onepass)
     psis_pass_a_lean_kernel<true><<<p.grid, 256, 0, stream>>>(lw, n, idx_off, q.sc, q.candx, q.candi, p.cap, q.blk, q.mom, q.ghist);
-  else if (pass_a_v1())
-    psis_pass_a_kernel<<<p.grid, 256, 0, stream>>>(lw, n, idx_off, q.sc, q.candx, q.candi, p.cap, q.blk);
   else
     psis_pass_a_lean_kernel<false><<<p.grid, 256, 0, stream>>>(lw, n, idx_off, q.sc, q.candx, q.candi, p.cap, q.blk, q.mom, q.ghist);
   VB_CHECK_LAUNCH();
@@ -1750,7 +1607,7 @@ static int psis_stage_local(const double* lw, int64_t n, int64_t idx_off, int ex
 // stage 2 (replicated): cutoff, tail ranking, GPD fit, smoothed values, log-sum-exp from the candidate list
 static int psis_stage_select(const PsisPlan& p, PsisPtrs& q, int nblk, int raw, cudaStream_t stream, bool need_hist) {
   const int cgrid = sm_count() * 2;
-  if (need_hist)      // the lean pass A has filled the histogram already
+  if (need_hist)      // pass A fills the histogram itself; candidates imported from records need it built here
     VB_CUDA(launch_pdl(psis_cand_hist_kernel, dim3(cgrid), dim3(256), stream, q.sc, q.candx, p.cap, q.ghist));
   VB_CUDA(launch_pdl(psis_cand_gather_kernel, dim3(cgrid / 4 > 0 ? cgrid / 4 : 1), dim3(kSelThreads), stream, q.sc, q.candx, p.cap, q.ghist, q.gbuf,
                      q.blk, q.mom, nblk));
@@ -1897,11 +1754,10 @@ extern "C" int vb_psislw_f64(const double* lw, double* out, int64_t n, double re
   PsisPtrs q;
   psis_ptrs(static_cast<char*>(workspace), p, q);
   VB_CUDA(cudaMemsetAsync(result, 0, sizeof(double) * R_COUNT, stream));
-  // no output array: k-hat and the bound moments from ONE pass over the draws (VB_PSIS_ONEPASS=0: the two-pass form)
-  static const bool allow_onepass = [] { const char* e = getenv("VB_PSIS_ONEPASS"); return !(e && e[0] == '0'); }();
-  const int onepass = (!out && allow_onepass) ? 1 : 0;
+  // no output array: k-hat and the bound moments from ONE pass over the draws
+  const int onepass = !out ? 1 : 0;
   if ((rc = psis_stage_local(lw, n, 0, exact, p, q, stream, onepass))) return rc;
-  if ((rc = psis_stage_global(p, q, p.grid, result, tail_idx, tail_rank, stream, pass_a_v1() && !onepass))) return rc;
+  if ((rc = psis_stage_global(p, q, p.grid, result, tail_idx, tail_rank, stream, false))) return rc;
   if (onepass) return VB_OK;
   return psis_stage_apply(lw, out, n, 0, 1, p, q, result, stream);
 }
@@ -1936,7 +1792,7 @@ extern "C" int vb_psis_dist_local(const double* lw, int64_t n_local, int64_t idx
   psis_ptrs(static_cast<char*>(workspace), p, q);
   const bool small = n_local < (int64_t)p.M + 1;         // the sample is the whole shard and everything is a candidate
   if ((rc = psis_stage_local(lw, n_local, idx_off, small ? 0 : exact, p, q, stream))) return rc;
-  if (!small && (rc = psis_stage_select(p, q, p.grid, 1, stream, pass_a_v1()))) return rc;
+  if (!small && (rc = psis_stage_select(p, q, p.grid, 1, stream, false))) return rc;
   int blocks = (p.M + 1 + 255) / 256;
   if (blocks > sm_count()) blocks = sm_count();
   psis_export_kernel<<<blocks, 256, 0, stream>>>(q.sc, q.tmpv, q.tmpi, q.candx, q.candi, small ? 1 : 0, record);
