@@ -100,7 +100,8 @@ struct Philox {
   }
 };
 
-// 2 x 32 bits -> uniform double in (0,1) with 53 bits
+// 2 x 32 bits -> uniform double in (0,1] with 53 bits: from v = 2^52 up, v + 0.5 rounds to even, so the top value
+// (2^53 - 1) gives exactly 1.0 (harmless: Box-Muller's radius is then 0 and the gamma boost 1)
 __host__ __device__ inline double u01_53(uint32_t a, uint32_t b) {
   uint64_t v = (((uint64_t)a << 32) | b) >> 11;                 // 53 bits
   return ((double)v + 0.5) * (1.0 / 9007199254740992.0);
