@@ -381,7 +381,12 @@ int vb_gemm_f64(int trans_a, int trans_b, int M, int N, int K, double alpha, con
  *   vb_mvt_transform_f64  P = (z / u) V, theta = mu + (P . sqrt(w)) V^T = mu + (z / u) sqrtm(Sigma), zu2[s] = |z_s/u_s|^2,
  *                         u_s = sqrt(chi2_s / df)                                 (sample :342-349)
  *   vb_mvt_objective_f64  value[1], grad[d + d(d+1)/2] of ExclusiveKL (entropy form) / AlphaDivergence from the
- *                         model's f[S], G[S,d] at theta: the sqrtm / Cholesky-parameter VJPs as five GEMMs
+ *                         model's f[S], G[S,d] at theta: the sqrtm / Cholesky-parameter VJPs as five GEMMs.
+ *                         VB_OBJ_EXCLUSIVE_KL_PATH (use_path_deriv=True, objectives.py:156-159): value = -mean(f - log q)
+ *                         at var_param held fixed, gradient = the same VJPs of G + diag(kappa) Y without the entropy
+ *                         term, Y = (theta - mu) Sigma^+ with the 1e-10 eigenvalue floor of log_density (:26-28),
+ *                         kappa_s = (df + d) / (df + delta_s), delta_s = sum of P[s,k]^2 over w_k > 1e-10.  Needs
+ *                         vb_mvt_path_workspace_bytes(S, d) of workspace (2 S + 3 d doubles more); VB_ERR_WORKSPACE below.
  *   vb_mvt_log_density_f64  multivariate_t_logpdf with the 1e-10 eigenvalue floor of the pseudo-inverse (:26-30)
  * ------------------------------------------------------------------------------------- */
 int vb_mvt_unpack_f64(const double* var_param, int d, double* L, double* half_logdet, cudaStream_t stream);
@@ -391,6 +396,7 @@ int vb_mvt_transform_f64(const double* var_param, const double* z, const double*
                          const double* w, const double* V, double* P, double* theta, double* zu2, void* workspace,
                          size_t workspace_bytes, cudaStream_t stream);
 size_t vb_mvt_objective_workspace_bytes(int S, int d);
+size_t vb_mvt_path_workspace_bytes(int S, int d);
 int vb_mvt_objective_f64(const double* L, const double* half_logdet, const double* w, const double* V,
                          const double* P, const double* zu2, const double* f, const double* G, int S, int d,
                          double df, int objective, double alpha, double* value, double* grad, void* workspace,
@@ -411,11 +417,18 @@ int vb_mvt_log_density_f64(const double* var_param, const double* w, const doubl
  *                              grad_mu = c sum_s sv_s G_s,  Fbar[i,j] = c sum_s sv_s G[s,i] z[s,j]/u_s (j < i),
  *                              Fbar[i,i] = (c sum_s sv_s G[s,i] z[s,i]/u_s) L_ii + diag_add;
  *                              c = -1/S, sv = 1, diag_add = -1 (ExclusiveKL) or c = alpha/S, sv_s = exp(lw_s - max lw)^alpha,
- *                              diag_add = c sum_s sv_s (AlphaDivergence)
+ *                              diag_add = c sum_s sv_s (AlphaDivergence).
+ *                              VB_OBJ_EXCLUSIVE_KL_PATH (use_path_deriv=True, objectives.py:156-159): value =
+ *                              -mean(f - log q) at var_param held fixed; the formulas above with c = -1/S, sv = 1,
+ *                              diag_add = 0 and G replaced by G + diag(kappa) Y, Y = diag(1/u) z L^-1, kappa_s =
+ *                              (df + d) / (df + zu2_s).  L^-1 is formed on the device (64 x 64 diagonal blocks by
+ *                              substitution, then log2 doubling levels), so this form needs
+ *                              vb_mvt_chol_path_workspace_bytes(S, d) of workspace (O(d^2 + S d)); VB_ERR_WORKSPACE below.
  * ------------------------------------------------------------------------------------- */
 int vb_mvt_chol_transform_f64(const double* var_param, const double* z, const double* chi2, double df, int S, int d,
                               double* theta, double* inv_u, double* zu2, cudaStream_t stream);
 size_t vb_mvt_chol_objective_workspace_bytes(int S, int d);
+size_t vb_mvt_chol_path_workspace_bytes(int S, int d);
 int vb_mvt_chol_objective_f64(const double* var_param, const double* z, const double* inv_u, const double* zu2,
                               const double* f, const double* G, int S, int d, double df, int objective, double alpha,
                               double* value, double* grad, void* workspace, size_t workspace_bytes, cudaStream_t stream);

@@ -83,11 +83,13 @@ _PROTOS = {
     'vb_mvt_transform_workspace_bytes': (c_size_t, [c_int, c_int]),
     'vb_mvt_transform_f64': (c_int, [P, P, P, c_double, c_int, c_int, P, P, P, P, P, P, c_size_t, P]),
     'vb_mvt_objective_workspace_bytes': (c_size_t, [c_int, c_int]),
+    'vb_mvt_path_workspace_bytes': (c_size_t, [c_int, c_int]),
     'vb_mvt_objective_f64': (c_int, [P, P, P, P, P, P, P, P, c_int, c_int, c_double, c_int, c_double, P, P, P, c_size_t, P]),
     'vb_mvt_log_density_workspace_bytes': (c_size_t, [c_int64, c_int]),
     'vb_mvt_log_density_f64': (c_int, [P, P, P, P, c_int64, c_int, c_double, P, P, c_size_t, P]),
     'vb_mvt_chol_transform_f64': (c_int, [P, P, P, c_double, c_int, c_int, P, P, P, P]),
     'vb_mvt_chol_objective_workspace_bytes': (c_size_t, [c_int, c_int]),
+    'vb_mvt_chol_path_workspace_bytes': (c_size_t, [c_int, c_int]),
     'vb_mvt_chol_objective_f64': (c_int, [P, P, P, P, P, P, c_int, c_int, c_double, c_int, c_double, P, P, P, c_size_t, P]),
     'vb_mvt_target_log_weights_workspace_bytes': (c_size_t, [c_int]),
     'vb_mvt_target_log_weights_f64': (c_int, [P, P, c_int64, c_int64, c_int64, c_int, c_double, c_uint64, c_uint64, c_int,

@@ -59,13 +59,16 @@ __global__ void __launch_bounds__(256) mvt_rows_kernel(const double* __restrict_
   }
 }
 
-// sqrtw[k] = sqrt(max(w_k, 0));  winv[k] = |w_k| <= 1e-10 ? 0 : 1 / w_k   (_distributions.py:26-28)
-__global__ void mvt_eig_kernel(const double* __restrict__ w, int d, double* __restrict__ sqrtw, double* __restrict__ winv) {
+// sqrtw[k] = sqrt(max(w_k, 0));  winv[k] = |w_k| <= 1e-10 ? 0 : 1 / w_k   (_distributions.py:26-28);
+// rinv[k] = winv_k sqrtw_k = w_k > 1e-10 ? 1 / sqrt(w_k) : 0   (Sigma^+ A = V diag(rinv) V^T)
+__global__ void mvt_eig_kernel(const double* __restrict__ w, int d, double* __restrict__ sqrtw, double* __restrict__ winv,
+                               double* __restrict__ rinv) {
   const int k = blockIdx.x * blockDim.x + threadIdx.x;
   if (k >= d) return;
   const double v = w[k];
   if (sqrtw) sqrtw[k] = sqrt(fmax(v, 0.0));
   if (winv) winv[k] = fabs(v) <= 1e-10 ? 0.0 : 1.0 / v;
+  if (rinv) rinv[k] = v > 1e-10 ? 1.0 / sqrt(v) : 0.0;
 }
 
 // Sample weights and objective value (single block).  scal: [0] value, [1] diag_add.
@@ -75,6 +78,20 @@ __global__ void __launch_bounds__(1024) mvt_weights_kernel(const double* __restr
                                                            double* __restrict__ scal) {
   __shared__ double red[32];
   const double half_logdet = sld[0];
+  if (objective == VB_OBJ_EXCLUSIVE_KL_PATH) {
+    // -mean(f - log q) at var_param held fixed (objectives.py:156-159); no entropy term in the gradient
+    double a = 0.0;
+    for (int s = threadIdx.x; s < S; s += blockDim.x) {
+      a += f[s] - (logq_const - half_logdet - 0.5 * (df + d) * log1p(zu2[s] / df));
+      sv[s] = 1.0;
+    }
+    a = block_sum(a, red);
+    if (threadIdx.x == 0) {
+      scal[0] = -a / (double)S;
+      scal[1] = 0.0;
+    }
+    return;
+  }
   if (objective == VB_OBJ_EXCLUSIVE_KL) {
     double a = 0.0;
     for (int s = threadIdx.x; s < S; s += blockDim.x) {
@@ -127,6 +144,38 @@ __global__ void __launch_bounds__(1024) mvt_gmu_kernel(const double* __restrict_
 #pragma unroll
     for (int r = 0; r < 32; ++r) t += sm[r][x];
     gmu[j] = c * t;
+  }
+}
+
+// Path-derivative ExclusiveKL, sqrtm mode: y_s = Sigma^+ (theta_s - mu) = V diag(rinv) P_s^T with the reference's
+// eigenvalue floor, so delta_s = (theta_s - mu)^T Sigma^+ (theta_s - mu) = sum over unfloored k of P[s][k]^2 and
+// kappa_s = (df + d) / (df + delta_s)   (one warp per sample)
+__global__ void __launch_bounds__(256) mvt_path_delta_kernel(const double* __restrict__ P, const double* __restrict__ rinv, int S,
+                                                             int d, double df, double* __restrict__ delta,
+                                                             double* __restrict__ kappa) {
+  const int lane = threadIdx.x & 31;
+  const int64_t nwarps = (int64_t)gridDim.x * (blockDim.x >> 5);
+  for (int64_t s = (blockIdx.x * (int64_t)blockDim.x + threadIdx.x) >> 5; s < S; s += nwarps) {
+    double a = 0.0;
+    for (int k = lane; k < d; k += 32) {
+      const double p = P[s * d + k];
+      if (rinv[k] > 0.0) a += p * p;
+    }
+    a = warp_sum(a);
+    if (lane == 0) {
+      delta[s] = a;
+      kappa[s] = (df + d) / (df + a);
+    }
+  }
+}
+
+// (G + diag(kappa) Y) V = Q + diag(kappa) P diag(rinv):  Q[s][k] += kappa_s rinv_k P[s][k]
+__global__ void mvt_path_q_kernel(const double* __restrict__ P, const double* __restrict__ kappa, const double* __restrict__ rinv,
+                                  int S, int d, double* __restrict__ Q) {
+  const int64_t total = (int64_t)S * d;
+  for (int64_t idx = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; idx < total; idx += (int64_t)gridDim.x * blockDim.x) {
+    const int64_t s = idx / d, k = idx - s * d;
+    Q[idx] += kappa[s] * (rinv[k] * P[idx]);
   }
 }
 
@@ -196,7 +245,7 @@ int mvt_logdiag(const double* var_param, int d, double* out, cudaStream_t stream
 
 int mvt_weights_gmu(const double* f, const double* G, const double* zu2, const double* half_logdet, int S, int d, double df,
                     int objective, double alpha, double* sv, double* scal, double* value, double* gmu, cudaStream_t stream) {
-  const double c = objective == VB_OBJ_EXCLUSIVE_KL ? -1.0 / S : alpha / S;
+  const double c = objective == VB_OBJ_ALPHA ? alpha / S : -1.0 / S;
   mvt_weights_kernel<<<1, 1024, 0, stream>>>(f, zu2, S, d, df, mvt_const(df, d), half_logdet, objective, alpha, sv, scal);
   VB_CHECK_LAUNCH();
   VB_CUDA(cudaMemcpyAsync(value, scal, sizeof(double), cudaMemcpyDeviceToDevice, stream));
@@ -257,7 +306,7 @@ extern "C" int vb_mvt_transform_f64(const double* var_param, const double* z, co
   double* sqrtw = reinterpret_cast<double*>(ws + align_up(sizeof(double) * S, 256));
   int rc = mvt_rows(z, chi2, df, S, d, inv_u, zu2, stream);
   if (rc) return rc;
-  mvt_eig_kernel<<<(d + 255) / 256, 256, 0, stream>>>(w, d, sqrtw, nullptr);
+  mvt_eig_kernel<<<(d + 255) / 256, 256, 0, stream>>>(w, d, sqrtw, nullptr, nullptr);
   VB_CHECK_LAUNCH();
   rc = gemm(false, false, S, d, d, 1.0, z, d, V, d, P, d, nullptr, inv_u, nullptr, nullptr, nullptr, stream);
   if (rc) return rc;
@@ -266,6 +315,7 @@ extern "C" int vb_mvt_transform_f64(const double* var_param, const double* z, co
 
 struct MvtObjLayout {
   size_t off_sv, off_scal, off_sqrtw, off_Q, off_M, off_M2, off_T, off_Lbar, total;
+  size_t off_delta, off_kappa, off_rinv, off_gmu, off_ksum, total_path;     // path-derivative ExclusiveKL only
 };
 static void mvt_obj_layout(int S, int d, MvtObjLayout& l) {
   size_t off = 0;
@@ -279,6 +329,12 @@ static void mvt_obj_layout(int S, int d, MvtObjLayout& l) {
   l.off_T = take(sizeof(double) * (size_t)d * d);
   l.off_Lbar = take(sizeof(double) * (size_t)d * d);
   l.total = off;
+  l.off_delta = take(sizeof(double) * S);
+  l.off_kappa = take(sizeof(double) * S);
+  l.off_rinv = take(sizeof(double) * d);
+  l.off_gmu = take(sizeof(double) * d);
+  l.off_ksum = take(sizeof(double) * d);
+  l.total_path = off;
 }
 
 extern "C" size_t vb_mvt_objective_workspace_bytes(int S, int d) {
@@ -288,20 +344,32 @@ extern "C" size_t vb_mvt_objective_workspace_bytes(int S, int d) {
   return l.total;
 }
 
-/* value[1] and grad[d + d(d+1)/2] of ExclusiveKL (entropy form) / AlphaDivergence from the model's per-sample log density
- * f[S] and gradient G[S,d] at theta (vb_mvt_transform_f64), L and half_logdet (vb_mvt_unpack_f64), w / V (eigh of Sigma),
- * P and zu2 (vb_mvt_transform_f64). */
+/* workspace of vb_mvt_objective_f64 with VB_OBJ_EXCLUSIVE_KL_PATH: the above plus 2 S + 3 d doubles */
+extern "C" size_t vb_mvt_path_workspace_bytes(int S, int d) {
+  if (S <= 0 || d <= 0) return 0;
+  MvtObjLayout l;
+  mvt_obj_layout(S, d, l);
+  return l.total_path;
+}
+
+/* value[1] and grad[d + d(d+1)/2] of ExclusiveKL (entropy or path-derivative form) / AlphaDivergence from the model's
+ * per-sample log density f[S] and gradient G[S,d] at theta (vb_mvt_transform_f64), L and half_logdet
+ * (vb_mvt_unpack_f64), w / V (eigh of Sigma), P and zu2 (vb_mvt_transform_f64).  The path-derivative form runs the
+ * entropy form's VJP on G + diag(kappa) Y, Y = (theta - mu) Sigma^+ (floored pseudo-inverse), without the entropy
+ * term: (G + diag(kappa) Y) V = Q + diag(kappa) P diag(rinv), and the mean part gains c V (rinv . sum_s kappa_s P_s). */
 extern "C" int vb_mvt_objective_f64(const double* L, const double* half_logdet, const double* w, const double* V,
                                     const double* P, const double* zu2, const double* f, const double* G, int S, int d,
                                     double df, int objective, double alpha, double* value, double* grad, void* workspace,
                                     size_t workspace_bytes, cudaStream_t stream) {
   if (!L || !half_logdet || !w || !V || !P || !zu2 || !f || !G || S <= 0 || d <= 0 || !value || !grad)
     return set_error(VB_ERR_INVALID_ARG, "mvt_objective: bad arguments");
-  if (objective != VB_OBJ_EXCLUSIVE_KL && objective != VB_OBJ_ALPHA)
-    return set_error(VB_ERR_UNSUPPORTED, "path-derivative estimator is not available for MultivariateT");
+  if (objective != VB_OBJ_EXCLUSIVE_KL && objective != VB_OBJ_EXCLUSIVE_KL_PATH && objective != VB_OBJ_ALPHA)
+    return set_error(VB_ERR_UNSUPPORTED, "mvt_objective: unknown objective");
+  const bool path = objective == VB_OBJ_EXCLUSIVE_KL_PATH;
   MvtObjLayout l;
   mvt_obj_layout(S, d, l);
-  if (!workspace || workspace_bytes < l.total) return set_error(VB_ERR_WORKSPACE, "mvt_objective: workspace too small");
+  if (!workspace || workspace_bytes < (path ? l.total_path : l.total))
+    return set_error(VB_ERR_WORKSPACE, "mvt_objective: workspace too small");
   char* ws = static_cast<char*>(workspace);
   double* sv = reinterpret_cast<double*>(ws + l.off_sv);
   double* scal = reinterpret_cast<double*>(ws + l.off_scal);
@@ -311,13 +379,37 @@ extern "C" int vb_mvt_objective_f64(const double* L, const double* half_logdet, 
   double* M2 = reinterpret_cast<double*>(ws + l.off_M2);
   double* T = reinterpret_cast<double*>(ws + l.off_T);
   double* Lbar = reinterpret_cast<double*>(ws + l.off_Lbar);
-  const double c = objective == VB_OBJ_EXCLUSIVE_KL ? -1.0 / S : alpha / S;
-  int rc = mvt_weights_gmu(f, G, zu2, half_logdet, S, d, df, objective, alpha, sv, scal, value, grad, stream);
-  if (rc) return rc;
-  mvt_eig_kernel<<<(d + 255) / 256, 256, 0, stream>>>(w, d, sqrtw, nullptr);
-  VB_CHECK_LAUNCH();
-  rc = gemm(false, false, S, d, d, 1.0, G, d, V, d, Q, d, nullptr, sv, nullptr, nullptr, nullptr, stream);     // Q = (sv . G) V
-  if (rc) return rc;
+  const double c = objective == VB_OBJ_ALPHA ? alpha / S : -1.0 / S;
+  int rc;
+  if (path) {
+    double* delta = reinterpret_cast<double*>(ws + l.off_delta);
+    double* kappa = reinterpret_cast<double*>(ws + l.off_kappa);
+    double* rinv = reinterpret_cast<double*>(ws + l.off_rinv);
+    double* gmu = reinterpret_cast<double*>(ws + l.off_gmu);
+    double* ksum = reinterpret_cast<double*>(ws + l.off_ksum);
+    mvt_eig_kernel<<<(d + 255) / 256, 256, 0, stream>>>(w, d, sqrtw, nullptr, rinv);
+    VB_CHECK_LAUNCH();
+    const int64_t blocks = ceil_div(S, 256 / 32), cap = 64LL * sm_count();
+    mvt_path_delta_kernel<<<(unsigned)(blocks < cap ? blocks : cap), 256, 0, stream>>>(P, rinv, S, d, df, delta, kappa);
+    VB_CHECK_LAUNCH();
+    rc = mvt_weights_gmu(f, G, delta, half_logdet, S, d, df, objective, alpha, sv, scal, value, gmu, stream);
+    if (rc) return rc;
+    rc = gemm(false, false, S, d, d, 1.0, G, d, V, d, Q, d, nullptr, sv, nullptr, nullptr, nullptr, stream);   // Q = G V
+    if (rc) return rc;
+    mvt_path_q_kernel<<<ew_grid((int64_t)S * d), 256, 0, stream>>>(P, kappa, rinv, S, d, Q);
+    VB_CHECK_LAUNCH();
+    mvt_gmu_kernel<<<(d + 31) / 32, 1024, 0, stream>>>(P, kappa, S, d, 1.0, ksum);                         // sum_s kappa_s P_s
+    VB_CHECK_LAUNCH();
+    rc = gemm(false, true, 1, d, d, c, ksum, d, V, d, grad, d, rinv, nullptr, gmu, nullptr, nullptr, stream);   // + c V (rinv . ksum)
+    if (rc) return rc;
+  } else {
+    rc = mvt_weights_gmu(f, G, zu2, half_logdet, S, d, df, objective, alpha, sv, scal, value, grad, stream);
+    if (rc) return rc;
+    mvt_eig_kernel<<<(d + 255) / 256, 256, 0, stream>>>(w, d, sqrtw, nullptr, nullptr);
+    VB_CHECK_LAUNCH();
+    rc = gemm(false, false, S, d, d, 1.0, G, d, V, d, Q, d, nullptr, sv, nullptr, nullptr, nullptr, stream);   // Q = (sv . G) V
+    if (rc) return rc;
+  }
   rc = gemm(true, false, d, d, S, c, P, d, Q, d, M, d, nullptr, nullptr, nullptr, sqrtw, sqrtw, stream);           // c P^T Q ./ (rw + rw')
   if (rc) return rc;
   mvt_symmetrise_kernel<<<dim3((d + 31) / 32, (d + 31) / 32), 256, 0, stream>>>(M, d, M2);
@@ -350,7 +442,7 @@ extern "C" int vb_mvt_log_density_f64(const double* var_param, const double* w, 
   double* nmv = reinterpret_cast<double*>(ws + align_up(sizeof(double) * (size_t)n * d, 256));
   double* winv = nmv + align_up(sizeof(double) * d, 256) / sizeof(double);
   double* lpd = winv + align_up(sizeof(double) * d, 256) / sizeof(double);
-  mvt_eig_kernel<<<(d + 255) / 256, 256, 0, stream>>>(w, d, nullptr, winv);
+  mvt_eig_kernel<<<(d + 255) / 256, 256, 0, stream>>>(w, d, nullptr, winv, nullptr);
   VB_CHECK_LAUNCH();
   mvt_sumlog_kernel<<<1, 256, 0, stream>>>(w, d, lpd);
   VB_CHECK_LAUNCH();

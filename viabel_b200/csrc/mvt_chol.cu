@@ -12,9 +12,12 @@
 //
 // with c = -1/S (ExclusiveKL, sv = 1) or alpha/S (AlphaDivergence); the value, the weights sv and diag_add come from
 // the kernels the sqrtm path uses (mvt_internal.cuh), because log q at a reparameterised draw is the same closed form.
+// The path-derivative ExclusiveKL feeds the cotangent G + diag(kappa) Zhat L^-1 instead of G (below) and needs a
+// d x d inverse: its workspace is O(d^2 + S d).
 //
 // Both products run on the FP64 tensor pipe (mma.sync m8n8k4 f64, DMMA) with one warp owning each output fragment and
-// a fixed k order: no split-K, no atomics, so repeated calls give identical bits.  Workspace is O(S).
+// a fixed k order: no split-K, no atomics, so repeated calls give identical bits.  Workspace is O(S) (entropy form,
+// AlphaDivergence).
 #include "mvt_internal.cuh"
 
 namespace vb {
@@ -220,16 +223,235 @@ __global__ void __launch_bounds__(256) mvt_chol_cotangent_kernel(const double* _
   }
 }
 
+// ---- path-derivative ExclusiveKL: G + diag(kappa) Y,  Y = Zhat L^-1 ------------------------------------------------
+// The path gradient is the cotangent above with G_s replaced by G_s + kappa_s y_s (minus the score of log q at a
+// var_param held fixed), y_s = Sigma^-1 (theta_s - mu) = L^-T zhat_s, kappa_s = (df + d) / (df + |zhat_s|^2), and no
+// entropy term.  As rows Y = Zhat X with X = L^-1, which is formed on the device in three steps:
+//   1. the ceil(d/64) diagonal 64 x 64 blocks of X by substitution in shared memory, one CTA each;
+//   2. log2 doubling levels: at half-size h, blocks [r0, r0 + h) and [r0 + h, r0 + 2h) (r0 = 2 h p) combine through
+//      X21 = -X22 (L21 X11), two batched products whose tiles all run at once;
+//   3. Gt = G + diag(kappa / u) Z X, where column n of the product has the K range [n, d).
+// All on the FP64 tensor pipe with a fixed k order.  X is lower triangular; the upper half of every diagonal 64 x 64
+// block is written as zeros, and no reader touches a block above those.
+// L's block sits in the lower triangle of sm (sm[i][k], k <= i), its inverse transposed above it (X[i][j] at
+// sm[j][i + 1], i >= j): one 33 KB array.  Thread j forms column j of the inverse by forward substitution.
+__global__ void __launch_bounds__(kTN) mvt_chol_diaginv_kernel(const double* __restrict__ vp, int d, double* __restrict__ X) {
+  __shared__ double sm[kTN][kTN + 1];
+  const int r0 = blockIdx.x * kTN, n = min(kTN, d - r0);
+  const int j = threadIdx.x;
+  for (int i = 0; i < n; ++i)
+    if (j <= i) {
+      const double v = vp[d + tri(r0 + i) + r0 + j];
+      sm[i][j] = i == j ? exp(v) : v;
+    }
+  __syncthreads();
+  if (j < n) {
+    double* x = sm[j] + 1;                   // x[i] = X[i][j]
+    x[j] = 1.0 / sm[j][j];
+    for (int i = j + 1; i < n; ++i) {
+      double a = 0.0;
+      for (int k = j; k < i; ++k) a += sm[i][k] * x[k];
+      x[i] = -a / sm[i][i];
+    }
+    for (int i = 0; i < n; ++i) X[(size_t)(r0 + i) * d + r0 + j] = j <= i ? x[i] : 0.0;
+  }
+}
+
+// One doubling level at half-size h (a multiple of 64), one CTA per 64 x 64 output tile of every pair:
+//   kSecond = false:  T21 = L21 X11,  tile (i0, j0) with K range [j0, r0 + h)        (X11 lower triangular)
+//   kSecond = true:   X21 = -X22 T21, tile (i0, j0) with K range [r0 + h, i0 + 64)   (X22 lower triangular)
+// 8 warps of 16 x 32 fragments, register-prefetched slabs as in the cotangent kernel.
+template <bool kSecond>
+__global__ void __launch_bounds__(256) mvt_chol_invlevel_kernel(const double* __restrict__ vp, int d, int h,
+                                                                double* __restrict__ X, double* __restrict__ T) {
+  __shared__ double sa[kSlab][kPadN], sb[kSlab][kPadN];
+  const int tpb = h / kTN;
+  const int64_t per = (int64_t)tpb * tpb;
+  const int pair = (int)(blockIdx.x / per), tix = (int)(blockIdx.x % per);
+  const int r0 = 2 * h * pair, r2 = r0 + h;
+  const int i0 = r2 + (tix / tpb) * kTN, j0 = r0 + (tix % tpb) * kTN;
+  if (i0 >= d) return;                       // past the end of a short last block: the whole CTA leaves
+  const int kb = kSecond ? r2 : j0, ke = kSecond ? min(i0 + kTN, d) : r2;
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int wm = warp >> 1, wn = warp & 1;
+  const int gq = lane >> 2, t = lane & 3;
+  double acc[2][4][2];
+#pragma unroll
+  for (int a = 0; a < 2; ++a)
+#pragma unroll
+    for (int b = 0; b < 4; ++b) acc[a][b][0] = acc[a][b][1] = 0.0;
+
+  // A[i][k] (L21 from the packed triangle, or X22) is read along k, B[k][j] (X11 or T21) along j
+  double ra[kSlab * kTN / 256], rb[kSlab * kTN / 256];
+  auto load = [&](int k0) {
+#pragma unroll
+    for (int p = 0; p < kSlab * kTN / 256; ++p) {
+      const int i = i0 + p * 8 + warp, k = k0 + lane;
+      double v = 0.0;
+      if (i < d && k < d) v = kSecond ? X[(size_t)i * d + k] : vp[d + tri(i) + k];     // k < r2 <= i: strictly lower
+      ra[p] = v;
+      const int kr = k0 + p * 4 + (threadIdx.x >> 6), j = j0 + (threadIdx.x & 63);
+      rb[p] = kr < d ? (kSecond ? T : X)[(size_t)kr * d + j] : 0.0;
+    }
+  };
+  load(kb);
+  for (int k0 = kb; k0 < ke; k0 += kSlab) {
+    __syncthreads();
+#pragma unroll
+    for (int p = 0; p < kSlab * kTN / 256; ++p) {
+      sa[lane][p * 8 + warp] = ra[p];
+      sb[p * 4 + (threadIdx.x >> 6)][threadIdx.x & 63] = rb[p];
+    }
+    __syncthreads();
+    if (k0 + kSlab < ke) load(k0 + kSlab);
+#pragma unroll
+    for (int k4 = 0; k4 < kSlab; k4 += 4) {
+      double af[2], bf[4];
+#pragma unroll
+      for (int a = 0; a < 2; ++a) af[a] = sa[k4 + t][wm * 16 + a * 8 + gq];
+#pragma unroll
+      for (int b = 0; b < 4; ++b) bf[b] = sb[k4 + t][wn * 32 + b * 8 + gq];
+#pragma unroll
+      for (int a = 0; a < 2; ++a)
+#pragma unroll
+        for (int b = 0; b < 4; ++b) dmma(acc[a][b][0], acc[a][b][1], af[a], bf[b]);
+    }
+  }
+  double* out = kSecond ? X : T;
+#pragma unroll
+  for (int a = 0; a < 2; ++a) {
+    const int i = i0 + wm * 16 + a * 8 + gq;
+    if (i >= d) continue;
+#pragma unroll
+    for (int b = 0; b < 4; ++b)
+#pragma unroll
+      for (int u = 0; u < 2; ++u) {
+        const int j = j0 + wn * 32 + b * 8 + 2 * t + u;
+        out[(size_t)i * d + j] = kSecond ? -acc[a][b][u] : acc[a][b][u];
+      }
+  }
+}
+
+// Gt[s][n] = G[s][n] + kappa_s / u_s sum_{k >= n} Z[s][k] X[k][n].  Column block c has the K range [64 c, d), so CTA
+// (p, r) takes column blocks p and nb - 1 - p of row tile r to even out the work, as the triangular transform does.
+__global__ void __launch_bounds__(256) mvt_chol_solve_kernel(const double* __restrict__ z, const double* __restrict__ X,
+                                                             const double* __restrict__ G, const double* __restrict__ inv_u,
+                                                             const double* __restrict__ zu2, double df, int S, int d,
+                                                             double* __restrict__ Gt) {
+  __shared__ double sa[kSlab][kPadM], sb[kSlab][kPadN];
+  const int nb = (d + kTN - 1) / kTN;
+  const unsigned npairs = (unsigned)(nb + 1) / 2;
+  const int pair = (int)(blockIdx.x % npairs);
+  const int m0 = (int)(blockIdx.x / npairs) * kTM;
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int wm = warp >> 2, wn = warp & 3;
+  const int gq = lane >> 2, t = lane & 3;
+  const int cb0 = pair, cb1 = nb - 1 - pair;
+  const int ns0 = (d - cb0 * kTN + kSlab - 1) / kSlab;
+  const int total = ns0 + (cb1 == cb0 ? 0 : (d - cb1 * kTN + kSlab - 1) / kSlab);
+
+  double ra[kSlab * kTM / 256], rb[kSlab * kTN / 256];
+  auto load = [&](int n0, int k0) {
+#pragma unroll
+    for (int p = 0; p < kSlab * kTM / 256; ++p) {
+      const int s = m0 + p * 8 + warp, k = k0 + lane;
+      ra[p] = (s < S && k < d) ? z[(size_t)s * d + k] : 0.0;
+    }
+#pragma unroll
+    for (int p = 0; p < kSlab * kTN / 256; ++p) {
+      const int k = k0 + p * 4 + (threadIdx.x >> 6), n = n0 + (threadIdx.x & 63);
+      rb[p] = (k < d && n < d) ? X[(size_t)k * d + n] : 0.0;
+    }
+  };
+  double acc[2][2][2];
+  load(cb0 * kTN, cb0 * kTN);
+  for (int it = 0; it < total; ++it) {
+    const bool second = it >= ns0;
+    const int sl = second ? it - ns0 : it;
+    const int n0 = (second ? cb1 : cb0) * kTN;
+    const int nsl = second ? total - ns0 : ns0;
+    if (sl == 0) {
+#pragma unroll
+      for (int a = 0; a < 2; ++a)
+#pragma unroll
+        for (int b = 0; b < 2; ++b) acc[a][b][0] = acc[a][b][1] = 0.0;
+    }
+    __syncthreads();
+#pragma unroll
+    for (int p = 0; p < kSlab * kTM / 256; ++p) sa[lane][p * 8 + warp] = ra[p];
+#pragma unroll
+    for (int p = 0; p < kSlab * kTN / 256; ++p) sb[p * 4 + (threadIdx.x >> 6)][threadIdx.x & 63] = rb[p];
+    __syncthreads();
+    if (it + 1 < total) {
+      const bool second1 = it + 1 >= ns0;
+      const int c1 = second1 ? cb1 : cb0;
+      load(c1 * kTN, c1 * kTN + (second1 ? it + 1 - ns0 : it + 1) * kSlab);
+    }
+#pragma unroll
+    for (int k4 = 0; k4 < kSlab; k4 += 4) {
+      double af[2], bf[2];
+#pragma unroll
+      for (int a = 0; a < 2; ++a) af[a] = sa[k4 + t][wm * 16 + a * 8 + gq];
+#pragma unroll
+      for (int b = 0; b < 2; ++b) bf[b] = sb[k4 + t][wn * 16 + b * 8 + gq];
+#pragma unroll
+      for (int a = 0; a < 2; ++a)
+#pragma unroll
+        for (int b = 0; b < 2; ++b) dmma(acc[a][b][0], acc[a][b][1], af[a], bf[b]);
+    }
+    if (sl + 1 == nsl) {
+#pragma unroll
+      for (int a = 0; a < 2; ++a) {
+        const int s = m0 + wm * 16 + a * 8 + gq;
+        if (s >= S) continue;
+        const double kiu = (df + d) / (df + zu2[s]) * inv_u[s];
+#pragma unroll
+        for (int b = 0; b < 2; ++b)
+#pragma unroll
+          for (int u = 0; u < 2; ++u) {
+            const int n = n0 + wn * 16 + b * 8 + 2 * t + u;
+            if (n < d) Gt[(size_t)s * d + n] = G[(size_t)s * d + n] + kiu * acc[a][b][u];
+          }
+      }
+    }
+  }
+}
+
 struct CholObjLayout {
   size_t off_sv, off_scal, off_hl, total;
+  size_t off_X, off_T, off_Gt, total_path;     // path-derivative ExclusiveKL only
 };
-static void chol_obj_layout(int S, CholObjLayout& l) {
+static void chol_obj_layout(int S, int d, CholObjLayout& l) {
   size_t off = 0;
   auto take = [&](size_t bytes) { size_t o = off; off = align_up(off + bytes, 256); return o; };
   l.off_sv = take(sizeof(double) * S);
   l.off_scal = take(sizeof(double) * 4);
   l.off_hl = take(sizeof(double));
   l.total = off;
+  l.off_X = take(sizeof(double) * (size_t)d * d);
+  l.off_T = take(sizeof(double) * (size_t)d * d);
+  l.off_Gt = take(sizeof(double) * (size_t)S * d);
+  l.total_path = off;
+}
+
+// Gt = G + diag(kappa) Zhat L^-1 (see above); X and T are d x d scratch
+static int chol_path_gradient(const double* vp, const double* z, const double* inv_u, const double* zu2, const double* G,
+                              int S, int d, double df, double* X, double* T, double* Gt, cudaStream_t stream) {
+  const int nb = (d + kTN - 1) / kTN;
+  mvt_chol_diaginv_kernel<<<nb, kTN, 0, stream>>>(vp, d, X);
+  VB_CHECK_LAUNCH();
+  for (int h = kTN; h < d; h *= 2) {
+    const int64_t ctas = ceil_div(d - h, 2 * h) * (int64_t)(h / kTN) * (h / kTN);
+    mvt_chol_invlevel_kernel<false><<<(unsigned)ctas, 256, 0, stream>>>(vp, d, h, X, T);
+    VB_CHECK_LAUNCH();
+    mvt_chol_invlevel_kernel<true><<<(unsigned)ctas, 256, 0, stream>>>(vp, d, h, X, T);
+    VB_CHECK_LAUNCH();
+    if (h > INT32_MAX / 2) break;
+  }
+  const int64_t ctas = (nb + 1) / 2 * ceil_div(S, kTM);
+  mvt_chol_solve_kernel<<<(unsigned)ctas, 256, 0, stream>>>(z, X, G, inv_u, zu2, df, S, d, Gt);
+  VB_CHECK_LAUNCH();
+  return VB_OK;
 }
 
 }  // namespace vb
@@ -256,35 +478,55 @@ extern "C" int vb_mvt_chol_transform_f64(const double* var_param, const double* 
 extern "C" size_t vb_mvt_chol_objective_workspace_bytes(int S, int d) {
   if (S <= 0 || d <= 0) return 0;
   CholObjLayout l;
-  chol_obj_layout(S, l);
+  chol_obj_layout(S, d, l);
   return l.total;
 }
 
-/* value[1] and grad[d + d(d+1)/2] of ExclusiveKL (entropy form) / AlphaDivergence (objectives.py:154-164, :443-460)
- * in the Cholesky reparameterisation, from the model's f[S] and G[S,d] at theta and inv_u / zu2 of
- * vb_mvt_chol_transform_f64. */
+/* workspace of vb_mvt_chol_objective_f64 with VB_OBJ_EXCLUSIVE_KL_PATH: the above plus 2 d^2 + S d doubles */
+extern "C" size_t vb_mvt_chol_path_workspace_bytes(int S, int d) {
+  if (S <= 0 || d <= 0) return 0;
+  CholObjLayout l;
+  chol_obj_layout(S, d, l);
+  return l.total_path;
+}
+
+/* value[1] and grad[d + d(d+1)/2] of ExclusiveKL (entropy or path-derivative form) / AlphaDivergence
+ * (objectives.py:154-164, :443-460) in the Cholesky reparameterisation, from the model's f[S] and G[S,d] at theta and
+ * inv_u / zu2 of vb_mvt_chol_transform_f64. */
 extern "C" int vb_mvt_chol_objective_f64(const double* var_param, const double* z, const double* inv_u, const double* zu2,
                                          const double* f, const double* G, int S, int d, double df, int objective, double alpha,
                                          double* value, double* grad, void* workspace, size_t workspace_bytes,
                                          cudaStream_t stream) {
   if (!var_param || !z || !inv_u || !zu2 || !f || !G || S <= 0 || d <= 0 || !value || !grad)
     return set_error(VB_ERR_INVALID_ARG, "mvt_chol_objective: bad arguments");
-  if (objective != VB_OBJ_EXCLUSIVE_KL && objective != VB_OBJ_ALPHA)
-    return set_error(VB_ERR_UNSUPPORTED, "path-derivative estimator is not available for MultivariateT");
+  if (objective != VB_OBJ_EXCLUSIVE_KL && objective != VB_OBJ_EXCLUSIVE_KL_PATH && objective != VB_OBJ_ALPHA)
+    return set_error(VB_ERR_UNSUPPORTED, "mvt_chol_objective: unknown objective");
+  const bool path = objective == VB_OBJ_EXCLUSIVE_KL_PATH;
   CholObjLayout l;
-  chol_obj_layout(S, l);
-  if (!workspace || workspace_bytes < l.total) return set_error(VB_ERR_WORKSPACE, "mvt_chol_objective: workspace too small");
+  chol_obj_layout(S, d, l);
+  if (!workspace || workspace_bytes < (path ? l.total_path : l.total))
+    return set_error(VB_ERR_WORKSPACE, "mvt_chol_objective: workspace too small");
+  const int nb = (d + kTN - 1) / kTN;
+  if (path && ((nb + 1) / 2 * ceil_div(S, kTM) > INT32_MAX || (int64_t)nb * nb > INT32_MAX))
+    return set_error(VB_ERR_UNSUPPORTED, "mvt_chol_objective: more than 2^31 - 1 tiles");
   char* ws = static_cast<char*>(workspace);
   double* sv = reinterpret_cast<double*>(ws + l.off_sv);
   double* scal = reinterpret_cast<double*>(ws + l.off_scal);
   double* hl = reinterpret_cast<double*>(ws + l.off_hl);
   int rc = mvt_logdiag(var_param, d, hl, stream);
   if (rc) return rc;
-  rc = mvt_weights_gmu(f, G, zu2, hl, S, d, df, objective, alpha, sv, scal, value, grad, stream);
+  const double* Gc = G;
+  if (path) {
+    double* Gt = reinterpret_cast<double*>(ws + l.off_Gt);
+    rc = chol_path_gradient(var_param, z, inv_u, zu2, G, S, d, df, reinterpret_cast<double*>(ws + l.off_X),
+                            reinterpret_cast<double*>(ws + l.off_T), Gt, stream);
+    if (rc) return rc;
+    Gc = Gt;
+  }
+  rc = mvt_weights_gmu(f, Gc, zu2, hl, S, d, df, objective, alpha, sv, scal, value, grad, stream);
   if (rc) return rc;
-  const double c = objective == VB_OBJ_EXCLUSIVE_KL ? -1.0 / S : alpha / S;
-  const int nb = (d + kTN - 1) / kTN;
-  mvt_chol_cotangent_kernel<<<(unsigned)(nb * (nb + 1) / 2), 256, 0, stream>>>(var_param, z, inv_u, G, sv, scal, c, S, d, grad);
+  const double c = objective == VB_OBJ_ALPHA ? alpha / S : -1.0 / S;
+  mvt_chol_cotangent_kernel<<<(unsigned)(nb * (nb + 1) / 2), 256, 0, stream>>>(var_param, z, inv_u, Gc, sv, scal, c, S, d, grad);
   VB_CHECK_LAUNCH();
   return VB_OK;
 }

@@ -79,13 +79,16 @@ class StochasticVariationalObjective(VariationalObjective):
         self._update_objective_and_grad()
 
 
+def _workspace(lib_fn_entropy, lib_fn_path, objective, S, d, device):
+    nbytes = (lib_fn_path if objective == _lib.OBJ_EXCLUSIVE_KL_PATH else lib_fn_entropy)(S, d)
+    return torch.empty(nbytes, dtype=torch.uint8, device=device)
+
+
 def _mvt_objective(approx, model, S, objective, alpha, var_param, base=None, seed=None):
-    """ExclusiveKL (entropy branch) / AlphaDivergence for the full-rank MultivariateT family
+    """ExclusiveKL (entropy and path-derivative branches) / AlphaDivergence for the full-rank MultivariateT family
     (objectives.py:154-164, :443-460 with approximations.py:342-357; gradient per SURVEY.md App. A.3).
     unpack -> Sigma -> [cuSOLVER eigh] -> reparameterise -> model plugin -> vb_mvt_objective_f64: everything except
     the eigensolver is this package's kernels (csrc/mvt.cu, float64 tensor-core GEMMs of csrc/gemm_f64.cu)."""
-    if objective == _lib.OBJ_EXCLUSIVE_KL_PATH:
-        raise NotImplementedError('path-derivative estimator is not available for MultivariateT')
     vp = to_dev(var_param)
     d, df = approx.dim, float(approx.df)
     chi2, z = approx.base_draws(S, seed) if base is None else (to_dev(base[0]).reshape(-1), to_dev(base[1]))
@@ -97,7 +100,8 @@ def _mvt_objective(approx, model, S, objective, alpha, var_param, base=None, see
     theta, P, zu2 = approx.transform(vp, chi2, z, w, V)
     f, G = model.logp_and_grad(theta)
     out = torch.empty(1 + vp.numel(), dtype=F64, device=vp.device)
-    ws = torch.empty(_lib.lib.vb_mvt_objective_workspace_bytes(S, d), dtype=torch.uint8, device=vp.device)
+    ws = _workspace(_lib.lib.vb_mvt_objective_workspace_bytes, _lib.lib.vb_mvt_path_workspace_bytes, objective, S, d,
+                    vp.device)
     _lib.check(_lib.lib.vb_mvt_objective_f64(
         _lib.ptr(L), _lib.ptr(hl), _lib.ptr(w), _lib.ptr(V), _lib.ptr(P), _lib.ptr(zu2), _lib.ptr(f.contiguous()),
         _lib.ptr(G.contiguous()), S, d, df, objective, float(alpha), _lib.ptr(out[:1]), _lib.ptr(out[1:]), _lib.ptr(ws),
@@ -107,12 +111,14 @@ def _mvt_objective(approx, model, S, objective, alpha, var_param, base=None, see
 
 def _mvt_chol_objective(approx, model, objective, alpha, vp, chi2, z):
     """The same objectives in MultivariateT's Cholesky reparameterisation, theta = mu + L z / u: triangular transform
-    -> model plugin -> vb_mvt_chol_objective_f64 (csrc/mvt_chol.cu).  No eigensolver and no host synchronisation."""
+    -> model plugin -> vb_mvt_chol_objective_f64 (csrc/mvt_chol.cu).  No eigensolver and no host synchronisation.
+    The path-derivative form inverts L on the device and needs an O(d^2 + S d) workspace; the others need O(S)."""
     S, d = int(z.shape[0]), approx.dim
     theta, inv_u, zu2 = approx.chol_transform(vp, chi2, z)
     f, G = model.logp_and_grad(theta)
     out = torch.empty(1 + vp.numel(), dtype=F64, device=vp.device)
-    ws = torch.empty(_lib.lib.vb_mvt_chol_objective_workspace_bytes(S, d), dtype=torch.uint8, device=vp.device)
+    ws = _workspace(_lib.lib.vb_mvt_chol_objective_workspace_bytes, _lib.lib.vb_mvt_chol_path_workspace_bytes, objective,
+                    S, d, vp.device)
     _lib.check(_lib.lib.vb_mvt_chol_objective_f64(
         _lib.ptr(vp), _lib.ptr(z), _lib.ptr(inv_u), _lib.ptr(zu2), _lib.ptr(f.contiguous()), _lib.ptr(G.contiguous()), S, d,
         float(approx.df), objective, float(alpha), _lib.ptr(out[:1]), _lib.ptr(out[1:]), _lib.ptr(ws), ws.numel(),
