@@ -45,6 +45,7 @@ def c5_problem(vb, mode):
 def kernel_ms(vb, torch, vp, model, approx, n, reps):
     """CUDA-event time of the streaming kernel alone over n draws (fused target, or theta_out chunks for a model)."""
     from viabel_b200 import _lib
+    from viabel_b200.models import _product_target
     d = approx.dim
     vpd = torch.as_tensor(vp, device='cuda')
     A = None
@@ -55,18 +56,18 @@ def kernel_ms(vb, torch, vp, model, approx, n, reps):
                                         _lib.ptr(torch.sqrt(w)), None, None, None, None, _lib.stream()))
     ws = torch.empty(_lib.lib.vb_mvt_target_log_weights_workspace_bytes(d), dtype=torch.uint8, device='cuda')
     lw = torch.empty(n, dtype=torch.float64, device='cuda')
-    fused = type(model) in (vb.GaussianTarget, vb.StudentTTarget)
+    target = _product_target(model)
+    fused = target is not None
     chunk = n if fused else max(1, 2 ** 28 // d)
     theta = None if fused else torch.empty(min(chunk, n), d, dtype=torch.float64, device='cuda')
-    loc = getattr(model, 'loc', None) if fused else None
-    scale = getattr(model, 'scale', None) if fused else None
+    kind, loc, scale, tdf = target if fused else (-1, None, None, 0.0)
 
     def once():
         for lo in range(0, n, chunk):
             m = min(chunk, n - lo)
             _lib.check(_lib.lib.vb_mvt_target_log_weights_f64(
-                _lib.ptr(vpd), _lib.ptr(A), n, lo, m, d, float(approx.df), approx._seed, 0, 1 if fused else -1,
-                _lib.ptr(loc), _lib.ptr(scale), float(getattr(model, 'df', 0.0)) if fused else 0.0,
+                _lib.ptr(vpd), _lib.ptr(A), n, lo, m, d, float(approx.df), approx._seed, 0, kind,
+                _lib.ptr(loc), _lib.ptr(scale), tdf,
                 _lib.ptr(lw[lo:lo + m]), _lib.ptr(None if theta is None else theta[:m]), _lib.ptr(ws), ws.numel(),
                 _lib.stream()))
     once()

@@ -27,6 +27,11 @@ int sm_count();
 constexpr double kLog2Pi = 1.8378770664093454835606594728112;
 constexpr double kInvSqrt2 = 0.70710678118654752440084436210485;
 
+// log of the Student-t density's normaliser, lgamma((df+1)/2) - lgamma(df/2) - log(pi df)/2 (host)
+inline double student_t_log_const(double df) {
+  return lgamma(0.5 * (df + 1.0)) - lgamma(0.5 * df) - 0.5 * log(df * 3.14159265358979323846);
+}
+
 __host__ __device__ inline int64_t ceil_div(int64_t a, int64_t b) { return (a + b - 1) / b; }
 __host__ __device__ inline size_t align_up(size_t x, size_t a) { return (x + a - 1) / a * a; }
 

@@ -131,8 +131,7 @@ extern "C" int vb_mf_score_f64(const double* var_param, const double* x, const i
   if (family == VB_FAMILY_MF_STUDENT && !(df > 2.0)) return set_error(VB_ERR_INVALID_ARG, "df must be greater than 2");
   const int nb = (d + 31) / 32;
   if (!workspace || workspace_bytes < vb_mf_score_workspace_bytes(d)) return set_error(VB_ERR_WORKSPACE, "mf_score: workspace too small");
-  const double tc = family == VB_FAMILY_MF_STUDENT
-                        ? lgamma(0.5 * (df + 1.0)) - lgamma(0.5 * df) - 0.5 * log(df * 3.14159265358979323846) : 0.0;
+  const double tc = family == VB_FAMILY_MF_STUDENT ? student_t_log_const(df) : 0.0;
   double* part = static_cast<double*>(workspace);
   mf_score_kernel<<<nb, 32 * kScoreGroups, 0, stream>>>(var_param, x, reinterpret_cast<const long long*>(idx), w, scale, n, d,
                                                         family, df, tc, grad, part);

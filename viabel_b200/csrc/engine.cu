@@ -455,10 +455,6 @@ __global__ void __launch_bounds__(32 * kPostGroups) mf_post_kernel(StepCfg c, St
   }
 }
 
-static inline double student_const_h(double df) {
-  return lgamma(0.5 * (df + 1.0)) - lgamma(0.5 * df) - 0.5 * log(df * 3.14159265358979323846);
-}
-
 }  // namespace vb
 
 using namespace vb;
@@ -645,7 +641,7 @@ extern "C" int vb_mf_step_glm(const vb_step_config* cfg, const vb_step_buffers* 
   c.quantize = cfg->quantize; c.inject = cfg->inject_base; c.fast = fast;
   c.d_pad = L.d_pad; c.chunks = L.chunks; c.rowsA = L.rowsA;
   c.df = cfg->df;
-  c.tconst = cfg->family == VB_FAMILY_MF_STUDENT ? student_const_h(cfg->df) : 0.0;
+  c.tconst = cfg->family == VB_FAMILY_MF_STUDENT ? student_t_log_const(cfg->df) : 0.0;
   if (cfg->prior_sd > 0.0 && isfinite(cfg->prior_sd)) {
     c.inv_tau2 = 1.0 / (cfg->prior_sd * cfg->prior_sd);
     c.prior_const = -(double)d * log(cfg->prior_sd * sqrt(2.0 * 3.14159265358979323846));

@@ -24,11 +24,12 @@
 // computed alone equals the same draws of a longer call.
 #include "mvt_internal.cuh"
 #include "philox_draws.cuh"
+#include "stream_internal.cuh"
 
 namespace vb {
 
-constexpr int kLrM = 32;                     // draws per tile
-constexpr int kLrN = 128;                    // theta column block
+constexpr int kLrM = kTileM;                 // draws per tile
+constexpr int kLrN = kTileN;                 // theta column block
 constexpr int kLrWN = 32;                    // w column block (rows of P)
 constexpr int kLrUSharedMax = 512;           // u tile in shared memory while k + d <= this
 constexpr int kLrMaxWidth = 1 << 26;         // k + d: tile offsets stay in 32 bits
@@ -187,30 +188,9 @@ __global__ void __launch_bounds__(256, 2) lr_stream_lw_kernel(const LrStreamArgs
 #pragma unroll
           for (int b = 0; b < 4; ++b) dmma(acc[a][b][0], acc[a][b][1], af[a], bf[b]);
       }
-#pragma unroll
-      for (int a = 0; a < 2; ++a) {
-        const int r = wm * 16 + a * 8 + gq;
-        const bool live = r < rows;
-        double part = 0.0;
-#pragma unroll
-        for (int b = 0; b < 4; ++b)
-#pragma unroll
-          for (int u = 0; u < 2; ++u) {
-            const int n = n0 + wn * 32 + b * 8 + 2 * t + u;
-            if (!live || n >= d) continue;
-            const double th = p.vp[n] + acc[a][b][u] + p.sig[n] * et[r * lde + n];
-            if (p.theta_out) p.theta_out[(size_t)(i0 - p.first + r) * d + n] = th;
-            if (p.target_kind >= 0) {
-              const double zz = (th - p.loc[n]) / p.scale[n];
-              part += p.target_kind == 0 ? -0.5 * zz * zz : -0.5 * (p.target_df + 1.0) * log1p(zz * zz / p.target_df);
-            }
-          }
-        part += __shfl_xor_sync(0xffffffffu, part, 1);
-        part += __shfl_xor_sync(0xffffffffu, part, 2);
-        if (t == 0) s_red[wn * kLrM + r] = part;
-      }
-      __syncthreads();
-      if (tid < kLrM) s_lp[tid] += ((s_red[tid] + s_red[kLrM + tid]) + s_red[2 * kLrM + tid]) + s_red[3 * kLrM + tid];
+      target_tile_epilogue(p, acc, i0, rows, n0, s_red, s_lp, [&](int r) {
+        return [&, r](int n, double v) { return p.vp[n] + v + p.sig[n] * et[r * lde + n]; };
+      });
       __syncthreads();                       // s_red is rewritten by the next column block
     }
     __syncthreads();
@@ -226,20 +206,19 @@ __global__ void __launch_bounds__(256) lr_stream_prep_kernel(const double* vp, c
                                                               int target_kind, const double* scale, double target_const,
                                                               double* consts, double* sig) {
   __shared__ double red[32];
-  double a = 0.0, b = 0.0, c = 0.0;
+  double a = 0.0, b = 0.0;
   for (int j = threadIdx.x; j < d; j += blockDim.x) {
     const double ls = vp[d + j];
     sig[j] = exp(ls);
     a += ls;
-    if (target_kind >= 0) c += log(scale[j]);
   }
   for (int l = threadIdx.x; l < k; l += blockDim.x) b += log(P[(size_t)l * (k + d) + l]);
   a = block_sum(a, red);
   b = block_sum(b, red);
-  c = block_sum(c, red);
+  const double c = target_kind >= 0 ? product_target_log_const(target_const, scale, d, red) : 0.0;
   if (threadIdx.x == 0) {
     consts[0] = -0.5 * kLog2Pi * d - a + b;
-    consts[1] = target_const - c;
+    consts[1] = c;
   }
 }
 
@@ -250,17 +229,10 @@ static inline size_t lr_smem(bool ushared, int d, int k) {
                            (ushared ? (size_t)kLrM * (lr_ld(k) + lr_ld(d)) : 0));
 }
 
-// CTAs per launch (persistent grid: as many as can be resident)
 static int lr_ctas(int d, int k, int64_t* ctas) {
   const bool ushared = k + d <= kLrUSharedMax;
-  auto kern = ushared ? lr_stream_lw_kernel<true> : lr_stream_lw_kernel<false>;
-  const size_t smem = lr_smem(ushared, d, k);
-  VB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  int per_sm = 0;
-  VB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, 256, smem));
-  if (per_sm < 1) return set_error(VB_ERR_UNSUPPORTED, "lr_target_log_weights: kernel does not fit on an SM");
-  *ctas = (int64_t)per_sm * sm_count();
-  return VB_OK;
+  return persistent_ctas(ushared ? lr_stream_lw_kernel<true> : lr_stream_lw_kernel<false>, 256, lr_smem(ushared, d, k),
+                         ctas);
 }
 
 // 256 bytes of constants, sigma[d], then one 32-row u tile per resident CTA when k + d > 512
@@ -268,10 +240,6 @@ static size_t lr_ws_layout(int d, int k, int64_t ctas, size_t* off_sig, size_t* 
   *off_sig = 256;
   *off_u = 256 + align_up(sizeof(double) * (size_t)d, 256);
   return *off_u + (k + d > kLrUSharedMax ? sizeof(double) * (size_t)ctas * kLrM * (lr_ld(k) + lr_ld(d)) : 0);
-}
-
-static inline double lr_t_coord_const(double df) {
-  return lgamma(0.5 * (df + 1.0)) - lgamma(0.5 * df) - 0.5 * log(df * 3.14159265358979323846);
 }
 
 }  // namespace vb
@@ -299,29 +267,22 @@ extern "C" int vb_lr_target_log_weights_f64(const double* var_param, const doubl
     return set_error(VB_ERR_INVALID_ARG, "lr_target_log_weights: bad arguments");
   if (n_total > (INT64_MAX / 2) / ((int64_t)d + k))
     return set_error(VB_ERR_INVALID_ARG, "lr_target_log_weights: n_total * (d + k) too large");
-  if (target_kind < -1 || target_kind > 1)
-    return set_error(VB_ERR_INVALID_ARG, "lr_target_log_weights: target_kind is -1 (none), 0 (Gaussian) or 1 (Student-t)");
-  if (target_kind >= 0 && (!target_loc || !target_scale))
-    return set_error(VB_ERR_INVALID_ARG, "lr_target_log_weights: bad arguments");
-  if (target_kind == 1 && !(target_df > 0.0))
-    return set_error(VB_ERR_INVALID_ARG, "lr_target_log_weights: target_df must be positive");
+  int rc = check_product_target("lr_target_log_weights", target_kind, true, target_loc, target_scale, target_df);
+  if (rc) return rc;
   if ((int64_t)k + d >= kLrMaxWidth) return set_error(VB_ERR_UNSUPPORTED, "lr_target_log_weights: k + d too large");
   int64_t ctas = 0;
-  int rc = lr_ctas(d, k, &ctas);
+  rc = lr_ctas(d, k, &ctas);
   if (rc) return rc;
   size_t off_sig, off_u;
   if (!workspace || workspace_bytes < lr_ws_layout(d, k, ctas, &off_sig, &off_u))
     return set_error(VB_ERR_WORKSPACE, "lr_target_log_weights: workspace too small");
   if (count == 0) return VB_OK;
-  const int64_t tiles = ceil_div(count, kLrM);
-  const int64_t grid = tiles < ctas ? tiles : ctas;
-  if (grid > INT32_MAX) return set_error(VB_ERR_UNSUPPORTED, "lr_target_log_weights: more than 2^31 - 1 CTAs");
+  const int64_t tiles = ceil_div(count, kLrM), grid = tiles < ctas ? tiles : ctas;
   char* ws = static_cast<char*>(workspace);
   double* consts = reinterpret_cast<double*>(ws);
   double* sig = reinterpret_cast<double*>(ws + off_sig);
-  const double target_const =
-      target_kind == 0 ? -0.5 * kLog2Pi * d : target_kind == 1 ? d * lr_t_coord_const(target_df) : 0.0;
-  lr_stream_prep_kernel<<<1, 256, 0, stream>>>(var_param, P, d, k, target_kind, target_scale, target_const, consts, sig);
+  lr_stream_prep_kernel<<<1, 256, 0, stream>>>(var_param, P, d, k, target_kind, target_scale,
+                                               product_target_const(target_kind, d, target_df), consts, sig);
   VB_CHECK_LAUNCH();
   LrStreamArgs p;
   p.vp = var_param;

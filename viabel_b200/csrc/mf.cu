@@ -4,10 +4,6 @@
 
 namespace vb {
 
-static inline double student_const(double df) {
-  return lgamma(0.5 * (df + 1.0)) - lgamma(0.5 * df) - 0.5 * log(df * 3.14159265358979323846);
-}
-
 // theta = mu + exp(log_sigma) * base   (approximations.py:212-216, :270-274)
 __global__ void mf_sample_kernel(const double* __restrict__ vp, const double* __restrict__ base,
                                  double* __restrict__ theta, int64_t S, int d) {
@@ -228,7 +224,7 @@ extern "C" int vb_mf_log_density_f64(const double* var_param, const double* x, i
   int rc = check_family(family, df);
   if (rc) return rc;
   if (n == 0) return VB_OK;
-  const double tc = family == VB_FAMILY_MF_STUDENT ? student_const(df) : 0.0;
+  const double tc = family == VB_FAMILY_MF_STUDENT ? student_t_log_const(df) : 0.0;
   mf_log_density_kernel<<<grid_for(n * 32, 256), 256, 0, stream>>>(var_param, x, n, d, family, df, tc, out);
   VB_CHECK_LAUNCH();
   return VB_OK;
@@ -244,7 +240,7 @@ extern "C" int vb_mf_alpha_weights_f64(const double* var_param, const double* th
   if (rc) return rc;
   double inv_tau2, pc;
   prior_consts(prior_sd, d, inv_tau2, pc);
-  const double tc = family == VB_FAMILY_MF_STUDENT ? student_const(df) : 0.0;
+  const double tc = family == VB_FAMILY_MF_STUDENT ? student_t_log_const(df) : 0.0;
   mf_log_weights_kernel<<<grid_for(S * 32, 256), 256, 0, stream>>>(var_param, theta, base, ll, S, d, family, df,
                                                                    tc, inv_tau2, pc, lw);
   VB_CHECK_LAUNCH();
@@ -269,7 +265,7 @@ extern "C" int vb_mf_objective_finish_f64(const double* var_param, const double*
   if (rc) return rc;
   double inv_tau2, pc;
   prior_consts(prior_sd, d, inv_tau2, pc);
-  const double tc = family == VB_FAMILY_MF_STUDENT ? student_const(df) : 0.0;
+  const double tc = family == VB_FAMILY_MF_STUDENT ? student_t_log_const(df) : 0.0;
   if (value || logp) {
     if (objective != VB_OBJ_ALPHA && !value)
       return set_error(VB_ERR_INVALID_ARG, "mf_objective_finish: value is required");

@@ -22,11 +22,12 @@
 // caller asks for theta_out.
 #include "mvt_internal.cuh"
 #include "philox_draws.cuh"
+#include "stream_internal.cuh"
 
 namespace vb {
 
-constexpr int kSM = 32;                      // draws per tile
-constexpr int kSN = 128;                     // column block width
+constexpr int kSM = kTileM;                  // draws per tile
+constexpr int kSN = kTileN;                  // column block width
 constexpr int kSK = 32;                      // K slab
 constexpr int kSPadM = kSM + 4, kSPadN = kSN + 4;
 constexpr int kZSharedMaxDim = 512;          // z tile in shared memory up to here (128 KB)
@@ -94,13 +95,9 @@ __global__ void __launch_bounds__(256, 2) mvt_stream_lw_kernel(const MvtStreamAr
   const int nb = (d + kSN - 1) / kSN;
   const int dslabs = (d + kSK - 1) / kSK;
 
-  // sum_j log scale_j: the same fixed-order sum in every CTA
+  // target_const - sum_j log scale_j: the same fixed-order sum in every CTA
   double pconst = 0.0;
-  if (p.target_kind >= 0) {
-    double a = 0.0;
-    for (int j = tid; j < d; j += blockDim.x) a += log(p.scale[j]);
-    pconst = p.target_const - block_sum(a, s_misc);
-  }
+  if (p.target_kind >= 0) pconst = product_target_log_const(p.target_const, p.scale, d, s_misc);
   const double hl = p.half_logdet[0];
   const Philox ph(p.seed);
   const int64_t ntiles = (p.count + kSM - 1) / kSM;
@@ -178,34 +175,11 @@ __global__ void __launch_bounds__(256, 2) mvt_stream_lw_kernel(const MvtStreamAr
 #pragma unroll
           for (int b = 0; b < 4; ++b) dmma(acc[a][b][0], acc[a][b][1], af[a], bf[b]);
       }
-      if (sl + 1 == ns) {                    // last slab of column block cb: epilogue
-        const int n0 = cb * kSN;
-#pragma unroll
-        for (int a = 0; a < 2; ++a) {
-          const int r = wm * 16 + a * 8 + gq;
-          const bool live = r < rows;
-          const double iu = live ? s_iu[r] : 0.0;
-          double part = 0.0;
-#pragma unroll
-          for (int b = 0; b < 4; ++b)
-#pragma unroll
-            for (int u = 0; u < 2; ++u) {
-              const int n = n0 + wn * 32 + b * 8 + 2 * t + u;
-              if (!live || n >= d) continue;
-              const double th = p.vp[n] + iu * acc[a][b][u];
-              if (p.theta_out) p.theta_out[(size_t)(i0 - p.first + r) * d + n] = th;
-              if (p.target_kind >= 0) {
-                const double zz = (th - p.loc[n]) / p.scale[n];
-                part += p.target_kind == 0 ? -0.5 * zz * zz : -0.5 * (p.target_df + 1.0) * log1p(zz * zz / p.target_df);
-              }
-            }
-          part += __shfl_xor_sync(0xffffffffu, part, 1);
-          part += __shfl_xor_sync(0xffffffffu, part, 2);
-          if (t == 0) s_red[wn * kSM + r] = part;
-        }
-        __syncthreads();
-        if (tid < kSM) s_lp[tid] += ((s_red[tid] + s_red[kSM + tid]) + s_red[2 * kSM + tid]) + s_red[3 * kSM + tid];
-      }
+      if (sl + 1 == ns)                      // last slab of column block cb: epilogue
+        target_tile_epilogue(p, acc, i0, rows, cb * kSN, s_red, s_lp, [&](int r) {
+          const double iu = s_iu[r];
+          return [&p, iu](int n, double v) { return p.vp[n] + iu * v; };
+        });
       if (ncb >= nb) break;
       if (ncb != cb) ns = nslabs(ncb);
       cb = ncb;
@@ -223,26 +197,16 @@ static inline size_t stream_smem(bool zshared, int d) {
   return sizeof(double) * ((size_t)kSK * (kSPadM + kSPadN) + 7 * kSM + 32 + (zshared ? (size_t)kSM * d : 0));
 }
 
-// CTAs per launch (persistent grid: as many as can be resident); the workspace holds one z tile per CTA for d > 512
+// CTAs per launch; the workspace holds one z tile per CTA for d > 512
 static int stream_ctas(int d, int64_t* ctas) {
   const bool zshared = d <= kZSharedMaxDim;
-  auto kern = zshared ? mvt_stream_lw_kernel<true> : mvt_stream_lw_kernel<false>;
-  const size_t smem = stream_smem(zshared, d);
-  VB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  int per_sm = 0;
-  VB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, 256, smem));
-  if (per_sm < 1) return set_error(VB_ERR_UNSUPPORTED, "mvt_target_log_weights: kernel does not fit on an SM");
-  *ctas = (int64_t)per_sm * sm_count();
-  return VB_OK;
+  return persistent_ctas(zshared ? mvt_stream_lw_kernel<true> : mvt_stream_lw_kernel<false>, 256, stream_smem(zshared, d),
+                         ctas);
 }
 
 static size_t stream_ws_layout(int d, int64_t ctas, size_t* off_z) {
   *off_z = 256;
   return 256 + (d > kZSharedMaxDim ? sizeof(double) * (size_t)ctas * kSM * d : 0);
-}
-
-static inline double t_coord_const(double df) {
-  return lgamma(0.5 * (df + 1.0)) - lgamma(0.5 * df) - 0.5 * log(df * 3.14159265358979323846);
 }
 
 }  // namespace vb
@@ -268,22 +232,16 @@ extern "C" int vb_mvt_target_log_weights_f64(const double* var_param, const doub
     return set_error(VB_ERR_INVALID_ARG, "mvt_target_log_weights: bad arguments");
   if (n_total > (INT64_MAX / 2) / d) return set_error(VB_ERR_INVALID_ARG, "mvt_target_log_weights: n_total * d too large");
   if (!(df > 2.0)) return set_error(VB_ERR_INVALID_ARG, "df must be greater than 2");
-  if (target_kind < -1 || target_kind > 1)
-    return set_error(VB_ERR_INVALID_ARG, "mvt_target_log_weights: target_kind is -1 (none), 0 (Gaussian) or 1 (Student-t)");
-  if (target_kind >= 0 && (!target_loc || !target_scale))
-    return set_error(VB_ERR_INVALID_ARG, "mvt_target_log_weights: bad arguments");
-  if (target_kind == 1 && !(target_df > 0.0))
-    return set_error(VB_ERR_INVALID_ARG, "mvt_target_log_weights: target_df must be positive");
+  int rc = check_product_target("mvt_target_log_weights", target_kind, true, target_loc, target_scale, target_df);
+  if (rc) return rc;
   int64_t ctas = 0;
-  int rc = stream_ctas(d, &ctas);
+  rc = stream_ctas(d, &ctas);
   if (rc) return rc;
   size_t off_z;
   if (!workspace || workspace_bytes < stream_ws_layout(d, ctas, &off_z))
     return set_error(VB_ERR_WORKSPACE, "mvt_target_log_weights: workspace too small");
   if (count == 0) return VB_OK;
-  const int64_t tiles = ceil_div(count, kSM);
-  const int64_t grid = tiles < ctas ? tiles : ctas;
-  if (grid > INT32_MAX) return set_error(VB_ERR_UNSUPPORTED, "mvt_target_log_weights: more than 2^31 - 1 CTAs");
+  const int64_t tiles = ceil_div(count, kSM), grid = tiles < ctas ? tiles : ctas;
   char* ws = static_cast<char*>(workspace);
   MvtStreamArgs p;
   p.vp = var_param;
@@ -304,7 +262,7 @@ extern "C" int vb_mvt_target_log_weights_f64(const double* var_param, const doub
   p.df = df;
   p.logq_const = mvt_const(df, d);
   p.target_df = target_df;
-  p.target_const = target_kind == 0 ? -0.5 * kLog2Pi * d : target_kind == 1 ? d * t_coord_const(target_df) : 0.0;
+  p.target_const = product_target_const(target_kind, d, target_df);
   rc = mvt_logdiag(var_param, d, reinterpret_cast<double*>(ws), stream);
   if (rc) return rc;
   const bool zshared = d <= kZSharedMaxDim;

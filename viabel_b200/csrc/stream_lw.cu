@@ -7,6 +7,7 @@
 //   vb_philox_student_t_f64), exactly what approx.sample(var_param, n) would have drawn.
 // ALU bound (Box-Muller / Marsaglia-Tsang per element), not an HBM kernel.
 #include "philox_draws.cuh"
+#include "stream_internal.cuh"
 
 namespace vb {
 
@@ -50,17 +51,13 @@ __global__ void __launch_bounds__(256) mf_target_lw_kernel(const double* __restr
       lq += family == VB_FAMILY_MF_GAUSSIAN ? -0.5 * e * e - 0.5 * kLog2Pi
                                             : tconst_q - 0.5 * (df + 1.0) * log1p(e * e / df);
       const double z = (th - tl[j]) / ts[j];
-      lp += target_kind == 0 ? -0.5 * z * z - 0.5 * kLog2Pi
-                             : tconst_p - 0.5 * (target_df + 1.0) * log1p(z * z / target_df);
+      lp += target_kind == 0 ? product_target_term(0, z, target_df) - 0.5 * kLog2Pi
+                             : tconst_p + product_target_term(1, z, target_df);
     }
     lq = warp_sum(lq);
     lp = warp_sum(lp);
     if (lane == 0) lw[i] = (lp - pconst) - (lq - qconst);
   }
-}
-
-static inline double t_const(double df) {
-  return lgamma(0.5 * (df + 1.0)) - lgamma(0.5 * df) - 0.5 * log(df * 3.14159265358979323846);
 }
 
 }  // namespace vb
@@ -70,13 +67,13 @@ extern "C" int vb_mf_target_log_weights_f64(const double* var_param, int64_t n, 
                                             uint64_t offset, int quantize, int target_kind, const double* target_loc,
                                             const double* target_scale, double target_df, double* lw, double* theta_out,
                                             cudaStream_t stream) {
-  if (!var_param || n < 0 || d <= 0 || !target_loc || !target_scale || (n > 0 && !lw))
+  if (!var_param || n < 0 || d <= 0 || (n > 0 && !lw))
     return set_error(VB_ERR_INVALID_ARG, "mf_target_log_weights: bad arguments");
+  const int rc = check_product_target("mf_target_log_weights", target_kind, false, target_loc, target_scale, target_df);
+  if (rc) return rc;
   if (d > kLwMaxDim) return set_error(VB_ERR_UNSUPPORTED, "mf_target_log_weights: d > 4096 not supported");
   if (family != VB_FAMILY_MF_GAUSSIAN && family != VB_FAMILY_MF_STUDENT) return set_error(VB_ERR_INVALID_ARG, "unknown mean-field family");
   if (family == VB_FAMILY_MF_STUDENT && !(df > 2.0)) return set_error(VB_ERR_INVALID_ARG, "df must be greater than 2");
-  if (target_kind != 0 && target_kind != 1) return set_error(VB_ERR_INVALID_ARG, "mf_target_log_weights: target_kind is 0 (Gaussian) or 1 (Student-t)");
-  if (target_kind == 1 && !(target_df > 0.0)) return set_error(VB_ERR_INVALID_ARG, "mf_target_log_weights: target_df must be positive");
   if (n == 0) return VB_OK;
   const size_t smem = sizeof(double) * 4 * (size_t)d;
   if (smem > 48 * 1024) VB_CUDA(cudaFuncSetAttribute(mf_target_lw_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
@@ -84,8 +81,8 @@ extern "C" int vb_mf_target_log_weights_f64(const double* var_param, int64_t n, 
   const int64_t cap = (int64_t)sm_count() * 8;
   if (blocks > cap) blocks = cap;
   mf_target_lw_kernel<<<(unsigned)blocks, 256, smem, stream>>>(
-      var_param, n, d, family, df, family == VB_FAMILY_MF_STUDENT ? t_const(df) : 0.0, seed, offset, quantize, target_kind,
-      target_loc, target_scale, target_df, target_kind == 1 ? t_const(target_df) : 0.0, lw, theta_out);
+      var_param, n, d, family, df, family == VB_FAMILY_MF_STUDENT ? student_t_log_const(df) : 0.0, seed, offset, quantize,
+      target_kind, target_loc, target_scale, target_df, target_kind == 1 ? student_t_log_const(target_df) : 0.0, lw, theta_out);
   VB_CHECK_LAUNCH();
   return VB_OK;
 }

@@ -5,7 +5,7 @@
 // In the reference these are user Python under autograd (models.py:27-39, objectives.py:161-167).  One warp per sample
 // row: coalesced reads of theta, coalesced writes of the gradient row, a warp reduction for log p.  HBM bound
 // (16 S d bytes), O(S d) flops; the streamed form used by vi_diagnostics at scale is stream_lw.cu.
-#include "common.cuh"
+#include "stream_internal.cuh"
 
 namespace vb {
 
@@ -22,10 +22,10 @@ __global__ void __launch_bounds__(256) target_logp_grad_kernel(const double* __r
       const double sc = scale[j];
       const double z = (theta[s * d + j] - loc[j]) / sc;
       if (kind == 0) {
-        lp += -0.5 * z * z;
+        lp += product_target_term(0, z, df);
         if (grad) grad[s * d + j] = -z / sc;
       } else {
-        lp += -0.5 * (df + 1.0) * log1p(z * z / df);
+        lp += product_target_term(1, z, df);
         if (grad) grad[s * d + j] = -(df + 1.0) * z / ((df + z * z) * sc);
       }
     }
@@ -41,9 +41,9 @@ using namespace vb;
 extern "C" int vb_target_logp_grad_f64(const double* theta, int64_t S, int d, int kind, const double* loc,
                                        const double* scale, double df, double log_norm_const, double* logp, double* grad,
                                        cudaStream_t stream) {
-  if (!theta || !loc || !scale || !logp || S <= 0 || d <= 0) return set_error(VB_ERR_INVALID_ARG, "target_logp_grad: bad arguments");
-  if (kind != 0 && kind != 1) return set_error(VB_ERR_INVALID_ARG, "target_logp_grad: kind must be 0 (Gaussian) or 1 (Student-t)");
-  if (kind == 1 && !(df > 0)) return set_error(VB_ERR_INVALID_ARG, "target_logp_grad: df must be positive");
+  if (!theta || !logp || S <= 0 || d <= 0) return set_error(VB_ERR_INVALID_ARG, "target_logp_grad: bad arguments");
+  const int rc = check_product_target("target_logp_grad", kind, false, loc, scale, df);
+  if (rc) return rc;
   int64_t blocks = (S + 7) / 8;                     // 8 warps per CTA, one sample row per warp
   const int64_t cap = (int64_t)sm_count() * 8;
   if (blocks > cap) blocks = cap;

@@ -362,6 +362,13 @@ def _target_logp_grad(theta, kind, loc, scale, df, const):
     return lp, G
 
 
+def _product_target(model):
+    """(kind, loc, scale, df) of a built-in product target for the fused kernels, else None (exact types only)."""
+    if type(model) in (GaussianTarget, StudentTTarget):
+        return (0, model.mean, model.sd, 0.0) if type(model) is GaussianTarget else (1, model.loc, model.scale, model.df)
+    return None
+
+
 class GaussianTarget(Model):
     """Independent Gaussian target sum_j N(theta_j; mean_j, sd_j) (the reference tests' target,
     tests/test_objectives.py:18-19) with its analytic gradient."""
