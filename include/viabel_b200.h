@@ -136,6 +136,9 @@ int vb_glm_fast_sweep(void* handle, const double* theta, const double* base, con
  *   w[s] = exp(alpha*(lw[s]-m)); value = log(mean w)/alpha + m          (:456-459)
  * vb_mf_objective_finish_f64: value[0] and grad[2d] from the (all-reduced) sweep sums.
  *   For VB_OBJ_ALPHA pass the weights used in the sweep; otherwise w = NULL.
+ *   The ExclusiveKL value is summed over blocks of 8 samples in a fixed order through
+ *   vb_mf_objective_finish_workspace_bytes(S) bytes of workspace (VB_ERR_WORKSPACE below;
+ *   not used, and may be NULL, for VB_OBJ_ALPHA or without value and logp).
  * ------------------------------------------------------------------------------------- */
 int vb_mf_alpha_weights_f64(const double* var_param, const double* theta, const double* base,
                             const double* ll, int64_t S, int d, int family, double df,
@@ -145,7 +148,9 @@ int vb_mf_objective_finish_f64(const double* var_param, const double* theta, con
                                const double* ll, const double* gmu, const double* ge,
                                const double* w, int64_t S, int d, int family, double df,
                                double prior_sd, int objective, double alpha, double* value,
-                               double* grad, double* logp, cudaStream_t stream);
+                               double* grad, double* logp, void* workspace, size_t workspace_bytes,
+                               cudaStream_t stream);
+size_t vb_mf_objective_finish_workspace_bytes(int64_t S);
 
 /* ---------------------------------------------------------------------------------------
  * Optimiser steps fused with the parameter update (optimization.py:188-197 RMSProp,

@@ -41,8 +41,9 @@ _PROTOS = {
                                  P, P, P, P, c_size_t, P]),
     'vb_mf_alpha_weights_f64': (c_int, [P, P, P, P, c_int64, c_int, c_int, c_double, c_double, c_double,
                                         P, P, P, P]),
+    'vb_mf_objective_finish_workspace_bytes': (c_size_t, [c_int64]),
     'vb_mf_objective_finish_f64': (c_int, [P, P, P, P, P, P, P, c_int64, c_int, c_int, c_double, c_double,
-                                           c_int, c_double, P, P, P, P]),
+                                           c_int, c_double, P, P, P, P, c_size_t, P]),
     'vb_rmsprop_step_f64': (c_int, [P, P, P, P, c_int64, c_double, c_double, c_double, c_int, P]),
     'vb_adam_step_f64': (c_int, [P, P, P, P, P, c_int64, c_double, c_double, c_double, c_double, c_int, P]),
     'vb_glm_fast_model_bytes': (c_size_t, [c_int64, c_int]),

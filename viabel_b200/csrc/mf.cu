@@ -99,9 +99,9 @@ __global__ void __launch_bounds__(256) mf_value_kernel(const double* __restrict_
                                                        const double* __restrict__ base, const double* __restrict__ ll,
                                                        int64_t S, int d, int family, double df, double tconst,
                                                        double inv_tau2, double prior_const, int objective,
-                                                       double* __restrict__ value, double* __restrict__ logp) {
+                                                       double* __restrict__ part, double* __restrict__ logp) {
   PDL_SYNC();
-  // one warp per sample, 8 samples per block; value[0] (zeroed by the caller) receives every block's share
+  // one warp per sample, 8 samples per block; part[blockIdx.x] receives the block's share of the value
   __shared__ double red[32];
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const bool path = objective == VB_OBJ_EXCLUSIVE_KL_PATH;
@@ -124,7 +124,18 @@ __global__ void __launch_bounds__(256) mf_value_kernel(const double* __restrict_
     H = block_sum(H, red);
     if (family == VB_FAMILY_MF_GAUSSIAN) H += 0.5 * d * (1.0 + kLog2Pi);   // approximations.py:218-220
   }
-  if (threadIdx.x == 0) atomicAdd(value, -(acc / (double)S + H));
+  if (threadIdx.x == 0) part[blockIdx.x] = -(acc / (double)S + H);
+}
+
+// value[0] = sum of the n block shares of mf_value_kernel, in a fixed order (one block): deterministic
+__global__ void __launch_bounds__(256) mf_value_sum_kernel(const double* __restrict__ part, int64_t n,
+                                                           double* __restrict__ value) {
+  PDL_SYNC();
+  __shared__ double red[32];
+  double acc = 0.0;
+  for (int64_t i = threadIdx.x; i < n; i += blockDim.x) acc += part[i];
+  acc = block_sum(acc, red);
+  if (threadIdx.x == 0) value[0] = acc;
 }
 
 // gradient wrt [mu, log_sigma]  (SURVEY.md App. A.1): block = 32 coordinates x 8 sample groups
@@ -249,11 +260,16 @@ extern "C" int vb_mf_alpha_weights_f64(const double* var_param, const double* th
   return VB_OK;
 }
 
+extern "C" size_t vb_mf_objective_finish_workspace_bytes(int64_t S) {
+  return S > 0 ? sizeof(double) * (size_t)((S + 7) / 8) : 0;
+}
+
 extern "C" int vb_mf_objective_finish_f64(const double* var_param, const double* theta, const double* base,
                                           const double* ll, const double* gmu, const double* ge,
                                           const double* w, int64_t S, int d, int family, double df,
                                           double prior_sd, int objective, double alpha, double* value,
-                                          double* grad, double* logp, cudaStream_t stream) {
+                                          double* grad, double* logp, void* workspace, size_t workspace_bytes,
+                                          cudaStream_t stream) {
   if (S <= 0 || d <= 0 || !var_param || !theta || !base || !ll)
     return set_error(VB_ERR_INVALID_ARG, "mf_objective_finish: bad arguments");
   if (objective < VB_OBJ_EXCLUSIVE_KL || objective > VB_OBJ_ALPHA)
@@ -266,12 +282,18 @@ extern "C" int vb_mf_objective_finish_f64(const double* var_param, const double*
   double inv_tau2, pc;
   prior_consts(prior_sd, d, inv_tau2, pc);
   const double tc = family == VB_FAMILY_MF_STUDENT ? student_t_log_const(df) : 0.0;
+  const bool want_value = objective != VB_OBJ_ALPHA && (value || logp);
+  if (want_value) {
+    if (!value) return set_error(VB_ERR_INVALID_ARG, "mf_objective_finish: value is required");
+    if (!workspace || workspace_bytes < vb_mf_objective_finish_workspace_bytes(S))
+      return set_error(VB_ERR_WORKSPACE, "mf_objective_finish: workspace too small");
+  }
   if (value || logp) {
-    if (objective != VB_OBJ_ALPHA && !value)
-      return set_error(VB_ERR_INVALID_ARG, "mf_objective_finish: value is required");
-    if (objective != VB_OBJ_ALPHA) VB_CUDA(cudaMemsetAsync(value, 0, sizeof(double), stream));
-    VB_CUDA(launch_pdl(mf_value_kernel, dim3((unsigned)((S + 7) / 8)), dim3(256), stream, var_param, theta, base, ll, S, d, family,
-                       df, tc, inv_tau2, pc, objective, value, logp));
+    const int64_t nb = (S + 7) / 8;
+    double* part = want_value ? static_cast<double*>(workspace) : nullptr;
+    VB_CUDA(launch_pdl(mf_value_kernel, dim3((unsigned)nb), dim3(256), stream, var_param, theta, base, ll, S, d, family,
+                       df, tc, inv_tau2, pc, objective, part, logp));
+    if (want_value) VB_CUDA(launch_pdl(mf_value_sum_kernel, dim3(1), dim3(256), stream, (const double*)part, nb, value));
   }
   if (grad) {
     VB_CUDA(launch_pdl(mf_grad_kernel, dim3((d + 31) / 32), dim3(256), stream, var_param, theta, base, gmu, ge,

@@ -262,9 +262,10 @@ def _mf_objective(approx, model, S, objective, alpha, var_param, base=None, seed
                                                prior_sd, float(alpha), ptr(lw), ptr(w), ptr(value), st))
         approx.last_log_weights = lw            # log p - log q per sample (objectives.py:446)
     ll, gmu, ge = sweep(w)
+    ws = torch.empty(max(8, lib.vb_mf_objective_finish_workspace_bytes(S)), dtype=torch.uint8, device=dev)
     _lib.check(lib.vb_mf_objective_finish_f64(
         ptr(vp), ptr(theta), ptr(e), ptr(ll), ptr(gmu), ptr(ge), ptr(w), S, d, family, df, prior_sd,
-        objective, float(alpha), ptr(value), ptr(grad), ptr(logp), st))
+        objective, float(alpha), ptr(value), ptr(grad), ptr(logp), ptr(ws), ws.numel(), st))
     if want_logp:
         return value[0], grad, logp
     return value[0], grad
