@@ -317,6 +317,15 @@ int vb_faso_ess_f64(double* acov_raw, int64_t ld, double scale, int64_t n_draw, 
  *   vb_mf_score_f64: value[1] = -sum_r c_r log q(x_{i_r}; var_param), grad[2d] = its gradient wrt [mu, log sigma]
  *     (:405-416 differentiates approx.log_density at FIXED samples), c_r = scale * w[r] (w NULL: 1), i_r = idx[r]
  *     (idx NULL: r), x: [*, d].  Workspace: vb_mf_score_workspace_bytes(d).
+ *   vb_mvt_score_f64: the same score for the full-rank MultivariateT (either reparameterisation: the score depends on
+ *     var_param and the fixed rows only), grad[d + d(d+1)/2].  L^-1 on the device, then Y = (x - mu) L^-T, V = Y L^-1
+ *     and the packed-triangle cotangent on the FP64 tensor pipe (about 3 n d^2 flops plus the d^3 / 3 of the
+ *     inverse).  Workspace: vb_mvt_score_workspace_bytes(n, d), O(d^2 + n d).
+ *   vb_lr_score_f64: the same score for LRGaussian, grad[2d + d k]; P = [C^-1 | -C^-1 B^T D^-1] (k x (k + d)), C C^T =
+ *     I + B^T D^-2 B, may be NULL when k = 0.  About 8 n d k flops, nothing of size d x d.  Workspace:
+ *     vb_lr_score_workspace_bytes(n, d, k), O(n (d + k)).
+ *   All three: deterministic (fixed summation orders, no atomics), no host synchronisation; idx entries must lie in
+ *   the rows of x (not checked on the device).
  * ------------------------------------------------------------------------------------- */
 int vb_dis_bisection_f64(const double* log_prior, const double* log_p, const double* log_q, int64_t S,
                          double eps_guess, double max_eps, double ess_target, int max_its, double* w,
@@ -324,6 +333,14 @@ int vb_dis_bisection_f64(const double* log_prior, const double* log_p, const dou
 size_t vb_mf_score_workspace_bytes(int d);
 int vb_mf_score_f64(const double* var_param, const double* x, const int64_t* idx, const double* w, double scale,
                     int64_t n, int d, int family, double df, double* value, double* grad, void* workspace,
+                    size_t workspace_bytes, cudaStream_t stream);
+size_t vb_mvt_score_workspace_bytes(int64_t n, int d);
+int vb_mvt_score_f64(const double* var_param, const double* x, const int64_t* idx, const double* w, double scale,
+                     int64_t n, int d, double df, double* value, double* grad, void* workspace, size_t workspace_bytes,
+                     cudaStream_t stream);
+size_t vb_lr_score_workspace_bytes(int64_t n, int d, int k);
+int vb_lr_score_f64(const double* var_param, const double* P, const double* x, const int64_t* idx, const double* w,
+                    double scale, int64_t n, int d, int k, double* value, double* grad, void* workspace,
                     size_t workspace_bytes, cudaStream_t stream);
 
 /* ---------------------------------------------------------------------------------------

@@ -76,6 +76,10 @@ _PROTOS = {
     'vb_dis_bisection_f64': (c_int, [P, P, P, c_int64, c_double, c_double, c_double, c_int, P, P, P]),
     'vb_mf_score_workspace_bytes': (c_size_t, [c_int]),
     'vb_mf_score_f64': (c_int, [P, P, P, P, c_double, c_int64, c_int, c_int, c_double, P, P, P, c_size_t, P]),
+    'vb_mvt_score_workspace_bytes': (c_size_t, [c_int64, c_int]),
+    'vb_mvt_score_f64': (c_int, [P, P, P, P, c_double, c_int64, c_int, c_double, P, P, P, c_size_t, P]),
+    'vb_lr_score_workspace_bytes': (c_size_t, [c_int64, c_int, c_int]),
+    'vb_lr_score_f64': (c_int, [P, P, P, P, P, c_double, c_int64, c_int, c_int, P, P, P, c_size_t, P]),
     'vb_mf_target_log_weights_f64': (c_int, [P, c_int64, c_int, c_int, c_double, c_uint64, c_uint64, c_int, c_int, P, P,
                                              c_double, P, P, P]),
     'vb_gemm_f64': (c_int, [c_int, c_int, c_int, c_int, c_int, c_double, P, c_int64, P, c_int64, P, c_int64, P, P, P, P, P, P]),

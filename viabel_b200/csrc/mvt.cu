@@ -249,6 +249,10 @@ int mvt_weights_gmu(const double* f, const double* G, const double* zu2, const d
   mvt_weights_kernel<<<1, 1024, 0, stream>>>(f, zu2, S, d, df, mvt_const(df, d), half_logdet, objective, alpha, sv, scal);
   VB_CHECK_LAUNCH();
   VB_CUDA(cudaMemcpyAsync(value, scal, sizeof(double), cudaMemcpyDeviceToDevice, stream));
+  return mvt_gmu(G, sv, S, d, c, gmu, stream);
+}
+
+int mvt_gmu(const double* G, const double* sv, int S, int d, double c, double* gmu, cudaStream_t stream) {
   mvt_gmu_kernel<<<(d + 31) / 32, 1024, 0, stream>>>(G, sv, S, d, c, gmu);
   VB_CHECK_LAUNCH();
   return VB_OK;

@@ -38,22 +38,33 @@ struct TrmmStage {
   double b[kSlab * kTN / 256];               // L[n, k]
 };
 
-__device__ __forceinline__ void trmm_load(TrmmStage& st, const double* __restrict__ vp, const double* __restrict__ z, int S,
-                                          int d, int m0, int n0, int k0) {
+template <bool kScore>
+__device__ __forceinline__ void trmm_load(TrmmStage& st, const double* __restrict__ vp, const double* __restrict__ z,
+                                          const long long* __restrict__ idx, const double* __restrict__ X, int S, int d,
+                                          int m0, int n0, int k0) {
   const int k = threadIdx.x & 31, r = threadIdx.x >> 5;
   const int kk = k0 + k;
 #pragma unroll
   for (int p = 0; p < kTM / 8; ++p) {
     const int s = m0 + p * 8 + r;
-    st.a[p] = (s < S && kk < d) ? z[(size_t)s * d + kk] : 0.0;
+    double v = 0.0;
+    if (s < S && kk < d) {
+      if (kScore) v = z[(size_t)(idx ? idx[s] : s) * d + kk] - vp[kk];     // x - mu before the product
+      else v = z[(size_t)s * d + kk];
+    }
+    st.a[p] = v;
   }
 #pragma unroll
   for (int p = 0; p < kTN / 8; ++p) {
     const int n = n0 + p * 8 + r;
     double v = 0.0;
     if (n < d && kk <= n) {
-      v = vp[d + tri(n) + kk];               // row n of L is contiguous in k
-      if (kk == n) v = exp(v);
+      if (kScore) {
+        v = X[(size_t)n * d + kk];           // row n of L^-1
+      } else {
+        v = vp[d + tri(n) + kk];             // row n of L is contiguous in k
+        if (kk == n) v = exp(v);
+      }
     }
     st.b[p] = v;
   }
@@ -67,7 +78,10 @@ __device__ __forceinline__ void trmm_store(const TrmmStage& st, double (*sa)[kPa
   for (int p = 0; p < kTN / 8; ++p) sb[k][p * 8 + r] = st.b[p];
 }
 
+// kScore: Y = (x[idx] - mu) L^-T for the DIS score (below), with B read from the dense L^-1 X and no epilogue scaling.
+template <bool kScore>
 __global__ void __launch_bounds__(256) mvt_chol_trmm_kernel(const double* __restrict__ vp, const double* __restrict__ z,
+                                                            const long long* __restrict__ idx, const double* __restrict__ X,
                                                             const double* __restrict__ inv_u, int S, int d,
                                                             double* __restrict__ theta) {
   __shared__ double sa[kSlab][kPadM], sb[kSlab][kPadN];
@@ -85,7 +99,7 @@ __global__ void __launch_bounds__(256) mvt_chol_trmm_kernel(const double* __rest
 
   double acc[2][2][2];
   TrmmStage st;
-  trmm_load(st, vp, z, S, d, m0, cb0 * kTN, 0);
+  trmm_load<kScore>(st, vp, z, idx, X, S, d, m0, cb0 * kTN, 0);
   for (int it = 0; it < total; ++it) {
     const bool second = it >= ns0;
     const int sl = second ? it - ns0 : it;
@@ -102,7 +116,7 @@ __global__ void __launch_bounds__(256) mvt_chol_trmm_kernel(const double* __rest
     __syncthreads();
     if (it + 1 < total) {
       const bool second1 = it + 1 >= ns0;
-      trmm_load(st, vp, z, S, d, m0, (second1 ? cb1 : cb0) * kTN, (second1 ? it + 1 - ns0 : it + 1) * kSlab);
+      trmm_load<kScore>(st, vp, z, idx, X, S, d, m0, (second1 ? cb1 : cb0) * kTN, (second1 ? it + 1 - ns0 : it + 1) * kSlab);
     }
 #pragma unroll
     for (int k4 = 0; k4 < kSlab; k4 += 4) {
@@ -121,13 +135,13 @@ __global__ void __launch_bounds__(256) mvt_chol_trmm_kernel(const double* __rest
       for (int a = 0; a < 2; ++a) {
         const int s = m0 + wm * 16 + a * 8 + gq;
         if (s >= S) continue;
-        const double iu = inv_u[s];
+        const double iu = kScore ? 1.0 : inv_u[s];
 #pragma unroll
         for (int b = 0; b < 2; ++b)
 #pragma unroll
           for (int u = 0; u < 2; ++u) {
             const int n = n0 + wn * 16 + b * 8 + 2 * t + u;
-            if (n < d) theta[(size_t)s * d + n] = vp[n] + iu * acc[a][b][u];
+            if (n < d) theta[(size_t)s * d + n] = kScore ? acc[a][b][u] : vp[n] + iu * acc[a][b][u];
           }
       }
     }
@@ -136,7 +150,7 @@ __global__ void __launch_bounds__(256) mvt_chol_trmm_kernel(const double* __rest
 
 // ---- cotangent ---------------------------------------------------------------------------------------------------
 // Fbar = G^T diag(c sv / u) Z on the lower-triangular 64 x 64 tiles only (one CTA per tile, K = S), written straight
-// into the packed gradient.  8 warps of 16 x 32 fragments; register-prefetched slabs as above.
+// into the packed gradient; inv_u NULL means u = 1 (the DIS score).  8 warps of 16 x 32 fragments; register-prefetched slabs as above.
 struct CotStage {
   double a[kSlab * kTN / 256];               // w_s G[s, i]
   double b[kSlab * kTN / 256];               // Z[s, j]
@@ -151,7 +165,7 @@ __device__ __forceinline__ void cot_load(CotStage& st, const double* __restrict_
     const int s = k0 + p * 4 + r;
     double va = 0.0, vb = 0.0;
     if (s < S) {
-      if (i0 + col < d) va = G[(size_t)s * d + i0 + col] * (c * sv[s] * inv_u[s]);
+      if (i0 + col < d) va = G[(size_t)s * d + i0 + col] * (inv_u ? c * sv[s] * inv_u[s] : c * sv[s]);
       if (j0 + col < d) vb = z[(size_t)s * d + j0 + col];
     }
     st.a[p] = va;
@@ -332,7 +346,7 @@ __global__ void __launch_bounds__(256) mvt_chol_invlevel_kernel(const double* __
   }
 }
 
-// Gt[s][n] = G[s][n] + kappa_s / u_s sum_{k >= n} Z[s][k] X[k][n].  Column block c has the K range [64 c, d), so CTA
+// Gt[s][n] = G[s][n] + kappa_s / u_s sum_{k >= n} Z[s][k] X[k][n]  (G NULL: 0, inv_u NULL: u = 1, as the DIS score uses).  Column block c has the K range [64 c, d), so CTA
 // (p, r) takes column blocks p and nb - 1 - p of row tile r to even out the work, as the triangular transform does.
 __global__ void __launch_bounds__(256) mvt_chol_solve_kernel(const double* __restrict__ z, const double* __restrict__ X,
                                                              const double* __restrict__ G, const double* __restrict__ inv_u,
@@ -404,13 +418,13 @@ __global__ void __launch_bounds__(256) mvt_chol_solve_kernel(const double* __res
       for (int a = 0; a < 2; ++a) {
         const int s = m0 + wm * 16 + a * 8 + gq;
         if (s >= S) continue;
-        const double kiu = (df + d) / (df + zu2[s]) * inv_u[s];
+        const double kappa = (df + d) / (df + zu2[s]), kiu = inv_u ? kappa * inv_u[s] : kappa;
 #pragma unroll
         for (int b = 0; b < 2; ++b)
 #pragma unroll
           for (int u = 0; u < 2; ++u) {
             const int n = n0 + wn * 16 + b * 8 + 2 * t + u;
-            if (n < d) Gt[(size_t)s * d + n] = G[(size_t)s * d + n] + kiu * acc[a][b][u];
+            if (n < d) Gt[(size_t)s * d + n] = G ? G[(size_t)s * d + n] + kiu * acc[a][b][u] : kiu * acc[a][b][u];
           }
       }
     }
@@ -434,9 +448,8 @@ static void chol_obj_layout(int S, int d, CholObjLayout& l) {
   l.total_path = off;
 }
 
-// Gt = G + diag(kappa) Zhat L^-1 (see above); X and T are d x d scratch
-static int chol_path_gradient(const double* vp, const double* z, const double* inv_u, const double* zu2, const double* G,
-                              int S, int d, double df, double* X, double* T, double* Gt, cudaStream_t stream) {
+// X = L^-1 (dense, lower triangular; see above): the diagonal blocks, then the doubling levels; T is d x d scratch
+static int chol_inverse(const double* vp, int d, double* X, double* T, cudaStream_t stream) {
   const int nb = (d + kTN - 1) / kTN;
   mvt_chol_diaginv_kernel<<<nb, kTN, 0, stream>>>(vp, d, X);
   VB_CHECK_LAUNCH();
@@ -448,10 +461,86 @@ static int chol_path_gradient(const double* vp, const double* z, const double* i
     VB_CHECK_LAUNCH();
     if (h > INT32_MAX / 2) break;
   }
+  return VB_OK;
+}
+
+// Gt = G + diag(kappa) Zhat L^-1 (see above); X and T are d x d scratch
+static int chol_path_gradient(const double* vp, const double* z, const double* inv_u, const double* zu2, const double* G,
+                              int S, int d, double df, double* X, double* T, double* Gt, cudaStream_t stream) {
+  const int nb = (d + kTN - 1) / kTN;
+  int rc = chol_inverse(vp, d, X, T, stream);
+  if (rc) return rc;
   const int64_t ctas = (nb + 1) / 2 * ceil_div(S, kTM);
   mvt_chol_solve_kernel<<<(unsigned)ctas, 256, 0, stream>>>(z, X, G, inv_u, zu2, df, S, d, Gt);
   VB_CHECK_LAUNCH();
   return VB_OK;
+}
+
+// ---- DISInclusiveKL score: value = -sum_r c_r log q(x_r), gradient at the fixed rows x_r = x[idx[r]] ----------------
+// With y_r = L^-1 (x_r - mu), delta_r = |y_r|^2, kappa_r = (df + d) / (df + delta_r) and v_r = L^-T y_r (rows of
+// V = Y L^-1):
+//     log q_r  = const - sum_i F_ii - (df + d)/2 log1p(delta_r / df)
+//     gbar_mu  = -sum_r c_r kappa_r v_r
+//     Fbar_ij  = -sum_r c_r kappa_r v_ri y_rj  (j < i),   Fbar_ii = -L_ii sum_r c_r kappa_r v_ri y_ri + sum_r c_r
+// i.e. the cotangent above with G -> diag(kappa) V, Z -> Y, u = 1, sv = c, c = -1 and diag_add = sum_r c_r.  Pipeline:
+// L^-1 (chol_inverse), Y (triangular transform, x - mu formed on load), delta and c (one warp per row), the value
+// (one block, fixed order), diag(kappa) V (the solve kernel), gbar_mu (mvt_gmu) and Fbar (cotangent kernel).
+
+// delta[r] = |Y_r|^2,  cr[r] = scale * w[r]   (one warp per row, grid-stride)
+__global__ void __launch_bounds__(256) mvt_score_rows_kernel(const double* __restrict__ Y, const double* __restrict__ w,
+                                                             double scale, int n, int d, double* __restrict__ delta,
+                                                             double* __restrict__ cr) {
+  const int lane = threadIdx.x & 31;
+  const int64_t nwarps = (int64_t)gridDim.x * (blockDim.x >> 5);
+  for (int64_t r = (blockIdx.x * (int64_t)blockDim.x + threadIdx.x) >> 5; r < n; r += nwarps) {
+    double a = 0.0;
+    for (int j = lane; j < d; j += 32) {
+      const double v = Y[r * d + j];
+      a += v * v;
+    }
+    a = warp_sum(a);
+    if (lane == 0) {
+      delta[r] = a;
+      cr[r] = scale * (w ? w[r] : 1.0);
+    }
+  }
+}
+
+// scal = {value, sum_r c_r}, value[0] = scal[0]   (single block, fixed summation order)
+__global__ void __launch_bounds__(1024) mvt_score_value_kernel(const double* __restrict__ delta, const double* __restrict__ cr,
+                                                               int n, int d, double df, double logq_const,
+                                                               const double* __restrict__ hl, double* __restrict__ scal,
+                                                               double* __restrict__ value) {
+  __shared__ double red[32];
+  const double c0 = logq_const - hl[0];
+  double a = 0.0, b = 0.0;
+  for (int r = threadIdx.x; r < n; r += blockDim.x) {
+    a += cr[r] * (c0 - 0.5 * (df + d) * log1p(delta[r] / df));
+    b += cr[r];
+  }
+  a = block_sum(a, red);
+  b = block_sum(b, red);
+  if (threadIdx.x == 0) {
+    scal[0] = value[0] = -a;
+    scal[1] = b;
+  }
+}
+
+struct ScoreLayout {
+  size_t off_X, off_T, off_Y, off_KV, off_delta, off_cr, off_scal, off_hl, total;
+};
+static void score_layout(int64_t n, int d, ScoreLayout& l) {
+  size_t off = 0;
+  auto take = [&](size_t bytes) { size_t o = off; off = align_up(off + bytes, 256); return o; };
+  l.off_X = take(sizeof(double) * (size_t)d * d);
+  l.off_T = take(sizeof(double) * (size_t)d * d);
+  l.off_Y = take(sizeof(double) * (size_t)n * d);
+  l.off_KV = take(sizeof(double) * (size_t)n * d);
+  l.off_delta = take(sizeof(double) * (size_t)n);
+  l.off_cr = take(sizeof(double) * (size_t)n);
+  l.off_scal = take(sizeof(double) * 4);
+  l.off_hl = take(sizeof(double));
+  l.total = off;
 }
 
 }  // namespace vb
@@ -469,7 +558,7 @@ extern "C" int vb_mvt_chol_transform_f64(const double* var_param, const double* 
   const int64_t nb = ceil_div(d, kTN);
   const int64_t ctas = (nb + 1) / 2 * ceil_div(S, kTM);
   if (ctas > INT32_MAX) return set_error(VB_ERR_UNSUPPORTED, "mvt_chol_transform: more than 2^31 - 1 tiles");
-  mvt_chol_trmm_kernel<<<(unsigned)ctas, 256, 0, stream>>>(var_param, z, inv_u, S, d, theta);
+  mvt_chol_trmm_kernel<false><<<(unsigned)ctas, 256, 0, stream>>>(var_param, z, nullptr, nullptr, inv_u, S, d, theta);
   VB_CHECK_LAUNCH();
   return VB_OK;
 }
@@ -527,6 +616,60 @@ extern "C" int vb_mvt_chol_objective_f64(const double* var_param, const double* 
   if (rc) return rc;
   const double c = objective == VB_OBJ_ALPHA ? alpha / S : -1.0 / S;
   mvt_chol_cotangent_kernel<<<(unsigned)(nb * (nb + 1) / 2), 256, 0, stream>>>(var_param, z, inv_u, Gc, sv, scal, c, S, d, grad);
+  VB_CHECK_LAUNCH();
+  return VB_OK;
+}
+
+/* workspace of vb_mvt_score_f64: 2 d^2 + 2 n d + 2 n + 5 doubles (256-byte aligned pieces) */
+extern "C" size_t vb_mvt_score_workspace_bytes(int64_t n, int d) {
+  if (n <= 0 || d <= 0) return 0;
+  ScoreLayout l;
+  score_layout(n, d, l);
+  return l.total;
+}
+
+/* value[1] = -sum_r c_r log q(x_{i_r}; var_param) and grad[d + d(d+1)/2] (DISInclusiveKL's score, see above),
+ * c_r = scale * w[r] (w NULL: 1), i_r = idx[r] (idx NULL: r).  Both reparameterisations: the score depends on
+ * var_param and the fixed rows only. */
+extern "C" int vb_mvt_score_f64(const double* var_param, const double* x, const int64_t* idx, const double* w, double scale,
+                                int64_t n, int d, double df, double* value, double* grad, void* workspace,
+                                size_t workspace_bytes, cudaStream_t stream) {
+  if (!var_param || !x || n <= 0 || d <= 0 || !value || !grad) return set_error(VB_ERR_INVALID_ARG, "mvt_score: bad arguments");
+  if (!(df > 2.0)) return set_error(VB_ERR_INVALID_ARG, "df must be greater than 2");
+  ScoreLayout l;
+  score_layout(n, d, l);
+  if (!workspace || workspace_bytes < l.total) return set_error(VB_ERR_WORKSPACE, "mvt_score: workspace too small");
+  const int64_t nb = ceil_div(d, kTN);
+  const int64_t row_ctas = (nb + 1) / 2 * ceil_div(n, kTM);
+  if (n > INT32_MAX || row_ctas > INT32_MAX || nb * nb > INT32_MAX)
+    return set_error(VB_ERR_UNSUPPORTED, "mvt_score: more than 2^31 - 1 tiles");
+  char* ws = static_cast<char*>(workspace);
+  double* X = reinterpret_cast<double*>(ws + l.off_X);
+  double* Y = reinterpret_cast<double*>(ws + l.off_Y);
+  double* KV = reinterpret_cast<double*>(ws + l.off_KV);
+  double* delta = reinterpret_cast<double*>(ws + l.off_delta);
+  double* cr = reinterpret_cast<double*>(ws + l.off_cr);
+  double* scal = reinterpret_cast<double*>(ws + l.off_scal);
+  double* hl = reinterpret_cast<double*>(ws + l.off_hl);
+  const int nr = (int)n;
+  int rc = chol_inverse(var_param, d, X, reinterpret_cast<double*>(ws + l.off_T), stream);
+  if (rc) return rc;
+  mvt_chol_trmm_kernel<true><<<(unsigned)row_ctas, 256, 0, stream>>>(var_param, x, reinterpret_cast<const long long*>(idx), X,
+                                                                       nullptr, nr, d, Y);
+  VB_CHECK_LAUNCH();
+  const int64_t blocks = ceil_div(n, 256 / 32), cap = 64LL * sm_count();
+  mvt_score_rows_kernel<<<(unsigned)(blocks < cap ? blocks : cap), 256, 0, stream>>>(Y, w, scale, nr, d, delta, cr);
+  VB_CHECK_LAUNCH();
+  rc = mvt_logdiag(var_param, d, hl, stream);
+  if (rc) return rc;
+  mvt_score_value_kernel<<<1, 1024, 0, stream>>>(delta, cr, nr, d, df, mvt_const(df, d), hl, scal, value);
+  VB_CHECK_LAUNCH();
+  mvt_chol_solve_kernel<<<(unsigned)row_ctas, 256, 0, stream>>>(Y, X, nullptr, nullptr, delta, df, nr, d, KV);
+  VB_CHECK_LAUNCH();
+  rc = mvt_gmu(KV, cr, nr, d, -1.0, grad, stream);
+  if (rc) return rc;
+  mvt_chol_cotangent_kernel<<<(unsigned)(nb * (nb + 1) / 2), 256, 0, stream>>>(var_param, Y, nullptr, KV, cr, scal, -1.0, nr, d,
+                                                                                grad);
   VB_CHECK_LAUNCH();
   return VB_OK;
 }

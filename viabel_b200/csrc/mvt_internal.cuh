@@ -32,4 +32,7 @@ int mvt_logdiag(const double* var_param, int d, double* out, cudaStream_t stream
 int mvt_weights_gmu(const double* f, const double* G, const double* zu2, const double* half_logdet, int S, int d, double df,
                     int objective, double alpha, double* sv, double* scal, double* value, double* gmu, cudaStream_t stream);
 
+// gmu[j] = c sum_s sv_s G[s][j], summed in a fixed order (32 sample groups, then the groups in order)
+int mvt_gmu(const double* G, const double* sv, int S, int d, double c, double* gmu, cudaStream_t stream);
+
 }  // namespace vb

@@ -5,6 +5,7 @@ The reference differentiates a Python closure with autograd; here `objective(var
 launches the fused CUDA sweep (sample -> model log density + gradient -> reduction) and
 assembles the analytic gradient of SURVEY.md App. A on the device.
 """
+import math
 from abc import ABC, abstractmethod
 
 import numpy as np
@@ -432,7 +433,9 @@ class DISInclusiveKL(StochasticVariationalObjective):
     Forward-only in the model (no model gradient is ever needed): every `num_resampling_batches`-th
     call draws S samples, evaluates log q and log p, finds the tempering epsilon by bisection on the
     effective sample size, and then each call resamples from the tempered weights and differentiates
-    -log q(lambda; x) at the FIXED samples (score terms).  Mean-field families only here."""
+    -log q(lambda; x) at the FIXED samples (score terms).  Any family with a log density: the mean-field families,
+    MultivariateT (both reparameterisations) and LRGaussian take the score from CUDA kernels (csrc/dis.cu,
+    csrc/mvt_chol.cu, csrc/lr_score.cu), NVPFlow from torch autograd of its log density; NeuralNet has no density."""
 
     def __init__(self, approx, model, num_mc_samples, ess_target, temper_prior, temper_prior_params,
                  use_resampling=True, num_resampling_batches=1, w_clip_threshold=10):
@@ -497,23 +500,70 @@ class DISInclusiveKL(StochasticVariationalObjective):
         return idx
 
     def _score(self, vp, x, idx, w, scale):
-        """(value, grad) = -sum_r c_r log q(x_r; lambda) and its gradient at the fixed samples (vb_mf_score_f64)."""
+        """(value, grad) = -sum_r c_r log q(x_r; lambda) and its gradient at the fixed samples, c_r = scale * w_r."""
         approx = self.approx
         d = approx.dim
-        out = torch.empty(1 + 2 * d, dtype=F64, device=vp.device)
-        ws = torch.empty(max(8, _lib.lib.vb_mf_score_workspace_bytes(d)), dtype=torch.uint8, device=vp.device)
         n = int(idx.numel()) if idx is not None else int(x.shape[0])
-        _lib.check(_lib.lib.vb_mf_score_f64(
-            _lib.ptr(vp), _lib.ptr(x), _lib.ptr(idx), _lib.ptr(w), float(scale), n, d, approx._family,
-            float(approx.df) if approx._family else 0.0, _lib.ptr(out[:1]), _lib.ptr(out[1:]), _lib.ptr(ws), ws.numel(),
-            _lib.stream()))
+        if not isinstance(approx, _MeanField) and vp.numel() != approx.var_param_dim:
+            raise ValueError('var_param has the wrong length')
+        if isinstance(approx, NVPFlow):
+            with torch.enable_grad():
+                lam = vp.detach().clone().requires_grad_(True)
+                lq = approx.log_density_t(lam, x if idx is None else x[idx])
+                value = -scale * (lq if w is None else w * lq).sum()
+                (grad,) = torch.autograd.grad(value, lam)
+            return value.detach().reshape(1), grad
+        out = torch.empty(1 + vp.numel(), dtype=F64, device=vp.device)
+        lib, ptr = _lib.lib, _lib.ptr
+        if isinstance(approx, MultivariateT):
+            ws = torch.empty(lib.vb_mvt_score_workspace_bytes(n, d), dtype=torch.uint8, device=vp.device)
+            _lib.check(lib.vb_mvt_score_f64(
+                ptr(vp), ptr(x), ptr(idx), ptr(w), float(scale), n, d, float(approx.df), ptr(out[:1]), ptr(out[1:]),
+                ptr(ws), ws.numel(), _lib.stream()))
+        elif isinstance(approx, LRGaussian):
+            from .convenience import _lr_projection
+            P = _lr_projection(vp, approx)
+            ws = torch.empty(lib.vb_lr_score_workspace_bytes(n, d, approx.k), dtype=torch.uint8, device=vp.device)
+            _lib.check(lib.vb_lr_score_f64(
+                ptr(vp), ptr(P), ptr(x), ptr(idx), ptr(w), float(scale), n, d, approx.k, ptr(out[:1]), ptr(out[1:]),
+                ptr(ws), ws.numel(), _lib.stream()))
+        else:
+            ws = torch.empty(max(8, lib.vb_mf_score_workspace_bytes(d)), dtype=torch.uint8, device=vp.device)
+            _lib.check(lib.vb_mf_score_f64(
+                ptr(vp), ptr(x), ptr(idx), ptr(w), float(scale), n, d, approx._family,
+                float(approx.df) if approx._family else 0.0, ptr(out[:1]), ptr(out[1:]), ptr(ws), ws.numel(),
+                _lib.stream()))
         return out[:1], out[1:]
+
+    def _mvt_draws(self, vp, S, base):
+        """(x, log q(x)) for MultivariateT at a refresh: log q from the closed form at the draw,
+        const - sum_i F_ii - (df + d)/2 log1p(|z/u|^2 / df), with no second eigensolver (sqrtm) and none at all
+        (Cholesky).  In sqrtm mode an eigenvalue of Sigma at or below 1e-10, which the reference's log density drops
+        from its pseudo-inverse, is refused, as streamed vi_diagnostics refuses it."""
+        approx = self.approx
+        d, df = approx.dim, float(approx.df)
+        if vp.numel() != approx.var_param_dim:
+            raise ValueError('var_param has the wrong length')
+        chi2, z = approx.base_draws(S) if base is None else (to_dev(base[0]).reshape(-1), to_dev(base[1]))
+        approx.last_base = (chi2, z)
+        if approx.reparam == 'cholesky':
+            x, _, zu2 = approx.chol_transform(vp, chi2, z)
+        else:
+            _, _, w, V = approx.decompose(vp)
+            if float(w.min()) <= 1e-10:
+                raise NotImplementedError('DISInclusiveKL for MultivariateT needs every eigenvalue of Sigma above 1e-10 '
+                                          "in sqrtm mode; use reparam='cholesky'")
+            x, _, zu2 = approx.transform(vp, chi2, z, w, V)
+        i = torch.arange(d, device=vp.device)
+        half_logdet = vp[d + i * (i + 3) // 2].sum()
+        const = math.lgamma(0.5 * (df + d)) - math.lgamma(0.5 * df) - 0.5 * d * math.log(math.pi * df)
+        return x, const - half_logdet - 0.5 * (df + d) * torch.log1p(zu2 / df)
 
     def _update_objective_and_grad(self):
         approx = self.approx
-        if approx is not None and not isinstance(approx, _MeanField):
-            def unsupported(var_param):
-                raise NotImplementedError('DISInclusiveKL is implemented for mean-field families')
+        if approx is not None and not isinstance(approx, (_MeanField, MultivariateT, LRGaussian, NVPFlow)):
+            def unsupported(var_param, base=None):
+                raise NotImplementedError('DISInclusiveKL needs a family with a log density')
             self._objective_and_grad = unsupported
             return
 
@@ -522,9 +572,12 @@ class DISInclusiveKL(StochasticVariationalObjective):
             vp = to_dev(var_param)
             S = self.num_mc_samples
             if not self._use_resampling or self._objective_step % self._num_resampling_batches == 0:
-                x = approx.sample(vp, S) if base is None else approx.sample(vp, S, base=base)
+                if isinstance(approx, MultivariateT):
+                    x, self._state_log_q = self._mvt_draws(vp, S, base)
+                else:
+                    x = approx.sample(vp, S) if base is None else approx.sample(vp, S, base=base)
+                    self._state_log_q = approx.log_density(vp, x)
                 self._state_samples = x
-                self._state_log_q = approx.log_density(vp, x)
                 self._state_log_p = self.model(x)
                 log_prior = self._temper_prior.log_density(to_dev(self._temper_prior_params), x)
                 self._eps, ess, w = self._get_eps_and_weights(self._eps, log_prior, self._state_log_p,
