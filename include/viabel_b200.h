@@ -522,6 +522,24 @@ int vb_psislw_f64(const double* lw, double* out, int64_t n, double reff, int exa
                   int64_t* tail_idx, int32_t* tail_rank, void* workspace, size_t workspace_bytes,
                   cudaStream_t stream);
 
+/* vb_psislw_batch_f64: every column of an n x m matrix of log-weights smoothed separately, in one launch
+ * (viabel/_psis.py:113-209 for 2-D lw, and psisloo :69-110).  Column j starts at lw + j*ld (column-major, ld >= n);
+ * one CTA holds one column in shared memory, so n may not exceed vb_psis_batch_max_n(reff) (VB_ERR_UNSUPPORTED
+ * above it; the limit falls as reff falls, because the tail length M can reach 0.2 n).  Same results as
+ * vb_psislw_f64 on each column: maximum and cutoff bit-equal, the same tail set, ties ranked by index.
+ *   out    [n x m, leading dimension ldo >= n] smoothed, normalised log-weights; may be lw itself (with ldo == ld)
+ *          or NULL (no write).
+ *   khat   [m] k-hat per column (+inf when the tail has <= 4 entries or the column holds a NaN).
+ *   result [m][16] or NULL: per-column rows in the layout of vb_psislw_f64's result[] -- [0] k-hat, [1] sigma,
+ *          [2] n2, [3] shifted cutoff, [4] log-sum-exp, [5] max, [9] M, [10] n, [11] smoothed; the other slots are 0.
+ *   loo    [m] or NULL: log-sum-exp over i of (out_i + (-lw_i)), psisloo's sumlogs(lw_smoothed + log_lik) for
+ *          lw = -log_lik.  With out == NULL this makes psisloo one read of the matrix.
+ * m == 0 is a no-op.  VB_ERR_INVALID_ARG for n <= 1, m < 0, ld < n, ldo < n (with out), reff <= 0 or a NULL lw /
+ * khat; nothing is written then.  No host synchronisation; repeated calls are bitwise equal. */
+int64_t vb_psis_batch_max_n(double reff);
+int vb_psislw_batch_f64(const double* lw, int64_t ld, int64_t n, int64_t m, double reff, double* out, int64_t ldo,
+                        double* khat, double* result, double* loo, cudaStream_t stream);
+
 /* Draw-sharded PSIS (SURVEY.md 8(e)): the n_global log-weights of ONE column are split over `world`
  * ranks, rank r holding n_local consecutive draws starting at global index idx_off.  Same
  * algorithm and results as vb_psislw_f64 (= viabel/_psis.py:113-209), in three stream-ordered

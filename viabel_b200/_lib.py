@@ -54,6 +54,8 @@ _PROTOS = {
     'vb_psis_workspace_bytes': (c_size_t, [c_int64, c_double]),
     'vb_psis_tail_capacity': (c_int64, [c_int64, c_double]),
     'vb_psislw_f64': (c_int, [P, P, c_int64, c_double, c_int, P, P, P, P, c_size_t, P]),
+    'vb_psis_batch_max_n': (c_int64, [c_double]),
+    'vb_psislw_batch_f64': (c_int, [P, c_int64, c_int64, c_int64, c_double, P, c_int64, P, P, P, P]),
     'vb_psis_dist_workspace_bytes': (c_size_t, [c_int64, c_int64, c_double, c_int]),
     'vb_psis_dist_record_doubles': (c_int64, [c_int64, c_double]),
     'vb_psis_dist_local': (c_int, [P, c_int64, c_int64, c_int64, c_double, c_int, c_int, P, P, c_size_t, P]),

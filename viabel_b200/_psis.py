@@ -4,13 +4,16 @@ The n log-weights stay on the device; the reference's full argsort is replaced b
 threshold + radix-select pipeline (see csrc/psis.cu).  gpdfitnew / gpinv / sumlogs keep their
 reference signatures as thin host helpers for small arrays.
 """
+from ctypes import c_void_p
+
 import numpy as np
 import torch
 
 from . import _lib
 from ._tensor import F64, device, is_host, to_dev
 
-__all__ = ['psislw', 'psislw_device', 'psislw_sharded', 'PsisShard', 'psisloo', 'gpdfitnew', 'gpinv', 'sumlogs']
+__all__ = ['psislw', 'psislw_device', 'psislw_batch_device', 'psis_batch_max_n', 'psislw_sharded', 'PsisShard',
+           'psisloo', 'gpdfitnew', 'gpinv', 'sumlogs']
 
 R_KHAT, R_SIGMA, R_N2, R_CUTOFF, R_LSE, R_MAX, R_STATUS, R_SUMV, R_SUMEXP2V, R_M, R_NCAND, R_SMOOTHED = range(12)
 
@@ -49,6 +52,77 @@ def psislw_device(lw, out=None, Reff=1.0, want_tail=False, exact=False):
                                       _lib.ptr(result), _lib.ptr(tail_idx), _lib.ptr(tail_rank),
                                       _lib.ptr(ws), ws.numel(), _lib.stream()))
     return out, result, tail_idx, tail_rank
+
+
+def psis_batch_max_n(Reff=1.0):
+    """Longest column the batched kernel holds in one CTA's shared memory (falls with Reff: M can reach 0.2 n)."""
+    return int(_lib.lib.vb_psis_batch_max_n(float(Reff)))
+
+
+def _column_major(t):
+    """Leading dimension of a 2-D tensor whose columns are contiguous, else None."""
+    n, m = t.shape
+    if m <= 1:
+        return n if (n <= 1 or t.stride(0) == 1) else None
+    return t.stride(1) if (t.stride(0) == 1 and t.stride(1) >= n) else None
+
+
+def psislw_batch_device(lw2d, out=None, Reff=1.0, want_loo=False, want_result=False):
+    """PSIS of every column of an n x m CUDA float64 matrix in one launch (vb_psislw_batch_f64).
+
+    lw2d and out must have contiguous columns (stride(0) == 1, any leading dimension >= n), as a transposed
+    contiguous [m, n] tensor or a Fortran-ordered copy has.  `out` may be lw2d itself or None (no output written).
+    Enqueues one kernel without a host sync and returns device tensors (out, khat[m], result[m, 16] or None,
+    loo[m] or None); loo[j] is log-sum-exp_i(out[i, j] - lw2d[i, j]), psisloo's term for lw2d = -log_lik.
+    n must not exceed psis_batch_max_n(Reff) (NotImplementedError)."""
+    if lw2d.dim() != 2 or lw2d.dtype != F64 or not lw2d.is_cuda:
+        raise ValueError('psislw_batch_device needs a 2-D CUDA float64 tensor')
+    n, m = lw2d.shape
+    ld = _column_major(lw2d)
+    if ld is None:
+        raise ValueError('psislw_batch_device needs contiguous columns (stride(0) == 1)')
+    ldo = n
+    if out is not None:
+        if tuple(out.shape) != (n, m) or out.dtype != F64 or out.device != lw2d.device:
+            raise ValueError('out must be an n x m float64 tensor on the device of lw2d')
+        ldo = _column_major(out)
+        if ldo is None:
+            raise ValueError('out needs contiguous columns (stride(0) == 1)')
+    khat = torch.empty(m, dtype=F64, device=lw2d.device)
+    result = torch.empty((m, 16), dtype=F64, device=lw2d.device) if want_result else None
+    loo = torch.empty(m, dtype=F64, device=lw2d.device) if want_loo else None
+    if m == 0:
+        return out, khat, result, loo
+    _lib.check(_lib.lib.vb_psislw_batch_f64(
+        c_void_p(lw2d.data_ptr()), max(ld, n), n, m, float(Reff),
+        None if out is None else c_void_p(out.data_ptr()), max(ldo, n),
+        _lib.ptr(khat), _lib.ptr(result), _lib.ptr(loo), _lib.stream()))
+    return out, khat, result, loo
+
+
+def _psis_columns(cols, Reff):
+    """Columns longer than the batched kernel holds: the one-column pipeline on every row of the contiguous [m, n]
+    tensor `cols` (smoothed in place), all enqueued before ONE read of the [m, 16] result rows; the columns whose
+    sampled threshold missed (status 1, nothing written) are rerun in exact mode.  Returns k-hat (numpy)."""
+    m, n = cols.shape
+    res = torch.empty((m, 16), dtype=F64, device=cols.device)
+    ws = _workspace(n, Reff)
+
+    def run(i, exact):
+        _lib.check(_lib.lib.vb_psislw_f64(_lib.ptr(cols[i]), _lib.ptr(cols[i]), n, float(Reff), int(exact),
+                                          _lib.ptr(res[i]), None, None, _lib.ptr(ws), ws.numel(), _lib.stream()))
+    for i in range(m):
+        run(i, False)
+    r = res.cpu().numpy()
+    redo = np.flatnonzero(r[:, R_STATUS] == 1)
+    for i in redo:
+        run(i, True)
+    if redo.size:
+        r[redo] = res[torch.as_tensor(redo, device=cols.device)].cpu().numpy()
+    bad = np.flatnonzero(r[:, R_STATUS] != 0)
+    if bad.size:
+        raise RuntimeError('viabel_b200: PSIS failed with status %d' % int(r[bad[0], R_STATUS]))
+    return r[:, R_KHAT].copy()
 
 
 def _psis_column(col, out, Reff, want_tail):
@@ -103,24 +177,41 @@ def psislw(lw, Reff=1.0, overwrite_lw=False, return_tail=False):
     if return_tail:
         raise ValueError('return_tail is only available for 1-D input')
     m = lw_np.shape[1] if host else lw.shape[1]
-    kss = np.empty(m)
+    # columns that fit one CTA's shared memory: one launch for the whole matrix; longer ones: the one-column pipeline
+    batched = n <= psis_batch_max_n(Reff)
     if host:
-        out_np = lw_np if (overwrite_lw and lw_np.flags.f_contiguous and lw_np.dtype == np.float64) \
-            else np.copy(lw_np, order='F').astype(np.float64, copy=False)
-        for i in range(m):
-            col = to_dev(np.ascontiguousarray(lw_np[:, i]))
-            res, _, _ = _psis_column(col, col, Reff, False)
-            out_np[:, i] = col.cpu().numpy()
-            kss[i] = res[R_KHAT]
-        return out_np, kss
-    cols = lw.to(F64).t().contiguous()           # [m, n]: each set contiguous
-    if cols.data_ptr() == lw.data_ptr() and not overwrite_lw:
-        cols = cols.clone()                      # [n,1] and F-ordered inputs: t() is already contiguous -> a view
-    for i in range(m):
-        res, _, _ = _psis_column(cols[i], cols[i], Reff, False)
-        kss[i] = res[R_KHAT]
-    out = cols.t()
-    if overwrite_lw:
+        inplace = overwrite_lw and isinstance(lw, np.ndarray) and lw_np.flags.f_contiguous and lw_np.dtype == np.float64
+        cols = torch.from_numpy(np.ascontiguousarray(lw_np.T, dtype=np.float64)).to(device())     # [m, n]
+        if batched:
+            _, khat, _, _ = psislw_batch_device(cols.t(), cols.t(), Reff)
+            kss = khat.cpu().numpy()
+        else:
+            kss = _psis_columns(cols, Reff)
+        res = cols.cpu().numpy().T                   # F-contiguous n x m
+        if inplace:
+            lw_np[...] = res
+            return lw_np, kss
+        return res, kss
+    src = lw.to(F64)
+    if batched and _column_major(src) is not None:
+        # columns already contiguous (an F-ordered or transposed tensor, any leading dimension): no staging copy
+        if overwrite_lw and src.data_ptr() == lw.data_ptr():
+            out = src
+        else:
+            out = torch.empty((m, n), dtype=F64, device=src.device).t()
+        _, khat, _, _ = psislw_batch_device(src, out, Reff)
+        kss = khat.cpu().numpy()
+    else:
+        cols = src.t().contiguous()                  # [m, n]: each set contiguous
+        if cols.data_ptr() == lw.data_ptr() and not overwrite_lw:
+            cols = cols.clone()                      # [n,1] and F-ordered inputs: t() is already contiguous -> a view
+        if batched:
+            _, khat, _, _ = psislw_batch_device(cols.t(), cols.t(), Reff)
+            kss = khat.cpu().numpy()
+        else:
+            kss = _psis_columns(cols, Reff)
+        out = cols.t()
+    if overwrite_lw and out.data_ptr() != lw.data_ptr():
         lw.copy_(out)
         out = lw
     return out, kss
@@ -271,14 +362,41 @@ def gpdfitnew(x, sort=True, sort_in_place=False, return_quadrature=False):
 def psisloo(log_lik, **kwargs):
     """PSIS leave-one-out log predictive densities (_psis.py:69-110): log_lik is n x m (n posterior draws of the m
     log-likelihood terms); every column is one PSIS problem on the raw log-weights -log_lik.  Returns (loo, loos[m],
-    ks[m]); further keyword arguments go to psislw (Reff)."""
-    ll = np.asarray(log_lik, dtype=np.float64)
+    ks[m]): Python float and numpy arrays for numpy input, device tensors (loo 0-d) for a CUDA tensor.  log_lik is
+    never modified.  Further keyword arguments go to psislw (Reff).
+
+    When n <= psis_batch_max_n(Reff) the whole matrix is one launch of the batched kernel without an output array:
+    one read of log_lik, and loos come out of the kernel (sumlogs(lw_smoothed + log_lik) per column)."""
+    host = is_host(log_lik)
+    ll = np.asarray(log_lik, dtype=np.float64) if host else log_lik
     if ll.ndim != 2:
         raise ValueError('log_lik must be an n x m array')
+    n, m = ll.shape
+    Reff = kwargs.get('Reff', 1.0)
+    if n > 1 and n <= psis_batch_max_n(Reff):
+        if host:
+            cols = torch.from_numpy(np.ascontiguousarray(ll.T)).to(device())       # [m, n]
+            cols.neg_()
+        else:
+            cols = torch.empty((m, n), dtype=F64, device=ll.device)
+            torch.neg(ll.to(F64).t(), out=cols)
+        _, khat, _, loos = psislw_batch_device(cols.t(), None, Reff, want_loo=True)
+        loo = loos.sum()
+        if host:
+            return float(loo), loos.cpu().numpy(), khat.cpu().numpy()
+        return loo, loos, khat
     kwargs['overwrite_lw'] = True
-    lw, ks = psislw(np.asfortranarray(-ll), **kwargs)
-    loos = sumlogs(lw + ll, axis=0)
-    return loos.sum(), loos, ks
+    if host:
+        lw, ks = psislw(np.asfortranarray(-ll), **kwargs)
+        loos = sumlogs(lw + ll, axis=0)
+        return loos.sum(), loos, ks
+    # columns longer than the batched kernel holds: the one-column pipeline smooths them, sumlogs of the m columns
+    # (one reduction each) runs as device tensor operations
+    lw, ks = psislw(-ll.to(F64), **kwargs)
+    t = lw + ll.to(F64)
+    mx = t.max(dim=0, keepdim=True).values
+    loos = torch.log(torch.exp(t - mx).sum(dim=0)) + mx[0]
+    return loos.sum(), loos, torch.as_tensor(ks, device=ll.device)
 
 
 def sumlogs(x, axis=None, out=None):
