@@ -188,22 +188,29 @@ int vb_comm_destroy(void* comm);
 
 /* ---------------------------------------------------------------------------------------
  * Fused ELBO-gradient step: the three calls of the reference loop (optimization.py:95-98)
- *     value, grad = objective(var_param)              objectives.py:154-168
+ *     value, grad = objective(var_param)              objectives.py:154-168, :440-463
  *     direction   = sgo.descent_direction(grad)       optimization.py:188-197 (RMSProp), :308-326 (Adam)
  *     var_param   = objective.update(var_param, lr * direction)        objectives.py:57-59
- * for ExclusiveKL (entropy or path-derivative form) with a mean-field family on a GLM plugin, enqueued as three
- * kernels with no host round trip: [draw + reparameterise + operand pack] -> [sweep] -> [partial reduction +
- * cross-rank all-reduce through `comm` + value + gradient + optimiser + histories].  Everything that changes
- * from step to step (the draw-stream position, "first step" of the optimiser, history slot) lives in
- * `counters` on the device, so a captured CUDA graph of one call can be replayed.
+ * for ExclusiveKL (entropy or path-derivative form) or AlphaDivergence with a mean-field family on a GLM plugin,
+ * enqueued with no host round trip.  ExclusiveKL is three kernels: [draw + reparameterise + operand pack] ->
+ * [sweep] -> [partial reduction + cross-rank all-reduce through `comm` + value + gradient + optimiser +
+ * histories].  AlphaDivergence is five: [draw + pack] -> [forward-only sweep] -> [ll reduction + all-reduce of
+ * the S log-likelihoods + log weights + alpha weights + value] -> [weighted sweep] -> [the last kernel above,
+ * with the alpha gradient].  Everything that changes from step to step (the draw-stream position, "first step"
+ * of the optimiser, history slot) lives in `counters` on the device, so a captured CUDA graph of one call can
+ * be replayed.
  *
- * Draws: element i of step t is element counters[2] + t * (S*d rounded up to even) + i of the family's Philox
- * stream (vb_philox_normal_f64 / vb_philox_student_t_f64), t = counters[0]; with inject_base != 0 the
+ * Draws: ExclusiveKL: element i of step t is element counters[2] + t * (S*d rounded up to even) + i of the
+ * family's Philox stream (vb_philox_normal_f64 / vb_philox_student_t_f64), t = counters[0].  AlphaDivergence:
+ * the draws of step t are elements 0 .. S*d-1 of the stream of key seeds[t % seed_len] (a fresh seed per
+ * iteration, objectives.py:455); the config's seed and counters[2] are not used.  With inject_base != 0 the
  * caller's `base` is used instead (parity by draw injection).
+ * Errors: VB_ERR_INVALID_ARG for a non-finite or zero alpha, or AlphaDivergence without injection and without
+ * seeds (seeds == NULL or seed_len <= 0); VB_ERR_WORKSPACE for a workspace below vb_mf_step_workspace_bytes.
  * ------------------------------------------------------------------------------------- */
 typedef struct {
   int32_t family;        /* VB_FAMILY_MF_*                                             */
-  int32_t objective;     /* VB_OBJ_EXCLUSIVE_KL or VB_OBJ_EXCLUSIVE_KL_PATH            */
+  int32_t objective;     /* VB_OBJ_EXCLUSIVE_KL, VB_OBJ_EXCLUSIVE_KL_PATH or VB_OBJ_ALPHA */
   int32_t S, d;          /* Monte Carlo samples, model dimension                        */
   int32_t optimizer;     /* 0: none (value + gradient only), 1: RMSProp, 2: Adam        */
   int32_t quantize;      /* draw quantisation, as vb_philox_normal_f64                  */
@@ -215,7 +222,8 @@ typedef struct {
   double beta1;          /* RMSProp beta / Adam beta1                                   */
   double beta2;          /* Adam beta2                                                  */
   double jitter;
-  uint64_t seed;         /* Philox key of the family's draw stream                      */
+  uint64_t seed;         /* Philox key of the family's draw stream (ExclusiveKL)        */
+  double alpha;          /* VB_OBJ_ALPHA: the divergence's alpha (finite, != 0)         */
 } vb_step_config;
 
 typedef struct {
@@ -235,6 +243,9 @@ typedef struct {
   double* grad_hist;     /* [ring, 2d] optional ring of the gradients                   */
   double* dir_hist;      /* [ring, 2d] optional ring of the descent directions          */
   int64_t hist_len, ring;
+  const uint64_t* seeds; /* [seed_len] VB_OBJ_ALPHA without injection: Philox key of step t is
+                          *       seeds[t % seed_len], read on the device when the step runs */
+  int64_t seed_len;
 } vb_step_buffers;
 
 typedef struct {
@@ -254,8 +265,8 @@ typedef struct {
   size_t sweep_workspace_bytes;
 } vb_step_model;
 
-/* The workspace carries state between calls (the block ticket of the last kernel): zero it once before the
- * first call and hand the same buffer to every later call of the same engine. */
+/* The workspace carries state between calls (the block tickets of the reducing kernels): zero it once before the
+ * first call and hand the same buffer to every later call of the same engine.  Its size covers every objective. */
 size_t vb_mf_step_workspace_bytes(int S, int d);
 int vb_mf_step_glm(const vb_step_config* cfg, const vb_step_buffers* buf, const vb_step_model* model,
                    void* comm, void* workspace, size_t workspace_bytes, cudaStream_t stream);

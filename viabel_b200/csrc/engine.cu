@@ -14,6 +14,10 @@
 //                      through peer memory (NVLink stores + flags; no NCCL call), objective value, gradient
 //                      wrt [mu, log sigma] (SURVEY.md App. A.1), RMSProp / Adam state and parameter update,
 //                      value / iterate histories, and the step counters.
+// AlphaDivergence (objectives.py:440-463) needs every sample's global log-likelihood before the weighted
+// back-projection, so its step is FIVE kernels: the pre kernel (draws from the step's own seed), a forward-only
+// sweep, mf_alpha_weights_step_kernel (ll reduction, all-reduce of the S sums, log weights, alpha weights, value),
+// the weighted sweep, and mf_post_kernel with the alpha gradient (SURVEY.md App. A.2).  Two collectives per step.
 //
 // Peer-memory communicator (SURVEY.md 8(b)#7 `vb_comm_*`): every rank cudaMalloc's one buffer
 // [flags | 2 parities x world slots], exports it with cudaIpcGetMemHandle, and maps the others'.  A collective
@@ -127,6 +131,7 @@ struct StepCfg {
   int d_pad, chunks, rowsA;          // pre-kernel geometry: rowsA sample rows, `chunks` column tiles of 64
   double df, tconst, inv_tau2, prior_const;
   double lr, beta1, beta2, jitter;
+  double alpha;                      // VB_OBJ_ALPHA
   unsigned long long seed, stride;
 };
 
@@ -146,11 +151,17 @@ struct StepPtrs {
   double* grad_hist;
   double* dir_hist;
   long long hist_len, ring;
+  const unsigned long long* seeds;   // VB_OBJ_ALPHA: Philox key of step t is seeds[t % seed_len]
+  long long seed_len;
   // engine workspace
   double* sq_part;                   // [S][chunks]
   double* lq_part;                   // [S][chunks]
   double* vec;                       // [S + 2d] reduced (and all-reduced) sweep sums
   double* aux;                       // [4][d]: p1, p2, pa, pb
+  double* w;                         // VB_OBJ_ALPHA [S]: the sweep weights exp(lw - max lw)^alpha
+  double* prior;                     // VB_OBJ_ALPHA [S]: log prior of each sample
+  double* logq;                      // VB_OBJ_ALPHA [S]: log q of each sample
+  double* aval;                      // VB_OBJ_ALPHA [1]: the objective value
   unsigned int* ticket;
 };
 
@@ -170,13 +181,15 @@ constexpr int kPreRows = 16, kPreCols = 64;
 __global__ void __launch_bounds__(256) mf_pre_kernel(StepCfg c, StepPtrs p, fast::FastOperands ops) {
   PDL_SYNC();
   __shared__ float tt[kPreCols][kPreRows + 1];
-  const Philox ph(c.seed);
-  const unsigned long long offset = p.counters[2] + p.counters[0] * c.stride;
+  const bool alpha = c.objective == VB_OBJ_ALPHA;
+  // AlphaDivergence: a fresh stream per step from element 0, as RandomState(seed) in approx.base_draws(S, seed)
+  const Philox ph(!alpha ? c.seed : c.inject ? 0ull : p.seeds[p.counters[0] % (unsigned long long)p.seed_len]);
+  const unsigned long long offset = alpha ? 0ull : p.counters[2] + p.counters[0] * c.stride;
   const int d = c.d;
   const int s0 = blockIdx.y * kPreRows, j0 = blockIdx.x * kPreCols;
   const int cp = threadIdx.x & 31, w = threadIdx.x >> 5;
   const int j = j0 + 2 * cp;
-  const bool path = c.objective == VB_OBJ_EXCLUSIVE_KL_PATH;
+  const bool want_lq = alpha || c.objective == VB_OBJ_EXCLUSIVE_KL_PATH;
   double mu[2] = {0.0, 0.0}, ls[2] = {0.0, 0.0}, sig[2] = {0.0, 0.0};
 #pragma unroll
   for (int u = 0; u < 2; ++u)
@@ -231,7 +244,7 @@ __global__ void __launch_bounds__(256) mf_pre_kernel(StepCfg c, StepPtrs p, fast
     double sq = th[0] * th[0] + th[1] * th[1];
     sq = warp_sum(sq);
     if (cp == 0 && s < c.S) p.sq_part[(size_t)s * c.chunks + blockIdx.x] = sq;
-    if (path) {
+    if (want_lq) {
       double lq = 0.0;
       if (s < c.S) {
 #pragma unroll
@@ -285,22 +298,106 @@ struct PartDesc {
 
 constexpr int kPostGroups = 32;      // row groups of the post kernel's reduction: block = 32 columns x 32 groups
 
+// AlphaDivergence, between the forward-only and the weighted sweep (objectives.py:443-459).  Every block reduces 32
+// samples' ll over the sweep's per-CTA partials and their |theta|^2 / log q over the pre kernel's column tiles (32
+// groups, fixed-order combination); the ll sums go to the peers (or straight to vec).  The last block exchanges them,
+// then forms lw = ll + log prior - log q, m = max lw, w = exp(lw - m)^alpha, value = log(mean w) / alpha + m, as
+// alpha_weights_kernel does; on the tensor-core path it also writes w as the sweep's fp32 weight operand.  One block
+// walks all S samples in the last phase: a few strided passes, small next to the two sweeps at any S.
+__global__ void __launch_bounds__(32 * kPostGroups) mf_alpha_weights_step_kernel(StepCfg c, StepPtrs p, PartDesc q,
+                                                                                  CommView cm, fast::FastOperands ops) {
+  PDL_SYNC();
+  __shared__ double sm[3][kPostGroups][33];
+  __shared__ double red[32];
+  __shared__ unsigned int last;
+  const int S = c.S;
+  const bool multi = cm.world > 1;
+  const unsigned long long e = multi ? *cm.epoch + 1 : 0;
+  const int64_t par_off = multi ? (int64_t)(e & 1) * cm.world * cm.slot_doubles : 0;
+  {
+    const int x = threadIdx.x & 31, y = threadIdx.x >> 5;
+    const int s = blockIdx.x * 32 + x;
+    double acc = 0.0, sq = 0.0, lq = 0.0;
+    if (s < S) {
+#pragma unroll 4
+      for (int b = y; b < q.nblk_ll; b += kPostGroups) acc += q.ll_part[(size_t)b * q.stride_ll + s];
+      for (int k = y; k < c.chunks; k += kPostGroups) {
+        sq += p.sq_part[(size_t)s * c.chunks + k];
+        lq += p.lq_part[(size_t)s * c.chunks + k];
+      }
+    }
+    sm[0][y][x] = acc; sm[1][y][x] = sq; sm[2][y][x] = lq;
+    __syncthreads();
+    if (y == 0 && s < S) {
+      double t = 0.0, tq = 0.0, tl = 0.0;
+#pragma unroll
+      for (int r = 0; r < kPostGroups; ++r) { t += sm[0][r][x]; tq += sm[1][r][x]; tl += sm[2][r][x]; }     // fixed order
+      t *= q.sign_ll;
+      if (multi) {
+        for (int r = 0; r < cm.world; ++r) cm.data_peer[r][par_off + (int64_t)cm.rank * cm.slot_doubles + s] = t;
+      } else {
+        p.vec[s] = t;
+      }
+      p.prior[s] = -0.5 * tq * c.inv_tau2 + c.prior_const;
+      p.logq[s] = tl;
+    }
+  }
+  if (multi) __threadfence_system(); else __threadfence();
+  __syncthreads();
+  if (threadIdx.x == 0) last = atomicAdd(p.ticket, 1u) == gridDim.x - 1 ? 1u : 0u;
+  __syncthreads();
+  if (!last) return;
+  __threadfence();
+  if (multi) comm_signal_and_wait(cm, e);
+  double m = -INFINITY;
+  for (int s = threadIdx.x; s < S; s += blockDim.x) {
+    double ll;
+    if (multi) {
+      ll = 0.0;
+      for (int r = 0; r < cm.world; ++r) ll += __ldcg(cm.data_local + par_off + (int64_t)r * cm.slot_doubles + s);
+      p.vec[s] = ll;
+    } else {
+      ll = __ldcg(p.vec + s);
+    }
+    const double lw = ll + __ldcg(p.prior + s) - __ldcg(p.logq + s);       // objectives.py:443-446
+    p.w[s] = lw;
+    m = fmax(m, lw);
+  }
+  m = block_max(m, red);
+  double acc = 0.0;
+  for (int s = threadIdx.x; s < S; s += blockDim.x) {
+    const double v = pow(exp(p.w[s] - m), c.alpha);          // np.exp(lw - m) ** alpha
+    p.w[s] = v;
+    acc += v;
+    if (c.fast) ops.wf[s] = (float)v;
+  }
+  if (c.fast)
+    for (int s = S + threadIdx.x; s < fast::kPadS; s += blockDim.x) ops.wf[s] = 0.0f;
+  acc = block_sum(acc, red);
+  if (threadIdx.x == 0) {
+    p.aval[0] = log(acc / (double)S) / c.alpha + m;
+    *p.ticket = 0;
+    if (multi) *cm.epoch = e;
+  }
+}
+
 __global__ void __launch_bounds__(32 * kPostGroups) mf_post_kernel(StepCfg c, StepPtrs p, PartDesc q, CommView cm) {
   PDL_SYNC();
   __shared__ double sm[3][kPostGroups][33];
   __shared__ double red[32];
   __shared__ unsigned int last;
   const int S = c.S, d = c.d, nvec = S + 2 * d;
-  const bool path = c.objective == VB_OBJ_EXCLUSIVE_KL_PATH;
+  const bool path = c.objective == VB_OBJ_EXCLUSIVE_KL_PATH, alpha = c.objective == VB_OBJ_ALPHA;
+  const int lo = alpha ? S : 0;          // alpha: the ll sums were reduced and exchanged by the weights kernel
   const bool multi = cm.world > 1;
   const unsigned long long e = multi ? *cm.epoch + 1 : 0;
   const int64_t par_off = multi ? (int64_t)(e & 1) * cm.world * cm.slot_doubles : 0;
 
-  // ---- phase 1: every block reduces 32 entries of [ll | gmu | ge] over the sweep's per-CTA partials, and the
-  //      per-column sums over the samples that the prior / path terms of the gradient need ----
+  // ---- phase 1: every block reduces 32 entries of [ll | gmu | ge] (alpha: [gmu | ge]) over the sweep's per-CTA
+  //      partials, and the per-column sums over the samples that the prior / path / alpha terms of the gradient need ----
   {
     const int x = threadIdx.x & 31, y = threadIdx.x >> 5;
-    const int i = blockIdx.x * 32 + x;
+    const int i = lo + blockIdx.x * 32 + x;
     double acc = 0.0, pp = 0.0, pq = 0.0;
     int kind = -1, col = 0;               // 0: ll, 1: gmu, 2: ge
     if (i < nvec) {
@@ -312,7 +409,22 @@ __global__ void __launch_bounds__(32 * kPostGroups) mf_post_kernel(StepCfg c, St
       else { kind = 2; col = i - S - d; part = q.ge_part; nblk = q.nblk_g; stride = q.stride_g; }
 #pragma unroll 4
       for (int b = y; b < nblk; b += kPostGroups) acc += part[(size_t)b * stride + col];
-      if (kind == 1) {
+      if (alpha) {          // sum_s w_s theta_sj, sum_s w_s (for the "+1" of d/d log sigma), sum_s w_s theta_sj e_sj
+        if (kind == 1) {
+#pragma unroll 4
+          for (int s = y; s < S; s += kPostGroups) {
+            const double ws = p.w[s];
+            pp += ws * p.theta[(size_t)s * d + col];
+            pq += ws;
+          }
+        } else {
+#pragma unroll 4
+          for (int s = y; s < S; s += kPostGroups) {
+            const double ws = p.w[s];
+            pp += ws * p.theta[(size_t)s * d + col] * p.base[(size_t)s * d + col];
+          }
+        }
+      } else if (kind == 1) {
 #pragma unroll 4
         for (int s = y; s < S; s += kPostGroups) {
           const double th = p.theta[(size_t)s * d + col];
@@ -357,7 +469,7 @@ __global__ void __launch_bounds__(32 * kPostGroups) mf_post_kernel(StepCfg c, St
   // ---- phase 2 (the last block): exchange, value, gradient, optimiser, histories ----
   if (multi) {
     comm_signal_and_wait(cm, e);
-    for (int i = threadIdx.x; i < nvec; i += blockDim.x) {
+    for (int i = lo + threadIdx.x; i < nvec; i += blockDim.x) {
       double t = 0.0;
       for (int r = 0; r < cm.world; ++r) t += __ldcg(cm.data_local + par_off + (int64_t)r * cm.slot_doubles + i);
       p.vec[i] = t;
@@ -377,7 +489,10 @@ __global__ void __launch_bounds__(32 * kPostGroups) mf_post_kernel(StepCfg c, St
     const double a = __ldcg(p.vec + S + j) - __ldcg(p.aux + j) * c.inv_tau2;              // sum_s g_s[j]
     const double b = __ldcg(p.vec + S + d + j) - __ldcg(p.aux + d + j) * c.inv_tau2;      // sum_s g_s[j] e_s[j]
     double g[2];
-    if (path) {
+    if (alpha) {                 // (alpha / S) sum_s w_s (...), not divided by mean w (SURVEY.md App. A.2)
+      g[0] = c.alpha * invS * a;
+      g[1] = c.alpha * invS * (b * sig + __ldcg(p.aux + 2 * d + j));
+    } else if (path) {
       g[0] = -invS * (a + __ldcg(p.aux + 2 * d + j) / sig);
       g[1] = -invS * (b * sig + __ldcg(p.aux + 3 * d + j));
     } else {
@@ -424,9 +539,10 @@ __global__ void __launch_bounds__(32 * kPostGroups) mf_post_kernel(StepCfg c, St
       if (p.param_hist && p.ring > 0) p.param_hist[(size_t)(step % (unsigned long long)p.ring) * (2 * d) + i] = nv;
     }
   }
-  // value (objectives.py:161-164): -(mean_s f(theta_s) + H), or -(mean_s (f - log q)) for the path-derivative form;
-  // samples are taken from the top of the block so that they overlap the coordinate work above
-  for (int s = (int)blockDim.x - 1 - (int)threadIdx.x; s < S; s += blockDim.x) {
+  // value (objectives.py:161-164): -(mean_s f(theta_s) + H), or -(mean_s (f - log q)) for the path-derivative form
+  // (alpha: from the weights kernel; only logp is formed here); samples are taken from the top of the block so that
+  // they overlap the coordinate work above
+  for (int s = (int)blockDim.x - 1 - (int)threadIdx.x; s < ((alpha && !p.logp) ? 0 : S); s += blockDim.x) {
     double sq = 0.0, lq = 0.0;
     for (int k = 0; k < c.chunks; ++k) {
       sq += __ldcg(p.sq_part + s * c.chunks + k);
@@ -442,7 +558,7 @@ __global__ void __launch_bounds__(32 * kPostGroups) mf_post_kernel(StepCfg c, St
   vh = block_sum(vh, red);
   if (threadIdx.x == 0) {
     if (!path && c.family == VB_FAMILY_MF_GAUSSIAN) vh += 0.5 * d * (1.0 + kLog2Pi);     // approximations.py:218-220
-    const double v = path ? -((va - vb_) * invS) : -(va * invS + vh);
+    const double v = alpha ? __ldcg(p.aval) : path ? -((va - vb_) * invS) : -(va * invS + vh);
     p.value[0] = v;
     if (p.value_hist && (long long)step < p.hist_len) p.value_hist[step] = v;
   }
@@ -578,11 +694,12 @@ extern "C" int vb_comm_allreduce_sum_f64(void* comm, double* buf, int64_t n, cud
 // fused step
 // =================================================================================================
 struct StepLayout {
-  size_t off_sq, off_lq, off_vec, off_aux, off_ticket, total;
+  size_t off_sq, off_lq, off_vec, off_aux, off_ticket, off_w, off_prior, off_logq, off_aval, total;
   int chunks, rowsA, d_pad;
 };
 
-static void step_layout(int S, int d, int fast, StepLayout& L) {
+// the alpha arrays follow everything else, so the ExclusiveKL layout (and its size) is the same with or without them
+static void step_layout(int S, int d, int fast, int alpha, StepLayout& L) {
   L.d_pad = fast ? (int)(ceil_div(d, 256) * 256) : d;
   L.chunks = (int)ceil_div(L.d_pad, kPreCols);          // column tiles of the pre kernel
   L.rowsA = fast ? fast::kPadS : S;
@@ -593,13 +710,20 @@ static void step_layout(int S, int d, int fast, StepLayout& L) {
   L.off_vec = take(sizeof(double) * ((size_t)S + 2 * (size_t)d));
   L.off_aux = take(sizeof(double) * 4 * (size_t)d);
   L.off_ticket = take(256);
+  L.off_w = L.off_prior = L.off_logq = L.off_aval = 0;
+  if (alpha) {
+    L.off_w = take(sizeof(double) * (size_t)S);
+    L.off_prior = take(sizeof(double) * (size_t)S);
+    L.off_logq = take(sizeof(double) * (size_t)S);
+    L.off_aval = take(sizeof(double));
+  }
   L.total = off;
 }
 
 extern "C" size_t vb_mf_step_workspace_bytes(int S, int d) {
   if (S <= 0 || d <= 0) return 0;
   StepLayout L;
-  step_layout(S, d, 1, L);         // the fast layout is the larger one
+  step_layout(S, d, 1, 1, L);      // the fast layout with the alpha arrays is the largest one
   return L.total;
 }
 
@@ -611,8 +735,13 @@ extern "C" int vb_mf_step_glm(const vb_step_config* cfg, const vb_step_buffers* 
   if (cfg->family != VB_FAMILY_MF_GAUSSIAN && cfg->family != VB_FAMILY_MF_STUDENT)
     return set_error(VB_ERR_INVALID_ARG, "unknown mean-field family");
   if (cfg->family == VB_FAMILY_MF_STUDENT && !(cfg->df > 2.0)) return set_error(VB_ERR_INVALID_ARG, "df must be greater than 2");
-  if (cfg->objective != VB_OBJ_EXCLUSIVE_KL && cfg->objective != VB_OBJ_EXCLUSIVE_KL_PATH)
-    return set_error(VB_ERR_UNSUPPORTED, "mf_step: only the ExclusiveKL objectives have a fused step");
+  if (cfg->objective != VB_OBJ_EXCLUSIVE_KL && cfg->objective != VB_OBJ_EXCLUSIVE_KL_PATH && cfg->objective != VB_OBJ_ALPHA)
+    return set_error(VB_ERR_UNSUPPORTED, "mf_step: only ExclusiveKL and AlphaDivergence have a fused step");
+  const int alpha = cfg->objective == VB_OBJ_ALPHA;
+  if (alpha && (!isfinite(cfg->alpha) || cfg->alpha == 0.0))
+    return set_error(VB_ERR_INVALID_ARG, "mf_step: alpha must be finite and non-zero");
+  if (alpha && !cfg->inject_base && (!buf->seeds || buf->seed_len <= 0))
+    return set_error(VB_ERR_INVALID_ARG, "mf_step: AlphaDivergence draws need per-step seeds (or injected draws)");
   if (cfg->optimizer < 0 || cfg->optimizer > 2) return set_error(VB_ERR_INVALID_ARG, "mf_step: unknown optimiser");
   if (!buf->var_param || !buf->counters || !buf->base || !buf->theta || !buf->value || !buf->grad)
     return set_error(VB_ERR_INVALID_ARG, "mf_step: missing buffer");
@@ -623,7 +752,7 @@ extern "C" int vb_mf_step_glm(const vb_step_config* cfg, const vb_step_buffers* 
   // the pre kernel's row tiles sit on gridDim.y (at most 65535)
   if (ceil_div(S, kPreRows) > 65535) return set_error(VB_ERR_UNSUPPORTED, "mf_step: at most 1048560 samples per step");
   StepLayout L;
-  step_layout(S, d, fast, L);
+  step_layout(S, d, fast, alpha, L);
   if (workspace_bytes < L.total) return set_error(VB_ERR_WORKSPACE, "mf_step: workspace too small");
   Comm* cm = static_cast<Comm*>(comm);
   CommView view;
@@ -650,6 +779,7 @@ extern "C" int vb_mf_step_glm(const vb_step_config* cfg, const vb_step_buffers* 
     c.prior_const = 0.0;
   }
   c.lr = cfg->lr; c.beta1 = cfg->beta1; c.beta2 = cfg->beta2; c.jitter = cfg->jitter;
+  c.alpha = alpha ? cfg->alpha : 0.0;
   c.seed = cfg->seed;
   const unsigned long long n = (unsigned long long)S * (unsigned long long)d;
   c.stride = n + (n & 1);
@@ -662,11 +792,16 @@ extern "C" int vb_mf_step_glm(const vb_step_config* cfg, const vb_step_buffers* 
   p.direction = buf->direction;
   p.value_hist = buf->value_hist; p.param_hist = buf->param_hist; p.grad_hist = buf->grad_hist; p.dir_hist = buf->dir_hist;
   p.hist_len = buf->hist_len; p.ring = buf->ring;
+  p.seeds = reinterpret_cast<const unsigned long long*>(buf->seeds); p.seed_len = buf->seed_len;
   p.sq_part = reinterpret_cast<double*>(ws + L.off_sq);
   p.lq_part = reinterpret_cast<double*>(ws + L.off_lq);
   p.vec = reinterpret_cast<double*>(ws + L.off_vec);
   p.aux = reinterpret_cast<double*>(ws + L.off_aux);
   p.ticket = reinterpret_cast<unsigned int*>(ws + L.off_ticket);
+  p.w = alpha ? reinterpret_cast<double*>(ws + L.off_w) : nullptr;
+  p.prior = alpha ? reinterpret_cast<double*>(ws + L.off_prior) : nullptr;
+  p.logq = alpha ? reinterpret_cast<double*>(ws + L.off_logq) : nullptr;
+  p.aval = alpha ? reinterpret_cast<double*>(ws + L.off_aval) : nullptr;
 
   fast::FastOperands ops = {};
   memset(&ops, 0, sizeof(ops));
@@ -681,36 +816,58 @@ extern "C" int vb_mf_step_glm(const vb_step_config* cfg, const vb_step_buffers* 
   // 1. draws + reparameterisation + operand pack
   VB_CUDA(launch_pdl(mf_pre_kernel, dim3(L.chunks, (unsigned)ceil_div(L.rowsA, kPreRows)), dim3(256), stream, c, p, ops));
 
-  // 2. the sweep over this rank's observations
+  // 2. the sweep over this rank's observations.  AlphaDivergence: forward only, then the weights, then the weighted
+  //    sweep (its ll is not needed again: on the tensor-core path only the total is formed)
   PartDesc q;
-  const int total_only = (cfg->objective == VB_OBJ_EXCLUSIVE_KL && !buf->logp) ? 1 : 0;
-  if (fast) {
-    fast::FastPartials parts;
-    int rc = fast::fast_launch(model->fast_handle, model->fast_workspace, model->fast_workspace_bytes, S, 1, total_only, 1,
-                               nullptr, stream, &parts);
-    if (rc) return rc;
-    q.ll_part = parts.ll_part; q.gmu_part = parts.gmu_part; q.ge_part = parts.ge_part;
-    q.nblk_ll = parts.nblk_ll; q.nblk_g = parts.nblk_g;
-    q.stride_ll = parts.stride_ll; q.stride_g = parts.stride_g;
-    q.sign_ll = -1.0;
-  } else {
+  double* out = nullptr;
+  size_t need = 0;
+  if (!fast) {
     if (!model->X || !model->y || !model->sweep_workspace) return set_error(VB_ERR_INVALID_ARG, "mf_step: float64 model data missing");
     // the float64 sweep reduces its own partials: its outputs are one-row "partials" placed in its workspace tail
-    const size_t need = vb_glm_sweep_workspace_bytes(model->N, d, S);
+    need = vb_glm_sweep_workspace_bytes(model->N, d, S);
     if (need == 0) return set_error(VB_ERR_UNSUPPORTED, "model dimension too large for the fused sweep");
     const size_t tail = align_up(need, 256);
     if (model->sweep_workspace_bytes < tail + sizeof(double) * ((size_t)S + 2 * (size_t)d))
       return set_error(VB_ERR_WORKSPACE, "mf_step: float64 sweep workspace too small (needs S + 2d extra doubles)");
-    double* out = reinterpret_cast<double*>(static_cast<char*>(model->sweep_workspace) + tail);
-    int rc = vb_glm_sweep_f64(model->X, model->ldx, model->y, model->N, d, model->link, buf->theta, buf->base, nullptr,
-                              nullptr, S, 1, out, out + S, out + S + d, model->sweep_workspace, need, stream);
+    out = reinterpret_cast<double*>(static_cast<char*>(model->sweep_workspace) + tail);
+  }
+  auto sweep = [&](int want_grad, int total_only, const double* w) -> int {
+    if (fast) {
+      fast::FastPartials parts;
+      int rc = fast::fast_launch(model->fast_handle, model->fast_workspace, model->fast_workspace_bytes, S, want_grad,
+                                 total_only, w ? 0 : 1, nullptr, stream, &parts);
+      if (rc) return rc;
+      q.ll_part = parts.ll_part; q.gmu_part = parts.gmu_part; q.ge_part = parts.ge_part;
+      q.nblk_ll = parts.nblk_ll; q.nblk_g = parts.nblk_g;
+      q.stride_ll = parts.stride_ll; q.stride_g = parts.stride_g;
+      q.sign_ll = -1.0;
+      return VB_OK;
+    }
+    int rc = vb_glm_sweep_f64(model->X, model->ldx, model->y, model->N, d, model->link, buf->theta,
+                              want_grad ? buf->base : nullptr, w, nullptr, S, want_grad, out,
+                              want_grad ? out + S : nullptr, want_grad ? out + S + d : nullptr,
+                              model->sweep_workspace, need, stream);
     if (rc) return rc;
     q.ll_part = out; q.gmu_part = out + S; q.ge_part = out + S + d;
     q.nblk_ll = 1; q.nblk_g = 1; q.stride_ll = S; q.stride_g = d; q.sign_ll = 1.0;
+    return VB_OK;
+  };
+  if (alpha) {
+    // (the tensor-core sweep reads its weight operand, which the pre kernel has reset to ones, as p.w)
+    int rc = sweep(0, 0, nullptr);
+    if (rc) return rc;
+    VB_CUDA(launch_pdl(mf_alpha_weights_step_kernel, dim3((unsigned)ceil_div(S, 32)), dim3(32 * kPostGroups), stream,
+                       c, p, q, view, ops));
+    rc = sweep(1, fast, p.w);
+    if (rc) return rc;
+  } else {
+    const int total_only = (cfg->objective == VB_OBJ_EXCLUSIVE_KL && !buf->logp) ? 1 : 0;
+    int rc = sweep(1, total_only, nullptr);
+    if (rc) return rc;
   }
 
   // 3. reduce + exchange + finish + optimiser
-  const int nblocks_post = (S + 2 * d + 31) / 32;
+  const int nblocks_post = ((alpha ? 0 : S) + 2 * d + 31) / 32;
   VB_CUDA(launch_pdl(mf_post_kernel, dim3(nblocks_post), dim3(32 * kPostGroups), stream, c, p, q, view));
   return VB_OK;
 }

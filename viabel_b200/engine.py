@@ -1,12 +1,13 @@
 """Fused ELBO-gradient step -- the three hot-path calls of the reference loop
 (optimization.py:95-98: objective(var_param) -> descent_direction -> update) as ONE enqueue of
-three kernels through `vb_mf_step_glm`, replayed from a CUDA graph.
+three kernels (ExclusiveKL) or five (AlphaDivergence: a forward-only sweep, the weights and a
+weighted sweep) through `vb_mf_step_glm`, replayed from a CUDA graph.
 
-Everything that changes from step to step lives on the device (draw-stream position, optimiser
-"first step" flag, history slot), so the host only replays graphs; value / iterate / gradient
-histories are written by the step's last kernel into device rings.  With a sharded model the
-per-rank sums are exchanged inside that kernel through the peer-memory communicator
-(parallel.Communicator) -- no NCCL call on the hot path.
+Everything that changes from step to step lives on the device (draw-stream position or the
+per-step seed, optimiser "first step" flag, history slot), so the host only replays graphs;
+value / iterate / gradient histories are written by the step's last kernel into device rings.
+With a sharded model the per-rank sums are exchanged inside the step's kernels through the
+peer-memory communicator (parallel.Communicator) -- no NCCL call on the hot path.
 """
 import ctypes
 import gc
@@ -25,14 +26,15 @@ class StepConfig(ctypes.Structure):
     _fields_ = [('family', c_int32), ('objective', c_int32), ('S', c_int32), ('d', c_int32),
                 ('optimizer', c_int32), ('quantize', c_int32), ('inject_base', c_int32), ('reserved', c_int32),
                 ('df', c_double), ('prior_sd', c_double), ('lr', c_double), ('beta1', c_double),
-                ('beta2', c_double), ('jitter', c_double), ('seed', c_uint64)]
+                ('beta2', c_double), ('jitter', c_double), ('seed', c_uint64), ('alpha', c_double)]
 
 
 class StepBuffers(ctypes.Structure):
     _fields_ = [('var_param', c_void_p), ('opt_m', c_void_p), ('opt_nu', c_void_p), ('counters', c_void_p),
                 ('base', c_void_p), ('theta', c_void_p), ('value', c_void_p), ('grad', c_void_p),
                 ('logp', c_void_p), ('direction', c_void_p), ('value_hist', c_void_p), ('param_hist', c_void_p),
-                ('grad_hist', c_void_p), ('dir_hist', c_void_p), ('hist_len', c_int64), ('ring', c_int64)]
+                ('grad_hist', c_void_p), ('dir_hist', c_void_p), ('hist_len', c_int64), ('ring', c_int64),
+                ('seeds', c_void_p), ('seed_len', c_int64)]
 
 
 class StepModel(ctypes.Structure):
@@ -47,14 +49,24 @@ def _dp(t):
 
 
 def fused_step_supported(objective, optimizer=None):
-    """True when `objective` (and `optimizer`) can run as the fused three-kernel step: ExclusiveKL
-    (entropy or path-derivative form, no control variates) with a mean-field family on a GLM
-    plugin, and plain RMSProp / Adam (or no optimiser)."""
+    """True when `objective` (and `optimizer`) can run as the fused step: ExclusiveKL (entropy or
+    path-derivative form, no control variates) or AlphaDivergence (finite, non-zero alpha) with a
+    mean-field family on a GLM plugin, and plain RMSProp / Adam (or no optimiser)."""
     from .approximations import _MeanField
     from .models import GLMModel
-    from .objectives import ExclusiveKL
+    from .objectives import AlphaDivergence, ExclusiveKL
     from .optimization import Adam, RMSProp
-    if type(objective) is not ExclusiveKL or objective.hessian_approx_method is not None:
+    if type(objective) is ExclusiveKL:
+        if objective.hessian_approx_method is not None:
+            return False
+    elif type(objective) is AlphaDivergence:
+        try:
+            alpha = float(objective.alpha)
+        except (TypeError, ValueError):
+            return False
+        if not np.isfinite(alpha) or alpha == 0.0:
+            return False
+    else:
         return False
     if not isinstance(objective.approx, _MeanField) or not isinstance(objective.model, GLMModel):
         return False
@@ -75,6 +87,10 @@ class FusedStep(object):
 
     ring     : rows of the iterate / gradient / direction rings (0: none)
     hist_len : length of the value history (0: none)
+
+    AlphaDivergence draws step t from a fresh Philox stream keyed by seeds[t % seed_len] (the
+    reference draws a new global-numpy seed per call); set them with set_seeds() before the steps
+    that use them.  ExclusiveKL draws from the family's own stream.
     """
 
     def __init__(self, objective, optimizer=None, ring=0, hist_len=0, want_logp=False, want_grad_hist=False,
@@ -111,13 +127,23 @@ class FusedStep(object):
         # zero-initialised: the workspace carries the kernels' block ticket across calls
         self.ws = torch.zeros(_lib.lib.vb_mf_step_workspace_bytes(S, d), dtype=torch.uint8, device=dev)
         self.steps_done = 0
-        self.launches_per_step = 3
         self.path = model.path
         self.quantize = int(approx.quantize_draws)
+        from .objectives import AlphaDivergence
+        self.alpha = type(objective) is AlphaDivergence
+        # pre, sweep, post; AlphaDivergence: pre, forward sweep, weights, weighted sweep, post
+        self.launches_per_step = 5 if self.alpha else 3
+        # AlphaDivergence: per-step seeds, one per history slot; the family's own stream is not used
+        self.seed_len = max(1, self.hist_len) if self.alpha else 0
+        self.seeds = torch.zeros(self.seed_len, dtype=torch.int64, device=dev) if self.alpha else None
 
         cfg = StepConfig()
         cfg.family = approx._family
-        cfg.objective = _lib.OBJ_EXCLUSIVE_KL_PATH if objective._use_path_deriv else _lib.OBJ_EXCLUSIVE_KL
+        if self.alpha:
+            cfg.objective = _lib.OBJ_ALPHA
+            cfg.alpha = float(objective.alpha)
+        else:
+            cfg.objective = _lib.OBJ_EXCLUSIVE_KL_PATH if objective._use_path_deriv else _lib.OBJ_EXCLUSIVE_KL
         cfg.S, cfg.d = S, d
         cfg.optimizer = self.opt_kind
         cfg.quantize = self.quantize
@@ -152,7 +178,9 @@ class FusedStep(object):
             mdl.N, mdl.link = model.N, model.link
             mdl.sweep_workspace, mdl.sweep_workspace_bytes = sws.data_ptr(), sws.numel()
             self._keep = (sws,)
-            self.launches_per_step = 7     # pre, pack, sweep, 3 x reduce, post
+            # pre, pack, sweep, 3 x reduce, post; AlphaDivergence: pre, forward (pack, sweep, reduce), weights,
+            # weighted (pack, sweep, 3 x reduce), post
+            self.launches_per_step = 11 if self.alpha else 7
         self.mdl = mdl
 
         self.comm = None
@@ -170,8 +198,10 @@ class FusedStep(object):
         b.value_hist, b.param_hist = _dp(self.value_hist), _dp(self.param_hist)
         b.grad_hist, b.dir_hist = _dp(self.grad_hist), _dp(self.dir_hist)
         b.hist_len, b.ring = self.hist_len, self.ring
+        b.seeds, b.seed_len = _dp(self.seeds), self.seed_len
         self.buf = b
         self._graphs = {}
+        self._warm = False           # a step has been enqueued eagerly: the lazy state a capture may not create exists
         self._pin_in = self._pin_out = None
 
     # -- state ---------------------------------------------------------------------------------
@@ -180,6 +210,39 @@ class FusedStep(object):
         return (self.model is objective.model and self.approx is objective.approx and self.path == objective.model.path
                 and self.quantize == int(objective.approx.quantize_draws) and self.cfg.seed == objective.approx._seed
                 and (self.path != 'fast' or self._keep[0] is objective.model._fast[2]))
+
+    @property
+    def _own_stream(self):
+        """True when the steps draw from the family's own stream (ExclusiveKL without injected draws)."""
+        return not self.inject and not self.alpha
+
+    def set_seeds(self, t0, seeds):
+        """Philox keys of steps t0 .. t0 + len(seeds) - 1 (AlphaDivergence), stored at t % seed_len.  A
+        stream-ordered copy from pinned memory: it lands after the steps already enqueued and before the ones
+        enqueued after it, and the host does not wait for it."""
+        seeds = np.ascontiguousarray(seeds, dtype=np.uint64).reshape(-1)
+        m = seeds.size
+        if m == 0:
+            return
+        if m > self.seed_len:
+            raise ValueError('more seeds than the engine keeps (%d)' % self.seed_len)
+        # the pinned block is recycled by torch's host allocator only after the copy has run
+        host = torch.from_numpy(seeds.view(np.int64)).pin_memory()
+        a = int(t0) % self.seed_len
+        n1 = min(m, self.seed_len - a)
+        self.seeds[a:a + n1].copy_(host[:n1], non_blocking=True)
+        if n1 < m:
+            self.seeds[:m - n1].copy_(host[n1:], non_blocking=True)
+
+    def draw_seeds(self, m):
+        """Seeds of the next m AlphaDivergence steps from the global numpy RNG, as the reference draws one per call
+        (objectives.py:455).  One vectorised draw of m seeds gives the values of m scalar draws and leaves the RNG
+        in the same state.  On a sharded model rank 0's seeds are used everywhere (one broadcast for m steps)."""
+        seeds = np.random.randint(2 ** 32, dtype=np.uint64, size=int(m))
+        if getattr(self.model, 'sharded', False):
+            from .parallel import broadcast_seeds
+            seeds = broadcast_seeds(seeds, getattr(self.model, 'process_group', None))
+        self.set_seeds(self.steps_done, seeds)
 
     def _rebase(self):
         """Point step `steps_done` of this engine at the family's current stream position."""
@@ -190,7 +253,7 @@ class FusedStep(object):
 
     def sync_stream_position(self):
         """Call before enqueuing when something else may have drawn from the family's stream."""
-        if not self.inject and int(self.approx._offset) != self._offset0 + self.steps_done * self._stride:
+        if self._own_stream and int(self.approx._offset) != self._offset0 + self.steps_done * self._stride:
             self._rebase()
 
     def set_param(self, var_param):
@@ -212,12 +275,12 @@ class FusedStep(object):
         self.counters[0] = 0
         if not keep_optimizer_state:
             self.counters[1] = 0
-        if not self.inject:
+        if self._own_stream:
             self.approx._offset = pos
         self._rebase()
 
     def _after(self):
-        if not self.inject:
+        if self._own_stream:
             self.approx._offset = self._offset0 + self.steps_done * self._stride
         self.approx.last_base = self.base
 
@@ -255,24 +318,32 @@ class FusedStep(object):
     def _capture(self, key, body):
         g = self._graphs.get(key)
         if g is None:
-            # one eager step outside the capture (lazy function attributes, tensor maps), device state rolled back
-            snap = self._snapshot()
-            side = torch.cuda.Stream()
-            side.wait_stream(torch.cuda.current_stream())
-            with torch.cuda.stream(side):
-                self.enqueue()
-            torch.cuda.current_stream().wait_stream(side)
-            torch.cuda.synchronize()
-            self._restore(snap)
-            torch.cuda.synchronize()
+            if not self._warm:
+                # one eager step outside the capture (lazy function attributes, tensor maps), device state rolled back
+                snap = self._snapshot()
+                side = torch.cuda.Stream()
+                side.wait_stream(torch.cuda.current_stream())
+                with torch.cuda.stream(side):
+                    self.enqueue()
+                torch.cuda.current_stream().wait_stream(side)
+                torch.cuda.synchronize()
+                self._restore(snap)
+                torch.cuda.synchronize()
+                self._warm = True
             g = torch.cuda.CUDAGraph()
-            # no garbage collection inside the capture: a collected object that owns device resources (an old
-            # graph, a model handle) would call cudaFree / cudaGraphExecDestroy, which a global-mode capture forbids
+            # Captured on a fresh side stream without synchronising the device: the capture only records launches,
+            # so the host builds the graph while the steps already enqueued keep the GPU busy.
+            # No garbage collection inside the capture: a collected object that owns device resources (an old
+            # graph, a model handle) would call cudaFree / cudaGraphExecDestroy, which a capture forbids.
             gc_was_on = gc.isenabled()
             gc.disable()
             try:
-                with torch.cuda.graph(g, capture_error_mode='thread_local'):
-                    body()
+                with torch.cuda.stream(torch.cuda.Stream()):
+                    g.capture_begin(capture_error_mode='thread_local')
+                    try:
+                        body()
+                    finally:
+                        g.capture_end()
             finally:
                 if gc_was_on:
                     gc.enable()
@@ -286,13 +357,23 @@ class FusedStep(object):
         if not use_graph:
             for _ in range(n):
                 self.enqueue()
+            self._warm = self._warm or n > 0
         else:
-            big = n // unroll if unroll > 1 else 0
+            m = n
+            big = m // unroll if unroll > 1 else 0
+            if not self._warm and ((big and unroll not in self._graphs) or (m - big * unroll and 1 not in self._graphs)):
+                # the first step runs eagerly and counts: it creates what a capture may not (module loads, function
+                # attributes, tensor maps), so no rolled-back warm-up step is spent (eager and replayed steps are
+                # bitwise equal)
+                self.enqueue()
+                self._warm = True
+                m -= 1
+                big = m // unroll if unroll > 1 else 0
             if big:
                 g = self._capture(unroll, lambda: [self.enqueue() for _ in range(unroll)])
                 for _ in range(big):
                     g.replay()
-            rest = n - big * unroll
+            rest = m - big * unroll
             if rest:
                 g = self._capture(1, self.enqueue)
                 for _ in range(rest):

@@ -101,6 +101,8 @@ class StochasticGradientOptimizer(Optimizer):
         try:
             while done < n_iters:
                 m = min(chunk, n_iters - done)
+                if eng.alpha:
+                    eng.draw_seeds(m)
                 eng.run(m)
                 done += m
                 if self.progress:
@@ -134,10 +136,11 @@ class StochasticGradientOptimizer(Optimizer):
         from .engine import fused_step_supported
         from .objectives import VariationalObjective
         if n_iters > 0 and np.ndim(init_param) == 1 and fused_step_supported(objective, self):
+            rng = np.random.get_state()
             try:
                 return self._optimize_fused(n_iters, objective, init_param)
             except NotImplementedError:
-                pass
+                np.random.set_state(rng)         # AlphaDivergence seeds drawn for the fused step: draw them again
         var_param = to_dev(init_param).clone()
         iap = self._iterate_avg_prop
         results = defaultdict(list)
@@ -464,6 +467,8 @@ class FASO(Optimizer):
                     k_next = min(k_next, max(k_conv + W_check, done))
                 k_next = min(k_next, n_iters - 1)
                 t0 = _time.perf_counter()
+                if eng.alpha:
+                    eng.draw_seeds(k_next + 1 - done)
                 eng.run(k_next + 1 - done)
                 torch.cuda.current_stream().synchronize()
                 opt_time += _time.perf_counter() - t0
@@ -556,10 +561,11 @@ class FASO(Optimizer):
         sgo = self._sgo
         if (n_iters > 0 and np.ndim(init_param) == 1 and fused_step_supported(objective, sgo)
                 and 3 * n_iters * np.size(init_param) * 8 < 8e9):
+            rng = np.random.get_state()
             try:
                 return self._optimize_fused(n_iters, objective, init_param)
             except NotImplementedError:
-                pass
+                np.random.set_state(rng)         # AlphaDivergence seeds drawn for the fused step: draw them again
         diagnostics = sgo._diagnostics
         k_conv = k_stopped = k_Rhat = None
         lr = sgo._learning_rate

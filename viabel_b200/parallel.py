@@ -10,6 +10,7 @@ torch.distributed over NCCL (gloo in the CPU tests of this host logic).
 import ctypes
 import warnings
 
+import numpy as np
 import torch
 import torch.distributed as dist
 
@@ -121,12 +122,18 @@ def allreduce_sum_(t, group=None):
 
 def broadcast_seed(seed, group=None):
     """Rank 0's seed on every rank: the sharded objectives need identical base draws everywhere."""
+    return int(broadcast_seeds(np.array([int(seed)], dtype=np.uint64), group)[0])
+
+
+def broadcast_seeds(seeds, group=None):
+    """Rank 0's seeds (a uint64 array of values below 2^63) on every rank, in one collective."""
+    seeds = np.asarray(seeds, dtype=np.uint64)
     if not is_distributed(group):
-        return int(seed)
+        return seeds
     dev = torch.device('cuda', torch.cuda.current_device()) if dist.get_backend(group) == 'nccl' else 'cpu'
-    t = torch.tensor([int(seed)], dtype=torch.int64, device=dev)
+    t = torch.as_tensor(seeds.astype(np.int64), device=dev)
     dist.broadcast(t, src=dist.get_global_rank(group, 0) if group is not None else 0, group=group)
-    return int(t.item())
+    return t.cpu().numpy().astype(np.uint64)
 
 
 def allgather_ragged(t, group=None):
